@@ -9,6 +9,7 @@ reduction of the timings and the gather of the parity checksums.
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # our CUDA path
     python bench.py --impl reference [--steps K] [--warmup W]      # the CPU path timed on this box's host cores
+    python bench.py --dump-outputs DIR ...                         # also write the last timed step's results (rank 0)
 
 Prints ONE JSON line (rank 0).  Beyond the base contract it carries, all measured in the same run but OUTSIDE the
 headline timed region:
@@ -44,6 +45,7 @@ BATCH_PER_GPU = 65536               # configs[1]
 SEED = 1234                         # SURVEY.md s.8(d): timing seed
 HBM_FALLBACK_GBS = 6650.0           # /opt/skills/guides/B200_PROFILING.md fallback when MEASURED_PEAKS.json is absent
 PARITY_HEAD, PARITY_TAIL = 3072, 1024   # polynomials of every shard whose forward spectra are compared with the oracle
+DUMP_BYTES_PER_ARRAY = 16 << 20     # --dump-outputs: float64 data per file (both files with headers stay below 64 MB)
 
 
 def host_threads() -> int:
@@ -239,6 +241,33 @@ def load_traffic(kernel_key: str):
         return None, None
 
 
+def dump_outputs(out_dir: str, ctx, data, B: int) -> None:
+    """--dump-outputs: what the last timed step handed its caller, so that two builds can be compared output for output.
+    A step is fwd then inv in place: its caller receives the forward spectra, then the batch back from the inverse.  Every
+    step starts from the same batch (each is an exact round trip, checked by checksum), so the last step's spectra are
+    recomputed here, after the timed region, from the batch it left behind, and the batch is restored.  A fixed, seeded
+    sample of whole polynomials is written as float64 (exact for residues < 2^30): ntt_fwd.npy and ntt_inv.npy, both
+    [rows][L][n]."""
+    import numpy as np
+    import torch
+    L, n = ctx.L, ctx.n
+    rows = max(1, min(B, DUMP_BYTES_PER_ARRAY // (L * n * 8)))
+    idx = np.sort(np.random.default_rng(SEED).choice(B, size=rows, replace=False))
+    sel = torch.from_numpy(idx).to(data.device)
+    polys = data.view(B, L * n)
+
+    def sample():
+        return polys.index_select(0, sel).cpu().numpy().view(np.uint32).reshape(rows, L, n).astype(np.float64)
+
+    inv_out = sample()
+    ctx.fwd(data)
+    fwd_out = sample()
+    ctx.inv(data)
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ntt_fwd.npy"), fwd_out)
+    np.save(os.path.join(out_dir, "ntt_inv.npy"), inv_out)
+
+
 def run_ours(args, rank: int, local_rank: int, world: int):
     import numpy as np
     import torch
@@ -378,6 +407,9 @@ def run_ours(args, rank: int, local_rank: int, world: int):
     fwd_ms = [ev[k][0].elapsed_time(ev[k][1]) for k in range(K)]
     inv_ms = [ev[k][1].elapsed_time(ev[k][2]) for k in range(K)]
     ok = ok_roundtrip0 and ctx.checksum(data, first_index=first_poly * L * n) == chk0   # K round trips leave the batch unchanged
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, ctx, data, B)
+        ok = ok and ctx.checksum(data, first_index=first_poly * L * n) == chk0     # and so does the dump's extra one
 
     # ---- sustained: >= 2 s of back-to-back steps with NVML sampled throughout (a 20 ms burst says nothing about clocks)
     sustained = None
@@ -675,7 +707,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip BASELINE configs 3-5 and the strong-scaling block")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--full-parity", action="store_true", help="also compare the whole forward batch with the oracle")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's results for a fixed sample of rank 0's polynomials: DIR/ntt_inv.npy "
+                         "(the batch the last inverse returned) and DIR/ntt_fwd.npy (its forward spectra, recomputed "
+                         "after the timed region from that batch by one more fwd + inv)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
     rank, local_rank, world = env_int("RANK", 0), env_int("LOCAL_RANK", 0), env_int("WORLD_SIZE", 1)
     if world == 1 and args.gpus > 1 and args.impl == "ours":

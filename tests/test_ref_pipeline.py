@@ -162,6 +162,9 @@ def test_compat_driver_real_ntt_instance():
     assert (got == O.ref_fwd_u64(x, x, q, tw, pre, frames)).all()
     dummy = _run_driver("agx_main_compat")          # main.cpp's dummy data by default
     assert len(dummy) == 16384 and int(dummy[0]) == 15752083817248508221
+    # what the reference's main.cpp prints for the same data (the known answer of the unmodified-main.cpp test above)
+    assert hashlib.sha256("".join(l + "\n" for l in dummy).encode()).hexdigest() == \
+        "68db50a07a87d4e18387a721d88b42291198aba2f9e9138e2e52d45ad6537c5c"
 
 
 def test_c_abi_from_plain_c():

@@ -64,6 +64,9 @@ def _load() -> C.CDLL:
         "agx_ref_output": [vp, _u64p, C.c_int32],
         "agx_wait": [vp],
         "agx_ref_fwd_dev": [vp, C.c_uint32, vp, vp, vp, C.c_uint64, vp, vp, C.c_uint32, vp],
+        "agx_ref_inv_dev": [vp, C.c_uint32, vp, vp, C.c_uint64, vp, vp, C.c_uint32, vp],
+        "agx_ref_polymul_dev": [vp, C.c_uint32, vp, vp, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint32, vp],
+        "agx_ref_polymul_by_spectrum_dev": [vp, C.c_uint32, vp, vp, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint32, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -77,7 +80,8 @@ def _load() -> C.CDLL:
     return L
 
 
-EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_measure_butterfly_peak agx_destroy agx_get_psi agx_get_tables agx_ntt_fwd agx_ntt_inv agx_polymul agx_polymul_by_spectrum agx_polymul_by_spectrum_host agx_elementwise agx_bitrev "
+EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_inv_dev agx_ref_polymul_dev "
+           "agx_ref_polymul_by_spectrum_dev agx_measure_butterfly_peak agx_destroy agx_get_psi agx_get_tables agx_ntt_fwd agx_ntt_inv agx_polymul agx_polymul_by_spectrum agx_polymul_by_spectrum_host agx_elementwise agx_bitrev "
            "agx_ntt_fwd_host agx_ntt_inv_host agx_polymul_host agx_host_alloc agx_host_free agx_fill_synthetic "
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant").split()
@@ -349,12 +353,35 @@ class RefPipeline:
             self._keep.clear()
             self._n, self._out = 0, None
 
+    @staticmethod
+    def _ptr(t) -> int:
+        return t if isinstance(t, int) else t.data_ptr()
+
     def fwd_dev(self, N: int, d_in, d_in2, d_out, modulus: int, d_tw, d_pre, frames: int, stream=None):
         """agx_ref_fwd_dev on torch CUDA int64 tensors (or raw device addresses)."""
-        def ptr(t):
-            return t if isinstance(t, int) else t.data_ptr()
+        ptr = self._ptr
         _ck(lib().agx_ref_fwd_dev(self._h, N, ptr(d_in), ptr(d_in2), ptr(d_out), modulus, ptr(d_tw), ptr(d_pre), frames,
                                   _stream_ptr(stream)), "agx_ref_fwd_dev")
+
+    def inv_dev(self, N: int, d_in, d_out, modulus: int, d_itw, d_ipre, frames: int, stream=None):
+        """agx_ref_inv_dev: the inverse of fwd_dev (bit-reversed in, natural out); d_itw / d_ipre from psi^-1."""
+        ptr = self._ptr
+        _ck(lib().agx_ref_inv_dev(self._h, N, ptr(d_in), ptr(d_out), modulus, ptr(d_itw), ptr(d_ipre), frames,
+                                  _stream_ptr(stream)), "agx_ref_inv_dev")
+
+    def polymul_dev(self, N: int, d_c, d_a, d_b, modulus: int, d_tw, d_pre, d_itw, d_ipre, frames: int, stream=None):
+        """agx_ref_polymul_dev: c = a * b mod (X^N + 1, q) per frame (reduced operands; c may alias a and/or b)."""
+        ptr = self._ptr
+        _ck(lib().agx_ref_polymul_dev(self._h, N, ptr(d_c), ptr(d_a), ptr(d_b), modulus, ptr(d_tw), ptr(d_pre), ptr(d_itw),
+                                      ptr(d_ipre), frames, _stream_ptr(stream)), "agx_ref_polymul_dev")
+
+    def polymul_by_spectrum_dev(self, N: int, d_c, d_a, d_b_hat, modulus: int, d_tw, d_pre, d_itw, d_ipre, frames: int,
+                                stream=None):
+        """agx_ref_polymul_by_spectrum_dev: c = INTT(NTT(a) .* b_hat), b_hat = fwd_dev(b)."""
+        ptr = self._ptr
+        _ck(lib().agx_ref_polymul_by_spectrum_dev(self._h, N, ptr(d_c), ptr(d_a), ptr(d_b_hat), modulus, ptr(d_tw),
+                                                  ptr(d_pre), ptr(d_itw), ptr(d_ipre), frames, _stream_ptr(stream)),
+            "agx_ref_polymul_by_spectrum_dev")
 
     def launch_count(self) -> int:
         v = C.c_uint64()

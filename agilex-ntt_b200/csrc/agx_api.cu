@@ -722,6 +722,62 @@ int ref_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64_t *
     return (int)cudaGetLastError();
 }
 
+// The inverse transform of `frames` frames [frames][N] (bit-reversed in, natural out, results in [0,q)), with the
+// pointwise product by d_mul fused into its load when d_mul is not null.  d_out may equal d_in and/or d_mul.
+// Odd modulus, 3 <= q < 2^62 (checked by the callers).
+int ref_inv_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64_t *d_mul, uint64_t *d_out,
+                   const uint64_t *d_itw, const uint64_t *d_ipre, uint64_t q, size_t frames, cudaStream_t st) {
+    typedef unsigned __int128 u128;
+    RefInvConst p{};
+    p.q = q;
+    uint64_t half = (q + 1) / 2, ninv = 1;                         // n^-1 = ((q+1)/2)^logn mod q
+    for (uint32_t i = 0; i < logn; i++) ninv = (uint64_t)((u128)ninv * half % q);
+    p.ninv = ninv;
+    p.ninv_p = (uint64_t)(((u128)ninv << 64) / q);
+    p.k = 64 - (uint32_t)__builtin_clzll(q);
+    p.mu = (uint64_t)(((u128)1 << (2 * p.k)) / q);
+    p.recip = (uint64_t)(((u128)1 << (63 + p.k)) / q);
+    if (logn >= 10) {
+        // one CTA per frame up to N = 16384; two per frame and a streaming last stage at N = 32768
+        const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+        const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+        const unsigned grid = (unsigned)(frames << split);
+        switch (lg) {
+            case 14: ref_u64_inv_frame_kernel<512><<<grid, 512, smem, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn); break;
+            case 13: ref_u64_inv_frame_kernel<256><<<grid, 256, smem, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn); break;
+            case 12: ref_u64_inv_frame_kernel<128><<<grid, 128, smem, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn); break;
+            case 11: ref_u64_inv_frame_kernel<64><<<grid, 64, smem, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn); break;
+            default: ref_u64_inv_frame_kernel<32><<<grid, 32, smem, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn); break;
+        }
+        c->launches++;
+        if (split) {
+            const size_t units = frames << (logn - 2);
+            const unsigned blocks = (unsigned)std::min<size_t>((units + 255) / 256, (size_t)c->sms * 8);
+            ref_u64_inv_last_stage_kernel<<<blocks, 256, 0, st>>>(d_out, d_itw, p, logn, frames);
+            c->launches++;
+        }
+    } else {
+        const uint32_t N = 1u << logn;
+        const unsigned threads = N / 2 < 32 ? 32 : N / 2;
+        ref_inv_u64_kernel<<<(unsigned)frames, threads, 0, st>>>(d_in, d_mul, d_out, d_itw, d_ipre, p, logn);
+        c->launches++;
+    }
+    return (int)cudaGetLastError();
+}
+
+// Argument checks shared by the u64 inverse and product entry points: AGX_OK, or AGX_E_INVALID with *logn untouched.
+int ref_inv_check(agx_ctx *c, uint32_t N, std::initializer_list<const void *> ptrs, uint64_t modulus, uint32_t *logn) {
+    if (!c || N < 4 || N > 32768 || (N & (N - 1))) return AGX_E_INVALID;
+    // odd, and the lazy range [0,4q) inside 64 bits; q = 1 has no Barrett constants
+    if (!(modulus & 1) || modulus >= (1ull << 62) || modulus < 3) return AGX_E_INVALID;
+    for (const void *p : ptrs)                                    // frames and tables are read by 16-byte accesses
+        if (!p || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    uint32_t l = 0;
+    while ((1u << l) < N) l++;
+    *logn = l;
+    return AGX_OK;
+}
+
 // ------------------------------------------------------------------------------- reference-shaped u64 pipeline
 
 // Reference-shaped round: loader + compute unit + drain (ntt.cpp:508-607, 86-506, 610-640) as a chunked three-slot
@@ -898,6 +954,8 @@ int agx_create_tables(agx_ctx **out, const agx_parms *parms, const uint32_t *psi
         const int frame_smem = 17 * 1024 * 8;                          // N = 16384 image: 136 KB
         if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
         if (e == cudaSuccess) e = cudaFuncSetAttribute(bitrev_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 << 10);
         if (e != cudaSuccess) { delete c; return (int)e; }
     }
@@ -1203,6 +1261,63 @@ int agx_ref_fwd_dev(agx_ctx *c, uint32_t N, const uint64_t *d_in, const uint64_t
     uint32_t logn = 0;
     while ((1u << logn) < N) logn++;
     return ref_launch(c, logn, d_in, d_in2, d_out, d_twiddles, d_precon_twiddles, modulus, numFrames, (cudaStream_t)stream);
+}
+
+int agx_ref_inv_dev(agx_ctx *c, uint32_t N, const uint64_t *d_in, uint64_t *d_out, uint64_t modulus,
+                    const uint64_t *d_inv_twiddles, const uint64_t *d_inv_precon_twiddles, uint32_t numFrames, void *stream) {
+    uint32_t logn = 0;
+    if (ref_inv_check(c, N, {d_in, d_out, d_inv_twiddles, d_inv_precon_twiddles}, modulus, &logn)) return AGX_E_INVALID;
+    if (numFrames == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    return ref_inv_launch(c, logn, d_in, nullptr, d_out, d_inv_twiddles, d_inv_precon_twiddles, modulus, numFrames,
+                          (cudaStream_t)stream);
+}
+
+int agx_ref_polymul_dev(agx_ctx *c, uint32_t N, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b, uint64_t modulus,
+                        const uint64_t *d_twiddles, const uint64_t *d_precon_twiddles, const uint64_t *d_inv_twiddles,
+                        const uint64_t *d_inv_precon_twiddles, uint32_t numFrames, void *stream) {
+    uint32_t logn = 0;
+    if (ref_inv_check(c, N, {d_c, d_a, d_b, d_twiddles, d_precon_twiddles, d_inv_twiddles, d_inv_precon_twiddles}, modulus,
+                      &logn))
+        return AGX_E_INVALID;
+    if (numFrames == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (d_c == d_b && d_c != d_a) std::swap(d_a, d_b);             // the product commutes: c == a from here on
+    // c = NTT(a); scratch = NTT(b) unless squaring; c = INTT(c .* (scratch or c))
+    uint64_t *tmp = nullptr;
+    int rc = ref_launch(c, logn, d_a, d_a, d_c, d_twiddles, d_precon_twiddles, modulus, numFrames, st);
+    if (!rc && d_a != d_b) {
+        rc = (int)cudaMallocAsync(&tmp, (size_t)numFrames * N * 8, st);
+        if (!rc) rc = ref_launch(c, logn, d_b, d_b, tmp, d_twiddles, d_precon_twiddles, modulus, numFrames, st);
+    }
+    if (!rc) rc = ref_inv_launch(c, logn, d_c, tmp ? tmp : d_c, d_c, d_inv_twiddles, d_inv_precon_twiddles, modulus, numFrames, st);
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
+int agx_ref_polymul_by_spectrum_dev(agx_ctx *c, uint32_t N, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b_hat,
+                                    uint64_t modulus, const uint64_t *d_twiddles, const uint64_t *d_precon_twiddles,
+                                    const uint64_t *d_inv_twiddles, const uint64_t *d_inv_precon_twiddles, uint32_t numFrames,
+                                    void *stream) {
+    uint32_t logn = 0;
+    if (ref_inv_check(c, N, {d_c, d_a, d_b_hat, d_twiddles, d_precon_twiddles, d_inv_twiddles, d_inv_precon_twiddles},
+                      modulus, &logn))
+        return AGX_E_INVALID;
+    if (numFrames == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    // NTT(a) goes to c unless c holds b_hat, which the inverse still has to read: then to a scratch buffer
+    uint64_t *tmp = nullptr, *spec = d_c;
+    int rc = AGX_OK;
+    if (d_c == d_b_hat) {
+        rc = (int)cudaMallocAsync(&tmp, (size_t)numFrames * N * 8, st);
+        spec = tmp;
+    }
+    if (!rc) rc = ref_launch(c, logn, d_a, d_a, spec, d_twiddles, d_precon_twiddles, modulus, numFrames, st);
+    if (!rc) rc = ref_inv_launch(c, logn, spec, d_b_hat, d_c, d_inv_twiddles, d_inv_precon_twiddles, modulus, numFrames, st);
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }
+    return rc;
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

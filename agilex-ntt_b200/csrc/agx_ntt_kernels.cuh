@@ -1256,6 +1256,247 @@ __global__ void __launch_bounds__(NT, 512 / NT) ref_u64_frame_kernel(const uint6
     for (uint32_t i = tid; i < M; i += NT) dst[i] = img[i + (i >> 4)];
 }
 
+// ------------------------------------------------------------------- u64 inverse transform and negacyclic product
+// No reference counterpart (the reference has only the forward, SURVEY.md s.0).  The mirror of the forward above:
+// Gentleman-Sande stages h = N/2 .. 1 (h groups, group j reads iroots[h + j] -- the table order of ntt.cpp:298-300 built
+// from psi^-1, so stage h has the shape of the forward's stage m = h), Harvey-lazy on [0,2q):
+//   u' = u + v  (one conditional subtraction of 2q),   v' = Shoup(u - v + 2q, w)  (< 2q for any input below 2^64)
+// and n^-1 folded into the last stage (h = 1): u' = Shoup(u + v, n^-1), v' = Shoup(u - v + 2q, iroots[1] * n^-1), then
+// the reduction to [0,q).  The lazy range [0,4q) must fit 64 bits: q < 2^62 (agx_ref_inv_dev refuses larger moduli).
+// Optional fused operand `mul` (nullptr = none): the load phase replaces x[i] by x[i] * mul[i] mod q (Barrett, HAC 14.42
+// with b = 2: k = bitlen(q), mu = floor(2^2k / q) < 2^63; the remainder is < 3q, so two conditional subtractions), which
+// makes the pointwise product of agx_ref_polymul_dev part of the inverse's load.
+struct RefInvConst {
+    uint64_t q, ninv, ninv_p;      // n^-1 mod q and floor(n^-1 * 2^64 / q)
+    uint64_t mu;                   // floor(2^(2k) / q)
+    uint64_t recip;                // floor(2^(63+k) / q) < 2^64 (ref_inv_fold)
+    uint32_t k;                    // bit length of q, 2 <= k <= 62
+};
+
+__device__ __forceinline__ uint64_t ref_shoup_u64(uint64_t y, uint64_t W, uint64_t Wp, uint64_t q) {
+    const uint64_t c1 = __umul64hi(y, Wp);
+#if AGX_U64_NEGQ
+    uint64_t negq;                                // see ref_bfly_u64
+    asm("neg.s64 %0, %1;" : "=l"(negq) : "l"(q));
+    return W * y + c1 * negq;                     // W*y - c1*q mod 2^64, in [0,2q)
+#else
+    return W * y - c1 * q;
+#endif
+}
+
+__device__ __forceinline__ void ref_gs_bfly_u64(uint64_t &x, uint64_t &y, uint64_t W, uint64_t Wp, uint64_t q, uint64_t twice) {
+    const uint64_t d = x + twice - y;
+    x = ref_csub_u64(x + y, twice);
+    y = ref_shoup_u64(d, W, Wp, q);
+}
+
+// the last stage with n^-1 folded in, and the reduction to [0,q); f = (iroots[1] * n^-1, its Shoup companion)
+__device__ __forceinline__ void ref_gs_last_bfly_u64(uint64_t &x, uint64_t &y, const RefInvConst &p, ulonglong2 f) {
+    const uint64_t d = x + (p.q << 1) - y;
+    x = ref_csub_u64(ref_shoup_u64(x + y, p.ninv, p.ninv_p, p.q), p.q);
+    y = ref_csub_u64(ref_shoup_u64(d, f.x, f.y, p.q), p.q);
+}
+
+// (iroots[1] * n^-1 mod q, floor(that * 2^64 / q)): the table is the caller's and on the device, so this is computed here,
+// once per CTA (a blocking read on the host would break the call's asynchrony).  The companion without a 128-bit division
+// (a bit-serial loop of microseconds, which a whole CTA would wait for): w * recip >> (k-1) is floor(w * 2^64 / q) - e with
+// e in [0,2], so the remainder w * 2^64 - estimate * q lies in [0,3q) and is its own low 64 bits; each q it holds past the
+// first is one more unit of the quotient.
+__device__ __forceinline__ ulonglong2 ref_inv_fold(const uint64_t *__restrict__ roots, const RefInvConst &p) {
+    const uint64_t w = ref_csub_u64(ref_shoup_u64(__ldg(roots + 1), p.ninv, p.ninv_p, p.q), p.q);
+    const uint32_t s = p.k - 1;
+    uint64_t wp = (__umul64hi(w, p.recip) << (64 - s)) | ((w * p.recip) >> s);
+    uint64_t r = 0 - wp * p.q;
+#pragma unroll
+    for (int i = 0; i < 2; i++)
+        if (r >= p.q) { r -= p.q; wp++; }
+    return make_ulonglong2(w, wp);
+}
+
+// a * b mod q exactly, a, b < q (HAC 14.42, b = 2, computed from the low 64 bits of the remainder)
+__device__ __forceinline__ uint64_t ref_mulmod_u64(uint64_t a, uint64_t b, const RefInvConst &p) {
+    const uint64_t lo = a * b, hi = __umul64hi(a, b);
+    const uint64_t q1 = (hi << (65 - p.k)) | (lo >> (p.k - 1));                        // x >> (k-1)  < 2^(k+1)
+    const uint64_t q3 = (__umul64hi(q1, p.mu) << (63 - p.k)) | ((q1 * p.mu) >> (p.k + 1));   // q1 * mu >> (k+1)
+    uint64_t r = lo - q3 * p.q;                                                         // x - q3*q in [0,3q)
+    r = ref_csub_u64(r, p.q);
+    return ref_csub_u64(r, p.q);
+}
+
+// GS stage J of a register pass over 2^LS coefficients: pairs x[g*2h + i], x[g*2h + i + h], h = 2^LS >> (J+1)
+template <int LS, int J, bool VEC>
+__device__ __forceinline__ void ref_istage_u64(uint64_t (&x)[1 << LS], const uint64_t *__restrict__ roots,
+                                               const uint64_t *__restrict__ precons, uint32_t tbase, uint64_t q, uint64_t twice) {
+    constexpr int half = (1 << LS) >> (J + 1);
+    uint64_t W[1 << J], Wp[1 << J];
+    ref_load_tw_u64<(1 << J), VEC>(W, Wp, roots, precons, tbase);
+#pragma unroll
+    for (int g = 0; g < (1 << J); g++)
+#pragma unroll
+        for (int i = 0; i < half; i++) ref_gs_bfly_u64(x[g * 2 * half + i], x[g * 2 * half + i + half], W[g], Wp[g], q, twice);
+}
+
+// ref_pass16_u64 run backwards: local stages J = 3 .. JLO, local stage J being stage s_first + (J - JFIRST) of the
+// forward numbering (h = 2^that groups), twiddle index h + (t_hi << J) + g
+template <bool VEC, int JFIRST, int JLO = JFIRST, int J = 3>
+__device__ __forceinline__ void ref_ipass16_u64(uint64_t (&x)[16], const uint64_t *__restrict__ roots,
+                                                const uint64_t *__restrict__ precons, uint32_t s_first, uint32_t t_hi, uint64_t q,
+                                                uint64_t twice) {
+    ref_istage_u64<4, J, VEC>(x, roots, precons, (1u << (s_first + J - JFIRST)) + (t_hi << J), q, twice);
+    if constexpr (J > JLO) ref_ipass16_u64<VEC, JFIRST, JLO, J - 1>(x, roots, precons, s_first, t_hi, q, twice);
+}
+
+// ref_u64_frame_kernel's geometry (NT = N/32 threads, lg = log2(NT) + 5 coefficients per CTA, the 17-word-per-16 image,
+// 16-coefficient register passes) with the passes in the opposite order: the frame is loaded into the image with coalesced
+// reads (times `mul` when given), the first pass works on index bits 3..0, the middle passes move upward, and the last
+// pass on the top four bits writes global memory at (k << lo) + vt, coalesced.  logn = lg: one CTA per frame, n^-1 folded
+// into the last pass, results in [0,q).  logn = lg + 1 (N = 32768, split): two CTAs per frame, each running the first 14
+// stages of its own half (the half is the top bit of every group index, as the forward's half_id); no stage before the
+// last couples the halves, so each CTA reads and writes only its own half (in place is safe) and leaves it in [0,2q) for
+// ref_u64_inv_last_stage_kernel.
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_inv_frame_kernel(const uint64_t *in, const uint64_t *mul,   // may alias out
+                                                                  uint64_t *out, const uint64_t *__restrict__ roots,
+                                                                  const uint64_t *__restrict__ precons, RefInvConst p,
+                                                                  uint32_t logn) {
+    extern __shared__ uint64_t img[];
+    __shared__ ulonglong2 fold;
+    constexpr bool VEC = AGX_U64_VECTW >= 2 || (AGX_U64_VECTW == 1 && NT >= 512);
+    constexpr uint32_t lg = (NT == 512 ? 14u : NT == 256 ? 13u : NT == 128 ? 12u : NT == 64 ? 11u : 10u);
+    constexpr uint32_t M = 1u << lg, vthreads = M >> 4;
+    const uint32_t tid = threadIdx.x, split = logn - lg;
+    if (split > 1) return;                                         // launch contract (never taken)
+    const uint32_t frame = split ? blockIdx.x >> 1 : blockIdx.x, half_id = split ? blockIdx.x & 1u : 0u;
+    const uint64_t q = p.q, twice = q << 1;
+    const size_t base = ((size_t)frame << logn) + (size_t)half_id * M;
+    if (!split && tid == 0) fold = ref_inv_fold(roots, p);         // read after the barrier that ends the load
+
+    uint64_t x[16];
+    // ---- load (and the fused pointwise product): 16 coalesced reads in flight per thread, the forward's pass-0 pattern
+    {
+        constexpr uint32_t lo = lg - 4;
+        constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = in[base + (k << lo) + vt];
+            if (mul) {
+#pragma unroll
+                for (int k = 0; k < 16; k++) x[k] = ref_mulmod_u64(x[k], mul[base + (k << lo) + vt], p);
+            }
+            uint64_t *s = img + vt + (vt >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+    }
+    __syncthreads();
+    // ---- first pass: bits 3..0, stages h = N/2 .. N/16 of this CTA's sub-transform
+#pragma unroll 1
+    for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+        uint64_t *s = img + vt * 17;
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = s[k];
+        ref_ipass16_u64<VEC, 0>(x, roots, precons, lg - 4 + split, vt + (half_id << (lg - 4)), q, twice);
+#pragma unroll
+        for (int k = 0; k < 16; k++) s[k] = x[k];
+    }
+    __syncthreads();
+    // ---- middle passes: the forward's windows (lo, jfirst) from the lowest up; the lowest may be partial
+#pragma unroll
+    for (int rem = ((int)lg - 9) % 4 + 1; rem <= (int)lg - 8; rem += 4) {
+        const uint32_t lo = rem >= 4 ? (uint32_t)rem : 4u;
+        const uint32_t jfirst = rem >= 4 ? 0u : (uint32_t)(4 - rem);
+        const uint32_t stride = (1u << lo) + (1u << (lo - 4));
+        const uint32_t s_first = lg - 4 - lo + jfirst;             // sub-transform stage of local stage jfirst
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint32_t t_lo = vt & ((1u << lo) - 1), t_hi = vt >> lo;
+            const uint32_t idx0 = (t_hi << (lo + 4)) + t_lo;
+            uint64_t *s = img + idx0 + (idx0 >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            const uint32_t sg = s_first + split, th = t_hi + (half_id << (s_first - jfirst));
+            if (jfirst == 0) ref_ipass16_u64<VEC, 0>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 1) ref_ipass16_u64<VEC, 1>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 2) ref_ipass16_u64<VEC, 2>(x, roots, precons, sg, th, q, twice);
+            else ref_ipass16_u64<VEC, 3>(x, roots, precons, sg, th, q, twice);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+        __syncthreads();
+    }
+    // ---- last pass: the top four bits, straight to global memory
+    {
+        constexpr uint32_t lo = lg - 4;
+        constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+        uint64_t *dst = out + base;
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint64_t *s = img + vt + (vt >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            if (split) {
+                ref_ipass16_u64<VEC, 0>(x, roots, precons, 1, half_id, q, twice);
+            } else {
+                ref_ipass16_u64<VEC, 0, 1>(x, roots, precons, 0, 0, q, twice);
+                const ulonglong2 f = fold;
+#pragma unroll
+                for (int i = 0; i < 8; i++) ref_gs_last_bfly_u64(x[i], x[i + 8], p, f);
+            }
+#pragma unroll
+            for (int k = 0; k < 16; k++) dst[(k << lo) + vt] = x[k];
+        }
+    }
+}
+
+// N = 32768: the last stage (h = 1, pairs i and i + N/2) with n^-1 folded in and the reduction to [0,q), over frames
+// whose halves ref_u64_inv_frame_kernel left in [0,2q).  Grid-stride, two pairs per thread and step (16-byte accesses).
+__global__ void __launch_bounds__(256) ref_u64_inv_last_stage_kernel(uint64_t *data, const uint64_t *__restrict__ roots,
+                                                                     RefInvConst p, uint32_t logn, size_t frames) {
+    __shared__ ulonglong2 fold;
+    if (threadIdx.x == 0) fold = ref_inv_fold(roots, p);
+    __syncthreads();
+    const ulonglong2 f = fold;
+    const uint32_t hlog = logn - 2;                                // 2-pair units per half frame
+    const size_t units = frames << hlog;
+    for (size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x; u < units; u += (size_t)gridDim.x * blockDim.x) {
+        const size_t i = ((u >> hlog) << logn) + ((u & ((1u << hlog) - 1)) << 1);
+        ulonglong2 *lo = reinterpret_cast<ulonglong2 *>(data + i), *hi = reinterpret_cast<ulonglong2 *>(data + i + (1u << (logn - 1)));
+        const ulonglong2 a = *lo, b = *hi;
+        uint64_t u0 = a.x, u1 = a.y, v0 = b.x, v1 = b.y;
+        ref_gs_last_bfly_u64(u0, v0, p, f);
+        ref_gs_last_bfly_u64(u1, v1, p, f);
+        *lo = make_ulonglong2(u0, u1);
+        *hi = make_ulonglong2(v0, v1);
+    }
+}
+
+// N < 1024: plain radix-2 GS, one CTA per frame, the frame in shared memory (in the manner of ref_fwd_u64_kernel)
+__global__ void __launch_bounds__(256) ref_inv_u64_kernel(const uint64_t *in, const uint64_t *mul, uint64_t *out,
+                                                          const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
+                                                          RefInvConst p, uint32_t logn) {
+    __shared__ uint64_t X[512];
+    __shared__ ulonglong2 fold;
+    const uint32_t N = 1u << logn;
+    const size_t base = (size_t)blockIdx.x * N;
+    const uint64_t q = p.q, twice = q << 1;
+    if (threadIdx.x == 0) fold = ref_inv_fold(roots, p);
+    for (uint32_t i = threadIdx.x; i < N; i += blockDim.x)
+        X[i] = mul ? ref_mulmod_u64(in[base + i], mul[base + i], p) : in[base + i];
+    __syncthreads();
+    for (uint32_t h = N >> 1, tlog = 0; h >= 1; h >>= 1, tlog++) {        // butterfly distance 2^tlog
+        for (uint32_t bf = threadIdx.x; bf < N / 2; bf += blockDim.x) {
+            const uint32_t j = bf >> tlog, a0 = (j << (tlog + 1)) + (bf & ((1u << tlog) - 1)), a1 = a0 + (1u << tlog);
+            uint64_t u = X[a0], v = X[a1];
+            if (h == 1) ref_gs_last_bfly_u64(u, v, p, fold);
+            else ref_gs_bfly_u64(u, v, __ldg(roots + h + j), __ldg(precons + h + j), q, twice);
+            X[a0] = u; X[a1] = v;
+        }
+        __syncthreads();
+    }
+    for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) out[base + i] = X[i];
+}
+
 // ------------------------------------------------------------------------------------- twiddle tables on device
 // The step before the path: the reference fills its root / precon buffers on the host (main.cpp:46-55) and the loader
 // broadcasts them (ntt.cpp:544-571).  Here one thread per (limb, direction, k) computes

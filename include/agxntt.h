@@ -171,6 +171,39 @@ int agx_ref_fwd_dev(agx_ctx *ctx, uint32_t N, const uint64_t *d_in, const uint64
                     uint64_t modulus, const uint64_t *d_twiddles, const uint64_t *d_precon_twiddles, uint32_t numFrames,
                     void *stream);
 
+/* ---- u64 inverse transform and negacyclic product on DEVICE pointers (no reference counterpart: the reference has
+ * only the forward, SURVEY.md s.0).  Conventions of agx_ref_fwd_dev: frames [numFrames][N], N in {2^2 .. 2^15}, every
+ * device pointer 16-byte aligned, asynchronous on `stream`, the caller's tables in the reference's order (ntt.cpp:298-300)
+ * and not checked per call.  Unlike the forward, the modulus must be odd and 3 <= q < 2^62 (AGX_E_INVALID otherwise):
+ * there is no reference behaviour to reproduce above 2^62, and the lazy range [0,4q) must fit 64 bits.
+ * numFrames == 0 returns AGX_OK and launches nothing.  The results are the inverse NTT / the product exactly when the
+ * tables are the Shoup pairs of psi (d_twiddles, d_precon_twiddles: agx_ref_fwd_dev's) and of psi^-1:
+ * d_inv_twiddles[k] = psi^-bitrev(k) mod q, d_inv_precon_twiddles[k] = floor(d_inv_twiddles[k] * 2^64 / q)
+ * (the forward table's order built from psi^-1; entry 0 unused).
+ * Launches counted by agx_launch_count, out of place (N = 32768 in parentheses; an in-place forward there takes the
+ * multi-launch pass kernels, see agx_ref_fwd_dev): agx_ref_inv_dev 1 (2), agx_ref_polymul_by_spectrum_dev 2 (3),
+ * agx_ref_polymul_dev 3 (4). */
+
+/* x = INTT(X): bit-reversed in (inputs < 2q), natural out in [0,q), n^-1 folded in (Gentleman-Sande, the mirror of
+ * ntt.cpp:146-159, 292-300).  d_out == d_in (in place) or disjoint. */
+int agx_ref_inv_dev(agx_ctx *ctx, uint32_t N, const uint64_t *d_in, uint64_t *d_out, uint64_t modulus,
+                    const uint64_t *d_inv_twiddles, const uint64_t *d_inv_precon_twiddles, uint32_t numFrames,
+                    void *stream);
+/* c = a * b mod (X^N + 1, q) per frame = INTT(NTT(a) .* NTT(b)); operands reduced (< q), results in [0,q).  c may alias
+ * a and/or b, and a may equal b (squaring); any other overlap is not allowed.  NTT(b) goes to a stream-ordered scratch
+ * buffer (cudaMallocAsync on `stream`) unless a == b. */
+int agx_ref_polymul_dev(agx_ctx *ctx, uint32_t N, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b,
+                        uint64_t modulus, const uint64_t *d_twiddles, const uint64_t *d_precon_twiddles,
+                        const uint64_t *d_inv_twiddles, const uint64_t *d_inv_precon_twiddles, uint32_t numFrames,
+                        void *stream);
+/* c = INTT(NTT(a) .* b_hat) with b_hat = agx_ref_fwd_dev(b) (reduced, bit-reversed order): the product when one operand
+ * is kept in evaluation form.  c may alias a and/or b_hat (c == b_hat costs a stream-ordered scratch buffer for NTT(a)).
+ * Equals agx_ref_polymul_dev(c, a, b) bit for bit. */
+int agx_ref_polymul_by_spectrum_dev(agx_ctx *ctx, uint32_t N, uint64_t *d_c, const uint64_t *d_a,
+                                    const uint64_t *d_b_hat, uint64_t modulus, const uint64_t *d_twiddles,
+                                    const uint64_t *d_precon_twiddles, const uint64_t *d_inv_twiddles,
+                                    const uint64_t *d_inv_precon_twiddles, uint32_t numFrames, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

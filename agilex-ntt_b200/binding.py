@@ -27,6 +27,10 @@ class _Parms(C.Structure):
     _fields_ = [("n", C.c_uint32), ("logn", C.c_uint32), ("nlimbs", C.c_uint32), ("q", _u32p)]
 
 
+class _Parms64(C.Structure):
+    _fields_ = [("n", C.c_uint32), ("logn", C.c_uint32), ("nlimbs", C.c_uint32), ("q", _u64p)]
+
+
 def _load() -> C.CDLL:
     path = os.environ.get("AGX_LIB", _build.LIB)   # AGX_LIB: experiment builds of the same ABI (kernel variants)
     if not os.path.exists(path):
@@ -67,6 +71,14 @@ def _load() -> C.CDLL:
         "agx_ref_inv_dev": [vp, C.c_uint32, vp, vp, C.c_uint64, vp, vp, C.c_uint32, vp],
         "agx_ref_polymul_dev": [vp, C.c_uint32, vp, vp, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint32, vp],
         "agx_ref_polymul_by_spectrum_dev": [vp, C.c_uint32, vp, vp, vp, C.c_uint64, vp, vp, vp, vp, C.c_uint32, vp],
+        "agx_create64": [C.POINTER(vp), C.POINTER(_Parms64), _u64p, C.c_int],
+        "agx_get_psi64": [vp, C.c_uint32, _u64p],
+        "agx_get_tables64": [vp, C.c_uint32, C.c_int, _u64p, _u64p],
+        "agx_ntt64_fwd": [vp, vp, C.c_size_t, vp],
+        "agx_ntt64_inv": [vp, vp, C.c_size_t, vp],
+        "agx_polymul64": [vp, vp, vp, vp, C.c_size_t, vp],
+        "agx_polymul64_by_spectrum": [vp, vp, vp, vp, C.c_size_t, vp],
+        "agx_elementwise64": [vp, C.c_int, vp, vp, vp, C.c_size_t, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -84,7 +96,8 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_ref_polymul_by_spectrum_dev agx_measure_butterfly_peak agx_destroy agx_get_psi agx_get_tables agx_ntt_fwd agx_ntt_inv agx_polymul agx_polymul_by_spectrum agx_polymul_by_spectrum_host agx_elementwise agx_bitrev "
            "agx_ntt_fwd_host agx_ntt_inv_host agx_polymul_host agx_host_alloc agx_host_free agx_fill_synthetic "
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
-           "agx_variant").split()
+           "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
+           "agx_polymul64_by_spectrum agx_elementwise64").split()
 
 _lib = None
 
@@ -111,6 +124,15 @@ def _dev_ptr(t) -> int:
         return t
     if not t.is_cuda or not t.is_contiguous() or t.element_size() != 4:
         raise ValueError("need a contiguous CUDA tensor of a 4-byte integer dtype")
+    return t.data_ptr()
+
+
+def _dev_ptr8(t) -> int:
+    """Device pointer of a torch CUDA tensor of an 8-byte integer dtype (int64, uint64) or a raw int address."""
+    if isinstance(t, int):
+        return t
+    if not t.is_cuda or not t.is_contiguous() or t.element_size() != 8 or t.is_floating_point() or t.is_complex():
+        raise ValueError("need a contiguous CUDA tensor of an 8-byte integer dtype")
     return t.data_ptr()
 
 
@@ -294,6 +316,100 @@ class Context:
     def polymul_by_spectrum_host(self, c, a, b_hat, B=None):
         _ck(lib().agx_polymul_by_spectrum_host(self._h, self._host_ptr(c), self._host_ptr(a), self._host_ptr(b_hat),
                                                self._host_batch(a, B)), "agx_polymul_by_spectrum_host")
+        return c
+
+
+class Context64:
+    """One (n, primes) u64 parameter set bound to one GPU: L primes of up to 62 bits (q = 1 mod 2n), the device tables,
+    and batched [B][L][n] transforms and products over them (agx_create64).  Data are contiguous CUDA tensors of int64 or
+    uint64 words; every call works in place on them, on the current torch stream unless `stream` is given."""
+
+    EW = Context.EW
+
+    def __init__(self, n: int, primes, device: int = 0, psi=None):
+        """psi: the caller's primitive 2n-th root per limb; None = the minimal root of each prime."""
+        self._h = C.c_void_p()
+        self.n = int(n)
+        self.logn = self.n.bit_length() - 1
+        self.primes = [int(q) for q in primes]
+        self.L = len(self.primes)
+        self.device = device
+        self._q = (C.c_uint64 * max(self.L, 1))(*self.primes)
+        p = _Parms64(self.n, self.logn, self.L, C.cast(self._q, _u64p))
+        arr = None
+        if psi is not None:
+            psi = [int(v) for v in psi]
+            if len(psi) != self.L:
+                raise ValueError("need one psi per limb")
+            arr = C.cast((C.c_uint64 * self.L)(*psi), _u64p)
+        _ck(lib().agx_create64(C.byref(self._h), C.byref(p), arr, device), "agx_create64")
+
+    def close(self):
+        if getattr(self, "_h", None) and self._h.value:
+            lib().agx_destroy(self._h)
+            self._h = C.c_void_p()
+
+    __del__ = close
+
+    def psi(self, limb: int = 0) -> int:
+        v = C.c_uint64()
+        _ck(lib().agx_get_psi64(self._h, limb, C.byref(v)), "agx_get_psi64")
+        return v.value
+
+    def tables(self, limb: int = 0, inverse: bool = False):
+        """(roots, precons) of one limb as uint64 arrays in the reference's order: what agx_ref_fwd_dev / inv_dev take."""
+        r = np.empty(self.n, dtype=np.uint64)
+        p = np.empty(self.n, dtype=np.uint64)
+        _ck(lib().agx_get_tables64(self._h, limb, int(inverse), r.ctypes.data_as(_u64p), p.ctypes.data_as(_u64p)),
+            "agx_get_tables64")
+        return r, p
+
+    def launch_count(self) -> int:
+        v = C.c_uint64()
+        _ck(lib().agx_launch_count(self._h, C.byref(v)), "agx_launch_count")
+        return v.value
+
+    def _batch(self, t) -> int:
+        words = t.numel()
+        if words % (self.L * self.n):
+            raise ValueError("tensor is not a whole number of [L][n] polynomials")
+        return words // (self.L * self.n)
+
+    def _batch3(self, c, a, b) -> int:
+        B = self._batch(a)
+        if self._batch(b) != B or self._batch(c) != B:
+            raise ValueError("shape mismatch")
+        return B
+
+    def fwd(self, t, stream=None):
+        """Forward NTT of every limb (inputs < 4q), natural in, bit-reversed out, results in [0,q)."""
+        _ck(lib().agx_ntt64_fwd(self._h, _dev_ptr8(t), self._batch(t), _stream_ptr(stream)), "agx_ntt64_fwd")
+        return t
+
+    def inv(self, t, stream=None):
+        """Inverse NTT of every limb (inputs < 2q), bit-reversed in, natural out, n^-1 folded in."""
+        _ck(lib().agx_ntt64_inv(self._h, _dev_ptr8(t), self._batch(t), _stream_ptr(stream)), "agx_ntt64_inv")
+        return t
+
+    def polymul(self, c, a, b, stream=None):
+        """c = a * b mod (X^n + 1, q_limb) for every limb (reduced operands; c may alias a and/or b)."""
+        B = self._batch3(c, a, b)
+        _ck(lib().agx_polymul64(self._h, _dev_ptr8(c), _dev_ptr8(a), _dev_ptr8(b), B, _stream_ptr(stream)),
+            "agx_polymul64")
+        return c
+
+    def polymul_by_spectrum(self, c, a, b_hat, stream=None):
+        """c = INTT(NTT(a) .* b_hat) with b_hat = fwd(b): the product when one operand is kept in evaluation form."""
+        B = self._batch3(c, a, b_hat)
+        _ck(lib().agx_polymul64_by_spectrum(self._h, _dev_ptr8(c), _dev_ptr8(a), _dev_ptr8(b_hat), B,
+                                            _stream_ptr(stream)), "agx_polymul64_by_spectrum")
+        return c
+
+    def elementwise(self, op: str, c, a, b, stream=None):
+        """c = a + b | a - b | a * b | c + a * b, modulo each limb's prime (operands reduced)."""
+        B = self._batch3(c, a, b)
+        _ck(lib().agx_elementwise64(self._h, self.EW[op], _dev_ptr8(c), _dev_ptr8(a), _dev_ptr8(b), B,
+                                    _stream_ptr(stream)), "agx_elementwise64")
         return c
 
 

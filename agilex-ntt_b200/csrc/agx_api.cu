@@ -97,6 +97,11 @@ struct agx_ctx {
     struct MapSlot { const void *ptr = nullptr; size_t T = 0; int kind = 0; CUtensorMap map; };
     MapSlot maps[8];
     unsigned map_next = 0;
+    // u64 parameter set (agx_create64); a context holds either this or the u32 one
+    bool has_parms64 = false;
+    std::vector<uint64_t> q64, psi64;
+    uint64_t *d_tab64 = nullptr;                           // [4][L][n]: roots, companions; forward then inverse
+    RnsLimb64 *d_lc64 = nullptr;                           // per-limb modulus constants
     HostPipe pipe;
     RefState ref;
     CopyCrew *crew_in = nullptr, *crew_out = nullptr;      // created with the first pageable call
@@ -725,8 +730,8 @@ int ref_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64_t *
 // The inverse transform of `frames` frames [frames][N] (bit-reversed in, natural out, results in [0,q)), with the
 // pointwise product by d_mul fused into its load when d_mul is not null.  d_out may equal d_in and/or d_mul.
 // Odd modulus, 3 <= q < 2^62 (checked by the callers).
-int ref_inv_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64_t *d_mul, uint64_t *d_out,
-                   const uint64_t *d_itw, const uint64_t *d_ipre, uint64_t q, size_t frames, cudaStream_t st) {
+// The inverse's constants of an odd modulus 3 <= q < 2^62 at size 2^logn.
+RefInvConst ref_inv_const(uint64_t q, uint32_t logn) {
     typedef unsigned __int128 u128;
     RefInvConst p{};
     p.q = q;
@@ -737,6 +742,12 @@ int ref_inv_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64
     p.k = 64 - (uint32_t)__builtin_clzll(q);
     p.mu = (uint64_t)(((u128)1 << (2 * p.k)) / q);
     p.recip = (uint64_t)(((u128)1 << (63 + p.k)) / q);
+    return p;
+}
+
+int ref_inv_launch(agx_ctx *c, uint32_t logn, const uint64_t *d_in, const uint64_t *d_mul, uint64_t *d_out,
+                   const uint64_t *d_itw, const uint64_t *d_ipre, uint64_t q, size_t frames, cudaStream_t st) {
+    const RefInvConst p = ref_inv_const(q, logn);
     if (logn >= 10) {
         // one CTA per frame up to N = 16384; two per frame and a streaming last stage at N = 32768
         const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
@@ -775,6 +786,77 @@ int ref_inv_check(agx_ctx *c, uint32_t N, std::initializer_list<const void *> pt
     uint32_t l = 0;
     while ((1u << l) < N) l++;
     *logn = l;
+    return AGX_OK;
+}
+
+// ------------------------------------------------------------------------------------- u64 RNS batches
+
+// The library's tables of the u64 parameter set: forward roots, forward companions, inverse roots, inverse companions.
+const uint64_t *tab64(const agx_ctx *c, int which) { return c->d_tab64 + (size_t)which * c->L * c->n; }
+
+// Forward transform of T = B * L frames [T][n] (frame f = limb f % L), in -> out (in == out or disjoint): one launch.
+// N = 32768 runs the 2-CTA cluster kernel, which is safe in place.
+int rns_fwd_launch(agx_ctx *c, const uint64_t *in, uint64_t *out, size_t T, cudaStream_t st) {
+    const uint32_t logn = c->logn, L = c->L;
+    const uint64_t *tw = tab64(c, 0), *pre = tab64(c, 1);
+    const RnsLimb64 *lc = c->d_lc64;
+    const unsigned grid = (unsigned)T;
+    const size_t smem = logn >= 10 ? ((size_t)17 << (std::min(logn, 14u) - 4)) * 8 : 0;
+    switch (logn) {
+        case 15: ref_u64_rns_frame_pair_kernel<<<2 * grid, 512, smem, st>>>(in, out, tw, pre, lc, L); break;
+        case 14: ref_u64_rns_frame_kernel<512><<<grid, 512, smem, st>>>(in, out, tw, pre, lc, L, logn); break;
+        case 13: ref_u64_rns_frame_kernel<256><<<grid, 256, smem, st>>>(in, out, tw, pre, lc, L, logn); break;
+        case 12: ref_u64_rns_frame_kernel<128><<<grid, 128, smem, st>>>(in, out, tw, pre, lc, L, logn); break;
+        case 11: ref_u64_rns_frame_kernel<64><<<grid, 64, smem, st>>>(in, out, tw, pre, lc, L, logn); break;
+        case 10: ref_u64_rns_frame_kernel<32><<<grid, 32, smem, st>>>(in, out, tw, pre, lc, L, logn); break;
+        default: {
+            const uint32_t N = 1u << logn;
+            ref_fwd_u64_rns_kernel<<<grid, N / 2 < 32 ? 32 : N / 2, (size_t)N * 8, st>>>(in, out, tw, pre, lc, L, logn);
+        }
+    }
+    c->launches++;
+    return (int)cudaGetLastError();
+}
+
+// Inverse of T frames, times d_mul on load when not null (ref_inv_launch's geometry): one launch, two at N = 32768.
+int rns_inv_launch(agx_ctx *c, const uint64_t *in, const uint64_t *mul, uint64_t *out, size_t T, cudaStream_t st) {
+    const uint32_t logn = c->logn, L = c->L;
+    const uint64_t *itw = tab64(c, 2), *ipre = tab64(c, 3);
+    const RnsLimb64 *lc = c->d_lc64;
+    if (logn >= 10) {
+        const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+        const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+        const unsigned grid = (unsigned)(T << split);
+        switch (lg) {
+            case 14: ref_u64_rns_inv_frame_kernel<512><<<grid, 512, smem, st>>>(in, mul, out, itw, ipre, lc, L, logn); break;
+            case 13: ref_u64_rns_inv_frame_kernel<256><<<grid, 256, smem, st>>>(in, mul, out, itw, ipre, lc, L, logn); break;
+            case 12: ref_u64_rns_inv_frame_kernel<128><<<grid, 128, smem, st>>>(in, mul, out, itw, ipre, lc, L, logn); break;
+            case 11: ref_u64_rns_inv_frame_kernel<64><<<grid, 64, smem, st>>>(in, mul, out, itw, ipre, lc, L, logn); break;
+            default: ref_u64_rns_inv_frame_kernel<32><<<grid, 32, smem, st>>>(in, mul, out, itw, ipre, lc, L, logn); break;
+        }
+        c->launches++;
+        if (split) {
+            const size_t units = T << (logn - 2);
+            const unsigned blocks = (unsigned)std::min<size_t>((units + 255) / 256, (size_t)c->sms * 8);
+            ref_u64_rns_inv_last_stage_kernel<<<blocks, 256, 0, st>>>(out, lc, L, logn, T);
+            c->launches++;
+        }
+    } else {
+        const uint32_t N = 1u << logn;
+        ref_inv_u64_rns_kernel<<<(unsigned)T, N / 2 < 32 ? 32 : N / 2, 0, st>>>(in, mul, out, itw, ipre, lc, L, logn);
+        c->launches++;
+    }
+    return (int)cudaGetLastError();
+}
+
+// Argument checks of the u64 batched calls: a u64 context, 16-byte aligned operands, B * L frames within a grid.
+// *T = B * L.
+int check_dev_call64(const agx_ctx *c, std::initializer_list<const void *> ptrs, size_t B, size_t *T) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : ptrs)
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    if (B > 0x7fffffffull / c->L) return AGX_E_INVALID;
+    *T = B * c->L;
     return AGX_OK;
 }
 
@@ -911,20 +993,9 @@ int ref_flush(agx_ctx *c) {
     return rc ? fail(rc) : AGX_OK;
 }
 
-}  // namespace
-
-// ================================================================================================== C ABI
-
-extern "C" {
-
-int agx_create(agx_ctx **out, const agx_parms *parms, int device) { return agx_create_tables(out, parms, nullptr, device); }
-
-int agx_create_tables(agx_ctx **out, const agx_parms *parms, const uint32_t *psi, int device) {
-    if (!out) return AGX_E_INVALID;
-    *out = nullptr;
-    if (psi && !parms) return AGX_E_INVALID;
-    DeviceGuard guard__(device);
-    if (guard__.error()) return guard__.error();
+// A context without a parameter set on `device`, which the caller has made current: the driver's tensor-map encoder, and
+// the dynamic shared-memory opt-in of every kernel that takes more than 48 KB.
+int ctx_new(agx_ctx **out, int device) {
     CK(cudaFree(0));
     agx_ctx *c = new (std::nothrow) agx_ctx();
     if (!c) return AGX_E_NOMEM;
@@ -959,6 +1030,26 @@ int agx_create_tables(agx_ctx **out, const agx_parms *parms, const uint32_t *psi
         if (e == cudaSuccess) e = cudaFuncSetAttribute(bitrev_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 << 10);
         if (e != cudaSuccess) { delete c; return (int)e; }
     }
+    *out = c;
+    return AGX_OK;
+}
+
+}  // namespace
+
+// ================================================================================================== C ABI
+
+extern "C" {
+
+int agx_create(agx_ctx **out, const agx_parms *parms, int device) { return agx_create_tables(out, parms, nullptr, device); }
+
+int agx_create_tables(agx_ctx **out, const agx_parms *parms, const uint32_t *psi, int device) {
+    if (!out) return AGX_E_INVALID;
+    *out = nullptr;
+    if (psi && !parms) return AGX_E_INVALID;
+    DeviceGuard guard__(device);
+    if (guard__.error()) return guard__.error();
+    agx_ctx *c = nullptr;
+    if (const int rc = ctx_new(&c, device)) return rc;
     if (const char *e = getenv("AGX_CARVEOUT")) {      // A/B knob: shared-memory carve-out (percent) of the n = 4096 kernels
         const int pct = atoi(e);
         cudaFuncSetAttribute(ntt_fwd_loop_kernel<12, 6, false, true, true>, cudaFuncAttributePreferredSharedMemoryCarveout, pct);
@@ -1009,6 +1100,7 @@ int agx_destroy(agx_ctx *c) {
         cudaFree(c->d_tw_fwd); cudaFree(c->d_tw_inv); cudaFree(c->d_nat_fwd); cudaFree(c->d_nat_inv);
         cudaFree(c->d_twc_fwd); cudaFree(c->d_twc_inv);
         cudaFree(c->d_lc); cudaFree(c->d_sum);
+        cudaFree(c->d_tab64); cudaFree(c->d_lc64);
 #if AGX_WITH_R16
         cudaFree(c->d_tw16_fwd); cudaFree(c->d_tw16_inv); cudaFree(c->d_u16_fwd); cudaFree(c->d_u16_inv);
 #endif
@@ -1320,6 +1412,153 @@ int agx_ref_polymul_by_spectrum_dev(agx_ctx *c, uint32_t N, uint64_t *d_c, const
     return rc;
 }
 
+// ------------------------------------------------------------------------------------------------ u64 RNS batches
+
+int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, int device) {
+    typedef unsigned __int128 u128;
+    if (!out) return AGX_E_INVALID;
+    *out = nullptr;
+    if (!parms || !parms->q || parms->nlimbs == 0 || parms->nlimbs > 64 || parms->logn < 2 || parms->logn > 15 ||
+        parms->n != (1u << parms->logn))
+        return AGX_E_INVALID;
+    const uint32_t n = parms->n, logn = parms->logn, L = parms->nlimbs;
+    std::vector<RnsLimb64> lc(L);
+    for (uint32_t l = 0; l < L; l++) {
+        const uint64_t q = parms->q[l];
+        uint64_t root = minimal_psi_u64(n, q);                         // also validates q (prime, < 2^62, = 1 mod 2n)
+        if (!root) return AGX_E_INVALID;
+        if (psi) {                                                     // the caller's root: must be a primitive 2n-th root
+            root = psi[l];
+            if (root == 0 || root >= q || powmod_u64(root, n, q) != q - 1) return AGX_E_INVALID;
+        }
+        RnsLimb64 &x = lc[l];
+        x.p = ref_inv_const(q, logn);
+        x.psi = root;
+        x.psi_inv = powmod_u64(root, q - 2, q);
+        // iroots[1] = psi^-bitrev(1) = psi^-(n/2), with n^-1 folded in (what ref_inv_fold computes from a caller's table)
+        const uint64_t w = mulmod_u64(powmod_u64(x.psi_inv, n / 2, q), x.p.ninv, q);
+        x.fold = make_ulonglong2(w, (uint64_t)(((u128)w << 64) / q));
+    }
+    DeviceGuard guard__(device);
+    if (guard__.error()) return guard__.error();
+    agx_ctx *c = nullptr;
+    if (const int rc = ctx_new(&c, device)) return rc;
+    c->has_parms64 = true;
+    c->n = n; c->logn = logn; c->L = L;
+    c->q64.assign(parms->q, parms->q + L);
+    for (const RnsLimb64 &x : lc) c->psi64.push_back(x.psi);
+    const int frame_smem = 17 * 1024 * 8;                              // N = 16384 image: 136 KB
+    cudaError_t e = cudaFuncSetAttribute(ref_u64_rns_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_frame_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    const size_t entries = (size_t)L * n;
+    if (e == cudaSuccess) e = cudaMalloc(&c->d_tab64, 4 * entries * sizeof(uint64_t));
+    if (e == cudaSuccess) e = cudaMalloc(&c->d_lc64, L * sizeof(RnsLimb64));
+    if (e == cudaSuccess) e = cudaMemcpy(c->d_lc64, lc.data(), L * sizeof(RnsLimb64), cudaMemcpyHostToDevice);
+    if (e == cudaSuccess) {
+        const size_t total = 2 * entries;
+        gen_tables64_kernel<<<(unsigned)((total + 255) / 256), 256>>>(c->d_tab64, c->d_lc64, L, logn);
+        c->launches++;
+        e = cudaGetLastError();
+        if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    }
+    if (e != cudaSuccess) { agx_destroy(c); return (int)e; }
+    *out = c;
+    return AGX_OK;
+}
+
+int agx_get_psi64(const agx_ctx *c, uint32_t limb, uint64_t *psi) {
+    if (!c || !c->has_parms64 || limb >= c->L || !psi) return AGX_E_INVALID;
+    *psi = c->psi64[limb];
+    return AGX_OK;
+}
+
+int agx_get_tables64(const agx_ctx *c, uint32_t limb, int inverse, uint64_t *roots, uint64_t *precons) {
+    if (!c || !c->has_parms64 || limb >= c->L || !roots || !precons) return AGX_E_INVALID;
+    AGX_ON_DEVICE(c);
+    const size_t bytes = (size_t)c->n * sizeof(uint64_t), off = (size_t)limb * c->n;
+    CK(cudaMemcpy(roots, tab64(c, inverse ? 2 : 0) + off, bytes, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(precons, tab64(c, inverse ? 3 : 1) + off, bytes, cudaMemcpyDeviceToHost));
+    return AGX_OK;
+}
+
+int agx_ntt64_fwd(agx_ctx *c, uint64_t *d, size_t B, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d}, B, &T)) return rc;
+    if (T == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    return rns_fwd_launch(c, d, d, T, (cudaStream_t)stream);
+}
+
+int agx_ntt64_inv(agx_ctx *c, uint64_t *d, size_t B, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d}, B, &T)) return rc;
+    if (T == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    return rns_inv_launch(c, d, nullptr, d, T, (cudaStream_t)stream);
+}
+
+int agx_polymul64(agx_ctx *c, uint64_t *dc, const uint64_t *da, const uint64_t *db, size_t B, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {dc, da, db}, B, &T)) return rc;
+    if (T == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (dc == db && dc != da) std::swap(da, db);                   // the product commutes: c == a from here on
+    // c = NTT(a); scratch = NTT(b) unless squaring; c = INTT(c .* (scratch or c))  (agx_ref_polymul_dev's sequence)
+    uint64_t *tmp = nullptr;
+    int rc = rns_fwd_launch(c, da, dc, T, st);
+    if (!rc && da != db) {
+        rc = (int)cudaMallocAsync(&tmp, T * c->n * sizeof(uint64_t), st);
+        if (!rc) rc = rns_fwd_launch(c, db, tmp, T, st);
+    }
+    if (!rc) rc = rns_inv_launch(c, dc, tmp ? tmp : dc, dc, T, st);
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
+int agx_polymul64_by_spectrum(agx_ctx *c, uint64_t *dc, const uint64_t *da, const uint64_t *db_hat, size_t B, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {dc, da, db_hat}, B, &T)) return rc;
+    if (T == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    // NTT(a) goes to c unless c holds b_hat, which the inverse still has to read: then to a scratch buffer
+    uint64_t *tmp = nullptr, *spec = dc;
+    int rc = AGX_OK;
+    if (dc == db_hat) {
+        rc = (int)cudaMallocAsync(&tmp, T * c->n * sizeof(uint64_t), st);
+        spec = tmp;
+    }
+    if (!rc) rc = rns_fwd_launch(c, da, spec, T, st);
+    if (!rc) rc = rns_inv_launch(c, spec, db_hat, dc, T, st);
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }
+    return rc;
+}
+
+int agx_elementwise64(agx_ctx *c, int op, uint64_t *dc, const uint64_t *da, const uint64_t *db, size_t B, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {dc, da, db}, B, &T)) return rc;
+    if (op < 0 || op > 3) return AGX_E_INVALID;
+    if (T == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const size_t total2 = T * c->n / 2;
+    const unsigned blocks = (unsigned)std::min<size_t>((total2 + 255) / 256, (size_t)c->sms * 16);
+    const cudaStream_t s = (cudaStream_t)stream;
+    ulonglong2 *c2 = reinterpret_cast<ulonglong2 *>(dc);
+    const ulonglong2 *a2 = reinterpret_cast<const ulonglong2 *>(da), *b2 = reinterpret_cast<const ulonglong2 *>(db);
+    switch (op) {
+        case EW_ADD: elementwise64_kernel<EW_ADD><<<blocks, 256, 0, s>>>(c2, a2, b2, c->d_lc64, c->L, c->logn, total2); break;
+        case EW_SUB: elementwise64_kernel<EW_SUB><<<blocks, 256, 0, s>>>(c2, a2, b2, c->d_lc64, c->L, c->logn, total2); break;
+        case EW_MUL: elementwise64_kernel<EW_MUL><<<blocks, 256, 0, s>>>(c2, a2, b2, c->d_lc64, c->L, c->logn, total2); break;
+        default:     elementwise64_kernel<EW_MAC><<<blocks, 256, 0, s>>>(c2, a2, b2, c->d_lc64, c->L, c->logn, total2); break;
+    }
+    c->launches++;
+    return (int)cudaGetLastError();
+}
+
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {
     if (!c || !per_clk_per_sm || kind < 0 || kind > 6) return AGX_E_INVALID;
     if (threads_per_sm < 128 || threads_per_sm > 1024 || threads_per_sm % 128) return AGX_E_INVALID;
@@ -1391,7 +1630,8 @@ int agx_launch_count(const agx_ctx *c, uint64_t *count) {
 
 int agx_variant(const agx_ctx *c, char *buf, size_t buflen) {
     if (!c || !buf || !buflen) return AGX_E_INVALID;
-    if (!c->has_parms) snprintf(buf, buflen, "ref_u64");
+    if (c->has_parms64) snprintf(buf, buflen, "u64_rns<%u>", c->logn);
+    else if (!c->has_parms) snprintf(buf, buflen, "ref_u64");
     else if (c->r16) snprintf(buf, buflen, "ntt_r16<%u>", c->logn);
     else if (c->le) snprintf(buf, buflen, "ntt2p<%u,%d>", c->logn, c->le);
     else if (c->big) snprintf(buf, buflen, "ntt_big<%u>", c->logn);

@@ -901,6 +901,48 @@ __global__ void __launch_bounds__(256) elementwise_kernel(uint4 *c4, const uint4
 // wrap-around mod 2^64 when the tables are not Shoup pairs (main.cpp:49-55 feeds such data).  One CTA per frame
 // (ntt.cpp:579-595 frame layout: low half from `in`, high half from `in2`); work array in dynamic smem when
 // N*8 bytes fits, else in the output buffer itself.
+// ref_fwd_u64_body is this kernel's body for the per-limb variant (ref_fwd_u64_rns_kernel).  ref_fwd_u64_kernel keeps its
+// own copy: routed through the shared body it compiles to different SASS, and the single-modulus kernels stay as they were.
+__device__ __forceinline__ void ref_fwd_u64_body(const uint64_t *__restrict__ in, const uint64_t *__restrict__ in2,
+                                                 uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
+                                                 const uint64_t *__restrict__ precons, uint64_t q, uint32_t logn, int use_smem,
+                                                 uint32_t frame) {
+    extern __shared__ uint64_t s64[];
+    const uint32_t N = 1u << logn;
+    const size_t base = (size_t)frame * N;
+    uint64_t *X = use_smem ? s64 : out + base;
+    for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) X[i] = i < N / 2 ? in[base + i] : in2[base + i];
+    __syncthreads();
+    const uint64_t twice = q << 1;
+    uint32_t tlog = logn - 1;
+    for (uint32_t m = 1; m < N; m <<= 1, tlog--) {
+        const bool last = (m == N / 2);
+        for (uint32_t bf = threadIdx.x; bf < N / 2; bf += blockDim.x) {
+            const uint32_t i = bf >> tlog, j = bf & ((1u << tlog) - 1);
+            const uint32_t a0 = (i << (tlog + 1)) + j, a1 = a0 + (1u << tlog);
+            const uint64_t W = roots[m + i], Wp = precons[m + i];
+            uint64_t tx = X[a0];
+            if (tx >= twice) tx -= twice;
+            const uint64_t a = X[a1];
+            const uint64_t c1 = __umul64hi(a, Wp);
+            const uint64_t Q = W * a - c1 * q;
+            uint64_t o0 = tx + Q, o1 = tx + twice - Q;
+            if (last) {
+                if (o0 >= twice) o0 -= twice;
+                if (o0 >= q) o0 -= q;
+                if (o1 >= twice) o1 -= twice;
+                if (o1 >= q) o1 -= q;
+            }
+            X[a0] = o0; X[a1] = o1;
+        }
+        __syncthreads();
+    }
+    if (use_smem)
+        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) out[base + i] = X[i];
+}
+
+// TWIN: ref_fwd_u64_body is a copy of this kernel for the per-limb (RNS) variants; a fix here belongs there too (this copy is
+// kept apart so that the single-modulus kernel keeps its SASS).
 __global__ void __launch_bounds__(1024) ref_fwd_u64_kernel(const uint64_t *__restrict__ in, const uint64_t *__restrict__ in2,
                                                            uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
                                                            const uint64_t *__restrict__ precons, uint64_t q, uint32_t logn,
@@ -1159,6 +1201,109 @@ __device__ __forceinline__ void ref_pass16_u64(uint64_t (&x)[16], const uint64_t
     if constexpr (J < 3) ref_pass16_u64<VEC, JFIRST, J + 1>(x, roots, precons, s_first, t_hi, q, twice);
 }
 
+// ref_u64_frame_kernel (below) as the body of its per-limb variants (ref_u64_rns_frame_kernel, ...); the single-modulus
+// kernel keeps its own copy, as ref_fwd_u64_kernel does.  PAIR: the two CTAs of a split frame form a 2-CTA
+// cluster and each waits on the cluster barrier before its final global stores, so that neither overwrites a half its
+// partner has not read yet (pass 0 is the only phase that reads global memory): in place is then safe at N = 32768.
+template <int NT, bool PAIR = false>
+__device__ __forceinline__ void ref_u64_frame_body(const uint64_t *in, const uint64_t *in2, uint64_t *out,
+                                                   const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
+                                                   uint64_t q, uint32_t logn, uint32_t split, uint32_t frame, uint32_t half_id) {
+    // split = 0: one CTA per frame, logn <= 14.  split = 1: two CTAs per frame (logn = 15), CTA parity = which half.
+    extern __shared__ uint64_t img[];
+    constexpr bool VEC = AGX_U64_VECTW >= 2 || (AGX_U64_VECTW == 1 && NT >= 512);   // 16-byte twiddle pairs
+    const uint32_t tid = threadIdx.x;
+    // log2 of the coefficients this CTA owns: always log2(NT) + 5 (a CTA is N/32 threads, agx_api.cu ref_launch), so it is a
+    // compile-time constant and with it every pass's bit position, stride and stage count: shared-memory accesses become
+    // base + immediate and the pass loop unrolls into exactly the passes this size runs
+    constexpr uint32_t lg = (NT == 512 ? 14u : NT == 256 ? 13u : NT == 128 ? 12u : NT == 64 ? 11u : 10u);
+    constexpr uint32_t M = 1u << lg, vthreads = M >> 4;
+    if (logn - split != lg) return;                                // launch contract (never taken)
+    const uint64_t twice = q << 1;
+    const size_t fbase = (size_t)frame << logn;
+    const uint64_t *lo_src = in + fbase, *hi_src = in2 + fbase;    // low / high half of the frame (ntt.cpp:587-589)
+    uint64_t x[16];
+
+    // ---- pass 0: stages (split ..) on index bits [lg-4, lg), coefficients straight from global memory
+    {
+        constexpr uint32_t lo = lg - 4;
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            if (split) {
+                // stage 0 of the 32768-point frame, this CTA keeping only its half (ntt.cpp:331-369 with roots[1])
+                const uint64_t W = __ldg(roots + 1), Wp = __ldg(precons + 1);
+#pragma unroll
+                for (int k = 0; k < 16; k++) {
+                    const uint32_t i = (k << lo) + vt;
+                    uint64_t a = lo_src[i], b = hi_src[M + i];
+                    ref_bfly_u64(a, b, W, Wp, q, twice);
+                    x[k] = half_id ? b : a;
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 16; k++) {
+                    const uint32_t i = (k << lo) + vt;
+                    x[k] = (k < 8 ? lo_src : hi_src)[i];
+                }
+            }
+            // this CTA's sub-transform: stage s of it is global stage s + split, group offset half_id << s
+            // (roots index = 2^(s+split) + (half_id << s) + local group)
+            ref_pass16_u64<VEC, 0>(x, roots, precons, split, half_id, q, twice);
+            uint64_t *s = img + vt + (vt >> 4);
+            constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+    }
+    if constexpr (PAIR) asm volatile("barrier.cluster.arrive.aligned;" ::: "memory");   // this CTA's global reads are done
+    __syncthreads();
+    // ---- middle passes: index bits from lg-5 down to 4, four at a time (the last one may cover fewer)
+    uint32_t s_done = 4;                                           // stages of the sub-transform finished so far
+#pragma unroll
+    for (int rem = (int)lg - 8; rem > 0; rem -= 4) {
+        const uint32_t lo = rem >= 4 ? (uint32_t)rem : 4u;
+        const uint32_t jfirst = rem >= 4 ? 0u : (uint32_t)(4 - rem);
+        const uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint32_t t_lo = vt & ((1u << lo) - 1), t_hi = vt >> lo;
+            const uint32_t idx0 = (t_hi << (lo + 4)) + t_lo;
+            uint64_t *s = img + idx0 + (idx0 >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            // twiddle index: 2^(s+split) + ((half_id << s) + group) with group = (t_hi << j) + g at local stage j
+            const uint32_t sg = s_done + split;                    // global stage of the first active local stage
+            const uint32_t th = t_hi + (half_id << (s_done - jfirst));   // the CTA's half as the top bit of the group index
+            if (jfirst == 0) ref_pass16_u64<VEC, 0>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 1) ref_pass16_u64<VEC, 1>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 2) ref_pass16_u64<VEC, 2>(x, roots, precons, sg, th, q, twice);
+            else ref_pass16_u64<VEC, 3>(x, roots, precons, sg, th, q, twice);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+        s_done += 4 - jfirst;
+        __syncthreads();
+    }
+    // ---- final pass: bits 3..0 (16 consecutive coefficients), reduction to [0,q) (ntt.cpp:377-393)
+#pragma unroll 1
+    for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+        uint64_t *s = img + vt * 17;
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = s[k];
+        ref_pass16_u64<VEC, 0>(x, roots, precons, s_done + split, vt + (half_id << s_done), q, twice);
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            s[k] = ref_csub_u64(ref_csub_u64(x[k], twice), q);
+        }
+    }
+    __syncthreads();
+    if constexpr (PAIR) asm volatile("barrier.cluster.wait.aligned;" ::: "memory");     // ... and the partner's too
+    uint64_t *dst = out + fbase + (size_t)half_id * M;
+    for (uint32_t i = tid; i < M; i += NT) dst[i] = img[i + (i >> 4)];
+}
+
+// TWIN: ref_u64_frame_body is a copy of this kernel for the per-limb (RNS) variants; a fix here belongs there too (this copy is
+// kept apart so that the single-modulus kernel keeps its SASS).
 template <int NT>
 __global__ void __launch_bounds__(NT, 512 / NT) ref_u64_frame_kernel(const uint64_t *in, const uint64_t *in2,   // may alias each other and out
                                                               uint64_t *out, const uint64_t *__restrict__ roots,
@@ -1302,15 +1447,19 @@ __device__ __forceinline__ void ref_gs_last_bfly_u64(uint64_t &x, uint64_t &y, c
 // (a bit-serial loop of microseconds, which a whole CTA would wait for): w * recip >> (k-1) is floor(w * 2^64 / q) - e with
 // e in [0,2], so the remainder w * 2^64 - estimate * q lies in [0,3q) and is its own low 64 bits; each q it holds past the
 // first is one more unit of the quotient.
-__device__ __forceinline__ ulonglong2 ref_inv_fold(const uint64_t *__restrict__ roots, const RefInvConst &p) {
-    const uint64_t w = ref_csub_u64(ref_shoup_u64(__ldg(roots + 1), p.ninv, p.ninv_p, p.q), p.q);
+__device__ __forceinline__ uint64_t ref_shoup_companion(uint64_t w, const RefInvConst &p) {   // floor(w * 2^64 / q), w < q
     const uint32_t s = p.k - 1;
     uint64_t wp = (__umul64hi(w, p.recip) << (64 - s)) | ((w * p.recip) >> s);
     uint64_t r = 0 - wp * p.q;
 #pragma unroll
     for (int i = 0; i < 2; i++)
         if (r >= p.q) { r -= p.q; wp++; }
-    return make_ulonglong2(w, wp);
+    return wp;
+}
+
+__device__ __forceinline__ ulonglong2 ref_inv_fold(const uint64_t *__restrict__ roots, const RefInvConst &p) {
+    const uint64_t w = ref_csub_u64(ref_shoup_u64(__ldg(roots + 1), p.ninv, p.ninv_p, p.q), p.q);
+    return make_ulonglong2(w, ref_shoup_companion(w, p));
 }
 
 // a * b mod q exactly, a, b < q (HAC 14.42, b = 2, computed from the low 64 bits of the remainder)
@@ -1354,6 +1503,119 @@ __device__ __forceinline__ void ref_ipass16_u64(uint64_t (&x)[16], const uint64_
 // stages of its own half (the half is the top bit of every group index, as the forward's half_id); no stage before the
 // last couples the halves, so each CTA reads and writes only its own half (in place is safe) and leaves it in [0,2q) for
 // ref_u64_inv_last_stage_kernel.
+// ref_u64_inv_frame_body is that kernel for its per-limb variant (ref_u64_rns_inv_frame_kernel); the single-modulus kernel
+// keeps its own copy, as ref_fwd_u64_kernel does.  K supplies the modulus constants (RefInvOne, RefInvLimb).
+//
+// Where the inverse kernels take their modulus constants from.  One modulus (agx_ref_*): the kernel parameters, and the
+// folded last-stage twiddle computed from the caller's table.
+struct RefInvOne {
+    RefInvConst p;
+    const uint64_t *roots;
+    __device__ __forceinline__ uint64_t q() const { return p.q; }
+    __device__ __forceinline__ RefInvConst consts() const { return p; }
+    __device__ __forceinline__ ulonglong2 fold() const { return ref_inv_fold(roots, p); }
+};
+
+template <int NT>
+__host__ __device__ constexpr uint32_t ref_frame_lg() { return NT == 512 ? 14u : NT == 256 ? 13u : NT == 128 ? 12u : NT == 64 ? 11u : 10u; }
+
+template <int NT, class K>
+__device__ __forceinline__ void ref_u64_inv_frame_body(const uint64_t *in, const uint64_t *mul, uint64_t *out,
+                                                       const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
+                                                       const K &kc, uint32_t logn, uint32_t frame, uint32_t half_id) {
+    extern __shared__ uint64_t img[];
+    __shared__ ulonglong2 fold;
+    constexpr bool VEC = AGX_U64_VECTW >= 2 || (AGX_U64_VECTW == 1 && NT >= 512);
+    constexpr uint32_t lg = ref_frame_lg<NT>();
+    constexpr uint32_t M = 1u << lg, vthreads = M >> 4;
+    const uint32_t tid = threadIdx.x, split = logn - lg;
+    if (split > 1) return;                                         // launch contract (never taken)
+    const uint64_t q = kc.q(), twice = q << 1;
+    const size_t base = ((size_t)frame << logn) + (size_t)half_id * M;
+    if (!split && tid == 0) fold = kc.fold();                      // read after the barrier that ends the load
+
+    uint64_t x[16];
+    // ---- load (and the fused pointwise product): 16 coalesced reads in flight per thread, the forward's pass-0 pattern
+    {
+        constexpr uint32_t lo = lg - 4;
+        constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = in[base + (k << lo) + vt];
+            if (mul) {
+                const RefInvConst p = kc.consts();
+#pragma unroll
+                for (int k = 0; k < 16; k++) x[k] = ref_mulmod_u64(x[k], mul[base + (k << lo) + vt], p);
+            }
+            uint64_t *s = img + vt + (vt >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+    }
+    __syncthreads();
+    // ---- first pass: bits 3..0, stages h = N/2 .. N/16 of this CTA's sub-transform
+#pragma unroll 1
+    for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+        uint64_t *s = img + vt * 17;
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = s[k];
+        ref_ipass16_u64<VEC, 0>(x, roots, precons, lg - 4 + split, vt + (half_id << (lg - 4)), q, twice);
+#pragma unroll
+        for (int k = 0; k < 16; k++) s[k] = x[k];
+    }
+    __syncthreads();
+    // ---- middle passes: the forward's windows (lo, jfirst) from the lowest up; the lowest may be partial
+#pragma unroll
+    for (int rem = ((int)lg - 9) % 4 + 1; rem <= (int)lg - 8; rem += 4) {
+        const uint32_t lo = rem >= 4 ? (uint32_t)rem : 4u;
+        const uint32_t jfirst = rem >= 4 ? 0u : (uint32_t)(4 - rem);
+        const uint32_t stride = (1u << lo) + (1u << (lo - 4));
+        const uint32_t s_first = lg - 4 - lo + jfirst;             // sub-transform stage of local stage jfirst
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint32_t t_lo = vt & ((1u << lo) - 1), t_hi = vt >> lo;
+            const uint32_t idx0 = (t_hi << (lo + 4)) + t_lo;
+            uint64_t *s = img + idx0 + (idx0 >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            const uint32_t sg = s_first + split, th = t_hi + (half_id << (s_first - jfirst));
+            if (jfirst == 0) ref_ipass16_u64<VEC, 0>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 1) ref_ipass16_u64<VEC, 1>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 2) ref_ipass16_u64<VEC, 2>(x, roots, precons, sg, th, q, twice);
+            else ref_ipass16_u64<VEC, 3>(x, roots, precons, sg, th, q, twice);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+        __syncthreads();
+    }
+    // ---- last pass: the top four bits, straight to global memory
+    {
+        constexpr uint32_t lo = lg - 4;
+        constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+        uint64_t *dst = out + base;
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint64_t *s = img + vt + (vt >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            if (split) {
+                ref_ipass16_u64<VEC, 0>(x, roots, precons, 1, half_id, q, twice);
+            } else {
+                ref_ipass16_u64<VEC, 0, 1>(x, roots, precons, 0, 0, q, twice);
+                const ulonglong2 f = fold;
+                const RefInvConst p = kc.consts();
+#pragma unroll
+                for (int i = 0; i < 8; i++) ref_gs_last_bfly_u64(x[i], x[i + 8], p, f);
+            }
+#pragma unroll
+            for (int k = 0; k < 16; k++) dst[(k << lo) + vt] = x[k];
+        }
+    }
+}
+
+// TWIN: ref_u64_inv_frame_body is a copy of this kernel for the per-limb (RNS) variants; a fix here belongs there too (this copy is
+// kept apart so that the single-modulus kernel keeps its SASS).
 template <int NT>
 __global__ void __launch_bounds__(NT, 512 / NT) ref_u64_inv_frame_kernel(const uint64_t *in, const uint64_t *mul,   // may alias out
                                                                   uint64_t *out, const uint64_t *__restrict__ roots,
@@ -1472,15 +1734,17 @@ __global__ void __launch_bounds__(256) ref_u64_inv_last_stage_kernel(uint64_t *d
 }
 
 // N < 1024: plain radix-2 GS, one CTA per frame, the frame in shared memory (in the manner of ref_fwd_u64_kernel)
-__global__ void __launch_bounds__(256) ref_inv_u64_kernel(const uint64_t *in, const uint64_t *mul, uint64_t *out,
-                                                          const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
-                                                          RefInvConst p, uint32_t logn) {
+template <class K>
+__device__ __forceinline__ void ref_inv_u64_body(const uint64_t *in, const uint64_t *mul, uint64_t *out,
+                                                 const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
+                                                 const K &kc, uint32_t logn, uint32_t frame) {
     __shared__ uint64_t X[512];
     __shared__ ulonglong2 fold;
     const uint32_t N = 1u << logn;
-    const size_t base = (size_t)blockIdx.x * N;
+    const size_t base = (size_t)frame * N;
+    const RefInvConst p = kc.consts();
     const uint64_t q = p.q, twice = q << 1;
-    if (threadIdx.x == 0) fold = ref_inv_fold(roots, p);
+    if (threadIdx.x == 0) fold = kc.fold();
     for (uint32_t i = threadIdx.x; i < N; i += blockDim.x)
         X[i] = mul ? ref_mulmod_u64(in[base + i], mul[base + i], p) : in[base + i];
     __syncthreads();
@@ -1495,6 +1759,175 @@ __global__ void __launch_bounds__(256) ref_inv_u64_kernel(const uint64_t *in, co
         __syncthreads();
     }
     for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) out[base + i] = X[i];
+}
+
+__global__ void __launch_bounds__(256) ref_inv_u64_kernel(const uint64_t *in, const uint64_t *mul, uint64_t *out,
+                                                          const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
+                                                          RefInvConst p, uint32_t logn) {
+    ref_inv_u64_body(in, mul, out, roots, precons, RefInvOne{p, roots}, logn, blockIdx.x);
+}
+
+// ------------------------------------------------------------------------ u64 RNS batches ([B][L][N], agx_create64)
+// The kernels above over L primes at once: frame f = b * L + l is limb l = f % L of polynomial b.  Each CTA derives its
+// limb from its frame, offsets the library's tables ([L][N] words per table, the reference's order) by limb * N and reads
+// its modulus constants from a per-limb array built at create time -- including the inverse's folded last-stage twiddle
+// iroots[1] * n^-1, which the single-modulus kernels derive per CTA from the caller's table.  Arithmetic and geometry are
+// the single-modulus kernels' (the same bodies), so every limb's result equals the single-modulus call's bit for bit.
+struct RnsLimb64 {
+    RefInvConst p;          // q, n^-1 and its companion, Barrett mu / k, reciprocal floor(2^(63+k) / q)
+    ulonglong2 fold;        // iroots[1] * n^-1 mod q and floor(that * 2^64 / q)
+    uint64_t psi, psi_inv;  // table bases (gen_tables64_kernel)
+};
+
+// The inverse's constants from one limb's entry: q is loaded once, the rest where it is used (the frame kernels run at
+// the 128-register cap, so nothing is held in registers across the passes that the passes do not need).
+struct RefInvLimb {
+    const RnsLimb64 *lc;
+    uint64_t q_;
+    __device__ __forceinline__ uint64_t q() const { return q_; }
+    __device__ __forceinline__ RefInvConst consts() const {
+        RefInvConst p;
+        p.q = q_;
+        p.ninv = __ldg(&lc->p.ninv);
+        p.ninv_p = __ldg(&lc->p.ninv_p);
+        p.mu = __ldg(&lc->p.mu);
+        p.recip = __ldg(&lc->p.recip);
+        p.k = __ldg(&lc->p.k);
+        return p;
+    }
+    __device__ __forceinline__ ulonglong2 fold() const { return __ldg(&lc->fold); }
+};
+
+// forward, N >= 1024 except N = 32768: one CTA per frame
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_rns_frame_kernel(const uint64_t *in, uint64_t *out,   // in may be out
+                                                                  const uint64_t *__restrict__ roots,
+                                                                  const uint64_t *__restrict__ precons,
+                                                                  const RnsLimb64 *__restrict__ lc, uint32_t L, uint32_t logn) {
+    const uint32_t frame = blockIdx.x, limb = frame % L;
+    const size_t toff = (size_t)limb << logn;
+    ref_u64_frame_body<NT>(in, in, out, roots + toff, precons + toff, __ldg(&lc[limb].p.q), logn, 0, frame, 0);
+}
+
+// forward, N = 32768: the two CTAs of a frame as a 2-CTA cluster (ref_u64_frame_body<PAIR>), in place or not
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(512, 1)
+    ref_u64_rns_frame_pair_kernel(const uint64_t *in, uint64_t *out, const uint64_t *__restrict__ roots,
+                                  const uint64_t *__restrict__ precons, const RnsLimb64 *__restrict__ lc, uint32_t L) {
+    constexpr uint32_t logn = 15;
+    const uint32_t frame = blockIdx.x >> 1, limb = frame % L;
+    const size_t toff = (size_t)limb << logn;
+    ref_u64_frame_body<512, true>(in, in, out, roots + toff, precons + toff, __ldg(&lc[limb].p.q), logn, 1, frame,
+                                  blockIdx.x & 1u);
+}
+
+// inverse, N >= 1024 (two CTAs per frame and ref_u64_rns_inv_last_stage_kernel at N = 32768)
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_rns_inv_frame_kernel(const uint64_t *in, const uint64_t *mul,   // may alias out
+                                                                      uint64_t *out, const uint64_t *__restrict__ roots,
+                                                                      const uint64_t *__restrict__ precons,
+                                                                      const RnsLimb64 *__restrict__ lc, uint32_t L,
+                                                                      uint32_t logn) {
+    const uint32_t split = logn - ref_frame_lg<NT>();
+    const uint32_t frame = split ? blockIdx.x >> 1 : blockIdx.x, limb = frame % L;
+    const size_t toff = (size_t)limb << logn;
+    ref_u64_inv_frame_body<NT>(in, mul, out, roots + toff, precons + toff, RefInvLimb{lc + limb, __ldg(&lc[limb].p.q)}, logn,
+                               frame, split ? blockIdx.x & 1u : 0u);
+}
+
+// N = 32768: the last inverse stage (ref_u64_inv_last_stage_kernel), each 2-pair unit with its own frame's limb
+__global__ void __launch_bounds__(256) ref_u64_rns_inv_last_stage_kernel(uint64_t *data, const RnsLimb64 *__restrict__ lc,
+                                                                         uint32_t L, uint32_t logn, size_t frames) {
+    const uint32_t hlog = logn - 2;                                // 2-pair units per half frame
+    const size_t units = frames << hlog;
+    for (size_t u = (size_t)blockIdx.x * blockDim.x + threadIdx.x; u < units; u += (size_t)gridDim.x * blockDim.x) {
+        const RnsLimb64 *c = lc + (uint32_t)((u >> hlog) % L);
+        const RefInvConst p = RefInvLimb{c, __ldg(&c->p.q)}.consts();
+        const ulonglong2 f = __ldg(&c->fold);
+        const size_t i = ((u >> hlog) << logn) + ((u & ((1u << hlog) - 1)) << 1);
+        ulonglong2 *lo = reinterpret_cast<ulonglong2 *>(data + i), *hi = reinterpret_cast<ulonglong2 *>(data + i + (1u << (logn - 1)));
+        const ulonglong2 a = *lo, b = *hi;
+        uint64_t u0 = a.x, u1 = a.y, v0 = b.x, v1 = b.y;
+        ref_gs_last_bfly_u64(u0, v0, p, f);
+        ref_gs_last_bfly_u64(u1, v1, p, f);
+        *lo = make_ulonglong2(u0, u1);
+        *hi = make_ulonglong2(v0, v1);
+    }
+}
+
+// N < 1024: the radix-2 kernels, one CTA per frame
+__global__ void __launch_bounds__(1024) ref_fwd_u64_rns_kernel(const uint64_t *__restrict__ in, uint64_t *__restrict__ out,
+                                                               const uint64_t *__restrict__ roots,
+                                                               const uint64_t *__restrict__ precons,
+                                                               const RnsLimb64 *__restrict__ lc, uint32_t L, uint32_t logn) {
+    const uint32_t frame = blockIdx.x, limb = frame % L;
+    const size_t toff = (size_t)limb << logn;
+    ref_fwd_u64_body(in, in, out, roots + toff, precons + toff, __ldg(&lc[limb].p.q), logn, 1, frame);
+}
+
+__global__ void __launch_bounds__(256) ref_inv_u64_rns_kernel(const uint64_t *in, const uint64_t *mul, uint64_t *out,
+                                                              const uint64_t *__restrict__ roots,
+                                                              const uint64_t *__restrict__ precons,
+                                                              const RnsLimb64 *__restrict__ lc, uint32_t L, uint32_t logn) {
+    const uint32_t frame = blockIdx.x, limb = frame % L;
+    const size_t toff = (size_t)limb << logn;
+    ref_inv_u64_body(in, mul, out, roots + toff, precons + toff, RefInvLimb{lc + limb, __ldg(&lc[limb].p.q)}, logn, frame);
+}
+
+// c = a + b | a - b | a * b | c + a * b modulo each limb's prime over [B][L][N] words (operands < q, results in [0,q)),
+// two words per 16-byte access (N >= 4, so an access never straddles two limbs); grid-stride
+template <int OP>
+__global__ void __launch_bounds__(256) elementwise64_kernel(ulonglong2 *c2, const ulonglong2 *a2, const ulonglong2 *b2,
+                                                            const RnsLimb64 *__restrict__ lc, uint32_t L, uint32_t logn,
+                                                            size_t total2) {
+    for (size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x; i < total2; i += (size_t)gridDim.x * blockDim.x) {
+        const RnsLimb64 *l = lc + (uint32_t)(((i << 1) >> logn) % L);
+        const uint64_t q = __ldg(&l->p.q);
+        const ulonglong2 a = a2[i], b = b2[i];
+        uint64_t r[2];
+        const uint64_t av[2] = {a.x, a.y}, bv[2] = {b.x, b.y};
+        if constexpr (OP == EW_ADD) {
+#pragma unroll
+            for (int j = 0; j < 2; j++) r[j] = ref_csub_u64(av[j] + bv[j], q);
+        } else if constexpr (OP == EW_SUB) {
+#pragma unroll
+            for (int j = 0; j < 2; j++) r[j] = ref_csub_u64(av[j] + q - bv[j], q);
+        } else {
+            const RefInvConst p = RefInvLimb{l, q}.consts();
+#pragma unroll
+            for (int j = 0; j < 2; j++) r[j] = ref_mulmod_u64(av[j], bv[j], p);
+            if constexpr (OP == EW_MAC) {
+                const ulonglong2 c = c2[i];
+                r[0] = ref_csub_u64(r[0] + c.x, q);
+                r[1] = ref_csub_u64(r[1] + c.y, q);
+            }
+        }
+        c2[i] = make_ulonglong2(r[0], r[1]);
+    }
+}
+
+// The library's u64 tables: one thread per (direction, limb, k), w = base^bitrev(k) mod q (base = psi forward, psi^-1
+// inverse) by square-and-multiply with the exact Barrett product, and its Shoup companion floor(w * 2^64 / q) by the
+// reciprocal estimate and correction of ref_inv_fold (a 128-bit division compiles to a bit-serial loop).  The order is
+// the reference's (ntt.cpp:298-300), which the kernels above read directly.  tab: [4][L][n] = forward roots, forward
+// companions, inverse roots, inverse companions.
+__global__ void __launch_bounds__(256) gen_tables64_kernel(uint64_t *__restrict__ tab, const RnsLimb64 *__restrict__ lc,
+                                                           uint32_t L, uint32_t logn) {
+    const uint32_t n = 1u << logn;
+    const uint32_t gid = blockIdx.x * blockDim.x + threadIdx.x;
+    if (gid >= 2u * L * n) return;
+    const uint32_t k = gid & (n - 1), limb = (gid >> logn) % L;
+    const bool inverse = gid >= L * n;
+    const RefInvConst p = lc[limb].p;
+    const uint32_t e = __brev(k) >> (32 - logn);
+    uint64_t w = 1, b = inverse ? lc[limb].psi_inv : lc[limb].psi;
+    for (uint32_t i = 0; i < logn; i++) {
+        if ((e >> i) & 1) w = ref_mulmod_u64(w, b, p);
+        b = ref_mulmod_u64(b, b, p);
+    }
+    const uint64_t wp = ref_shoup_companion(w, p);
+    const size_t at = (size_t)(inverse ? 2 : 0) * L * n + (size_t)limb * n + k;
+    tab[at] = w;
+    tab[at + (size_t)L * n] = wp;
 }
 
 // ------------------------------------------------------------------------------------- twiddle tables on device

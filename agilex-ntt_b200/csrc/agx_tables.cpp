@@ -46,7 +46,11 @@ uint32_t bit_reverse(uint32_t x, uint32_t bits) {
 }
 
 uint32_t minimal_psi(uint32_t n, uint32_t q) {
-    if (n < 2 || (n & (n - 1)) || q >= (1u << 30) || (uint64_t)(q - 1) % (2ull * n) || !is_prime_u64(q)) return 0;
+    return q >= (1u << 30) ? 0u : (uint32_t)minimal_psi_u64(n, q);
+}
+
+uint64_t minimal_psi_u64(uint32_t n, uint64_t q) {
+    if (n < 2 || (n & (n - 1)) || q < 3 || q >= (1ull << 62) || (q - 1) % (2ull * n) || !is_prime_u64(q)) return 0;
     const uint64_t e = (q - 1) / (2ull * n);
     uint64_t g = 0;
     for (uint64_t x = 2; x < q && !g; x++) {
@@ -61,7 +65,7 @@ uint32_t minimal_psi(uint32_t n, uint32_t q) {
         if (cur < best) best = cur;
         cur = mulmod_u64(cur, g2, q);
     }
-    return (uint32_t)best;
+    return best;
 }
 
 }  // namespace agx

@@ -19,5 +19,7 @@ uint32_t bit_reverse(uint32_t x, uint32_t bits);
 
 // 0 when q is not a usable NTT prime for n (not prime, >= 2^30, q != 1 mod 2n)
 uint32_t minimal_psi(uint32_t n, uint32_t q);
+// the same for the u64 path: 0 unless q is prime, 3 <= q < 2^62 and q = 1 (mod 2n)
+uint64_t minimal_psi_u64(uint32_t n, uint64_t q);
 
 }  // namespace agx

@@ -204,6 +204,48 @@ int agx_ref_polymul_by_spectrum_dev(agx_ctx *ctx, uint32_t N, uint64_t *d_c, con
                                     const uint64_t *d_precon_twiddles, const uint64_t *d_inv_twiddles,
                                     const uint64_t *d_inv_precon_twiddles, uint32_t numFrames, void *stream);
 
+/* ---- u64 RNS batches: L primes of 50-62 bits, [B][L][n] DEVICE data (no reference counterpart; the u64 counterpart of
+ * agx_create / agx_ntt_fwd / agx_ntt_inv / agx_polymul / agx_polymul_by_spectrum / agx_elementwise, SURVEY.md s.8(f)).
+ * Conventions of the u32 batched entry points (device pointers, in place, asynchronous on `stream`, 16-byte aligned
+ * pointers, uint64_t data[B][L][n] row-major: frame f = b * L + l is limb l of polynomial b) with the arithmetic of
+ * agx_ref_fwd_dev / agx_ref_inv_dev.  A context holds either a u32 or a u64 parameter set: a u64 call on a u32 context
+ * and the reverse give AGX_E_INVALID; the agx_ref_* calls work on every context.
+ *
+ * agx_create64: n = 2^logn in [4, 32768]; 1 <= nlimbs <= 64; every q[i] prime with 3 <= q < 2^62 and q = 1 (mod 2n).
+ *   psi[nlimbs] is the caller's primitive 2n-th root per limb (AGX_E_INVALID unless psi[i]^n = -1 mod q[i]), NULL = the
+ *   minimal one.  Anything else gives AGX_E_INVALID and no context.  The tables are built on the device at create time.
+ * agx_get_tables64: one limb's table as HOST arrays of n words, in the reference's order (ntt.cpp:298-300): roots[k] =
+ *   psi^bitrev(k) (inverse != 0: psi^-bitrev(k)), precons[k] = floor(roots[k] * 2^64 / q), entry 0 = 1 -- exactly the
+ *   tables agx_ref_fwd_dev / agx_ref_inv_dev take.
+ * Inputs: the forward accepts words < 4q, the inverse < 2q; product and element-wise operands must be reduced (< q).
+ * Results are in [0,q).  For every limb, agx_ntt64_fwd, agx_ntt64_inv, agx_polymul64 and agx_polymul64_by_spectrum equal
+ * bit for bit agx_ref_fwd_dev, agx_ref_inv_dev, agx_ref_polymul_dev and agx_ref_polymul_by_spectrum_dev on that limb's
+ * frames with the tables of agx_get_tables64; agx_polymul64_by_spectrum(c, a, agx_ntt64_fwd(b)) = agx_polymul64(c, a, b).
+ * c may alias a and/or b (b_hat), and a may equal b.  NTT(b) of the product takes a stream-ordered scratch buffer unless
+ * a == b; so does NTT(a) of the by-spectrum product when c == b_hat.
+ * B == 0 returns AGX_OK and launches nothing; B * nlimbs > 2^31 - 1 gives AGX_E_INVALID.
+ * Launches (agx_launch_count), every limb in each: agx_ntt64_fwd 1, agx_ntt64_inv 1, agx_polymul64 3,
+ * agx_polymul64_by_spectrum 2, agx_elementwise64 1; at n = 32768 the inverse adds one (its last stage streams over the
+ * batch), so 1, 2, 4, 3, 1.  The forward at n = 32768 runs two CTAs per frame as a 2-CTA cluster, in place included. ---- */
+typedef struct {
+    uint32_t n;
+    uint32_t logn;
+    uint32_t nlimbs;
+    const uint64_t *q; /* [nlimbs] */
+} agx_parms64;
+
+int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, int device);
+int agx_get_psi64(const agx_ctx *ctx, uint32_t limb, uint64_t *psi);
+int agx_get_tables64(const agx_ctx *ctx, uint32_t limb, int inverse, uint64_t *roots, uint64_t *precons);
+int agx_ntt64_fwd(agx_ctx *ctx, uint64_t *d_data, size_t B, void *stream);
+int agx_ntt64_inv(agx_ctx *ctx, uint64_t *d_data, size_t B, void *stream);
+int agx_polymul64(agx_ctx *ctx, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b, size_t B, void *stream);
+int agx_polymul64_by_spectrum(agx_ctx *ctx, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b_hat, size_t B,
+                              void *stream);
+/* op = AGX_EW_*, modulo each limb's prime */
+int agx_elementwise64(agx_ctx *ctx, int op, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b, size_t B,
+                      void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

@@ -79,6 +79,7 @@ def _load() -> C.CDLL:
         "agx_polymul64": [vp, vp, vp, vp, C.c_size_t, vp],
         "agx_polymul64_by_spectrum": [vp, vp, vp, vp, C.c_size_t, vp],
         "agx_elementwise64": [vp, C.c_int, vp, vp, vp, C.c_size_t, vp],
+        "agx_rescale64": [vp, vp, vp, C.c_size_t, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -97,7 +98,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_ntt_fwd_host agx_ntt_inv_host agx_polymul_host agx_host_alloc agx_host_free agx_fill_synthetic "
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
-           "agx_polymul64_by_spectrum agx_elementwise64").split()
+           "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64").split()
 
 _lib = None
 
@@ -411,6 +412,23 @@ class Context64:
         _ck(lib().agx_elementwise64(self._h, self.EW[op], _dev_ptr8(c), _dev_ptr8(a), _dev_ptr8(b), B,
                                     _stream_ptr(stream)), "agx_elementwise64")
         return c
+
+    def rescale(self, out, inp, ntt_form=True, stream=None):
+        """Divide by the last prime and round (agx_rescale64): inp (B, L, n) -> out (B, L - 1, n), the residues of
+        floor((X + h) / q_{L-1}) with h = floor(q_{L-1} / 2) over the first L - 1 primes.  ntt_form: both in evaluation
+        form as fwd leaves them (else both in coefficient form).  Reduced inputs; out must not overlap inp.  The result
+        belongs to a context over primes[:-1] (same roots), whose tables are this context's first L - 1 limbs."""
+        for t in (out, inp):
+            if not t.is_cuda or t.device.index != self.device:
+                raise ValueError(f"need CUDA tensors on device {self.device}")
+        if inp.dim() != 3 or tuple(inp.shape[1:]) != (self.L, self.n):
+            raise ValueError(f"inp must have shape (B, {self.L}, {self.n})")
+        B = inp.shape[0]
+        if tuple(out.shape) != (B, self.L - 1, self.n):
+            raise ValueError(f"out must have shape ({B}, {self.L - 1}, {self.n})")
+        _ck(lib().agx_rescale64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, int(bool(ntt_form)), _stream_ptr(stream)),
+            "agx_rescale64")
+        return out
 
 
 class RefPipeline:

@@ -102,6 +102,8 @@ struct agx_ctx {
     std::vector<uint64_t> q64, psi64;
     uint64_t *d_tab64 = nullptr;                           // [4][L][n]: roots, companions; forward then inverse
     RnsLimb64 *d_lc64 = nullptr;                           // per-limb modulus constants
+    RescaleLimb64 *d_rs64 = nullptr;                       // [L-1] rescale constants (L >= 2, q_{L-1} unlike the others)
+    uint64_t rs_qlast = 0, rs_h = 0;                       // q_{L-1} and floor(q_{L-1} / 2)
     HostPipe pipe;
     RefState ref;
     CopyCrew *crew_in = nullptr, *crew_out = nullptr;      // created with the first pageable call
@@ -1100,7 +1102,7 @@ int agx_destroy(agx_ctx *c) {
         cudaFree(c->d_tw_fwd); cudaFree(c->d_tw_inv); cudaFree(c->d_nat_fwd); cudaFree(c->d_nat_inv);
         cudaFree(c->d_twc_fwd); cudaFree(c->d_twc_inv);
         cudaFree(c->d_lc); cudaFree(c->d_sum);
-        cudaFree(c->d_tab64); cudaFree(c->d_lc64);
+        cudaFree(c->d_tab64); cudaFree(c->d_lc64); cudaFree(c->d_rs64);
 #if AGX_WITH_R16
         cudaFree(c->d_tw16_fwd); cudaFree(c->d_tw16_inv); cudaFree(c->d_u16_fwd); cudaFree(c->d_u16_inv);
 #endif
@@ -1453,10 +1455,35 @@ int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, i
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_frame_pair_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rns_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_fwd_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_fwd_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
     const size_t entries = (size_t)L * n;
     if (e == cudaSuccess) e = cudaMalloc(&c->d_tab64, 4 * entries * sizeof(uint64_t));
     if (e == cudaSuccess) e = cudaMalloc(&c->d_lc64, L * sizeof(RnsLimb64));
     if (e == cudaSuccess) e = cudaMemcpy(c->d_lc64, lc.data(), L * sizeof(RnsLimb64), cudaMemcpyHostToDevice);
+    // the rescale's constants (agx_rescale64): for each i < L - 1, q_{L-1}^-1 mod q_i and its Shoup companion, h mod q_i
+    // and floor(2^64 / q_i); none when L = 1 or when q_{L-1} repeats an earlier prime (then it has no inverse)
+    const uint64_t qlast = parms->q[L - 1];
+    bool rescalable = L >= 2;
+    for (uint32_t i = 0; i + 1 < L; i++) rescalable = rescalable && parms->q[i] != qlast;
+    if (e == cudaSuccess && rescalable) {
+        std::vector<RescaleLimb64> rs(L - 1);
+        c->rs_qlast = qlast;
+        c->rs_h = qlast / 2;
+        for (uint32_t i = 0; i + 1 < L; i++) {
+            const uint64_t q = parms->q[i];
+            RescaleLimb64 &r = rs[i];
+            r.q = q;
+            r.one_p = (uint64_t)(((u128)1 << 64) / q);
+            r.h = c->rs_h % q;
+            r.qinv = powmod_u64(qlast % q, q - 2, q);
+            r.qinv_p = (uint64_t)(((u128)r.qinv << 64) / q);
+        }
+        e = cudaMalloc(&c->d_rs64, (L - 1) * sizeof(RescaleLimb64));
+        if (e == cudaSuccess) e = cudaMemcpy(c->d_rs64, rs.data(), (L - 1) * sizeof(RescaleLimb64), cudaMemcpyHostToDevice);
+    }
     if (e == cudaSuccess) {
         const size_t total = 2 * entries;
         gen_tables64_kernel<<<(unsigned)((total + 255) / 256), 256>>>(c->d_tab64, c->d_lc64, L, logn);
@@ -1557,6 +1584,86 @@ int agx_elementwise64(agx_ctx *c, int op, uint64_t *dc, const uint64_t *da, cons
     }
     c->launches++;
     return (int)cudaGetLastError();
+}
+
+int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
+    if (c->L < 2 || !c->d_rs64) return AGX_E_INVALID;
+    // in place is refused: the compaction from stride L to L - 1 lets one polynomial's CTAs overwrite input that
+    // another polynomial's CTAs have not read yet
+    const uintptr_t i0 = reinterpret_cast<uintptr_t>(d_in), i1 = i0 + T * c->n * sizeof(uint64_t);
+    const uintptr_t o0 = reinterpret_cast<uintptr_t>(d_out), o1 = o0 + (T - B) * c->n * sizeof(uint64_t);
+    if (B && i0 < o1 && o0 < i1) return AGX_E_INVALID;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const uint32_t logn = c->logn, L = c->L, N = c->n;
+    if (!ntt_form) {
+        const size_t pairs = B * N / 2;
+        const unsigned blocks = (unsigned)std::min<size_t>((pairs + 255) / 256, (size_t)c->sms * 16);
+        rescale64_coeff_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<ulonglong2 *>(d_out),
+                                                       reinterpret_cast<const ulonglong2 *>(d_in), c->d_rs64, c->rs_qlast,
+                                                       c->rs_h, L, logn, pairs);
+        c->launches++;
+        return (int)cudaGetLastError();
+    }
+    // evaluation form: scratch[b] = INTT_{L-1}(x_hat[b][L-1]); out[b][i] = (x_hat[b][i] - NTT_i(r_i(scratch[b]))) / q_{L-1}
+    uint64_t *tmp = nullptr;
+    int rc = (int)cudaMallocAsync(&tmp, B * N * sizeof(uint64_t), st);
+    if (!rc) {
+        const RnsLimb64 *last = c->d_lc64 + (L - 1);
+        const size_t toff = (size_t)(L - 1) * N;
+        const uint64_t *itw = tab64(c, 2) + toff, *ipre = tab64(c, 3) + toff;
+        if (logn >= 10) {
+            const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+            const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+            const unsigned grid = (unsigned)(B << split);
+            switch (lg) {
+                case 14: ref_u64_rescale_inv_frame_kernel<512><<<grid, 512, smem, st>>>(d_in, tmp, itw, ipre, last, L, logn); break;
+                case 13: ref_u64_rescale_inv_frame_kernel<256><<<grid, 256, smem, st>>>(d_in, tmp, itw, ipre, last, L, logn); break;
+                case 12: ref_u64_rescale_inv_frame_kernel<128><<<grid, 128, smem, st>>>(d_in, tmp, itw, ipre, last, L, logn); break;
+                case 11: ref_u64_rescale_inv_frame_kernel<64><<<grid, 64, smem, st>>>(d_in, tmp, itw, ipre, last, L, logn); break;
+                default: ref_u64_rescale_inv_frame_kernel<32><<<grid, 32, smem, st>>>(d_in, tmp, itw, ipre, last, L, logn); break;
+            }
+            c->launches++;
+            if (split) {                                           // the scratch as a batch of B frames of limb L - 1
+                const size_t units = B << (logn - 2);
+                const unsigned blocks = (unsigned)std::min<size_t>((units + 255) / 256, (size_t)c->sms * 8);
+                ref_u64_rns_inv_last_stage_kernel<<<blocks, 256, 0, st>>>(tmp, last, 1, logn, B);
+                c->launches++;
+            }
+        } else {
+            ref_inv_u64_rescale_kernel<<<(unsigned)B, N / 2 < 32 ? 32 : N / 2, 0, st>>>(d_in, tmp, itw, ipre, last, L, logn);
+            c->launches++;
+        }
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc) {
+        const uint64_t *tw = tab64(c, 0), *pre = tab64(c, 1);
+        const RescaleLimb64 *rs = c->d_rs64;
+        const uint64_t ql = c->rs_qlast, h = c->rs_h;
+        const unsigned frames = (unsigned)(T - B);                 // B * (L - 1)
+        if (logn >= 10) {
+            const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+            const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+            const unsigned grid = frames << split;
+            switch (lg) {
+                case 14: ref_u64_rescale_fwd_kernel<512><<<grid, 512, smem, st>>>(d_in, tmp, d_out, tw, pre, rs, ql, h, L, logn); break;
+                case 13: ref_u64_rescale_fwd_kernel<256><<<grid, 256, smem, st>>>(d_in, tmp, d_out, tw, pre, rs, ql, h, L, logn); break;
+                case 12: ref_u64_rescale_fwd_kernel<128><<<grid, 128, smem, st>>>(d_in, tmp, d_out, tw, pre, rs, ql, h, L, logn); break;
+                case 11: ref_u64_rescale_fwd_kernel<64><<<grid, 64, smem, st>>>(d_in, tmp, d_out, tw, pre, rs, ql, h, L, logn); break;
+                default: ref_u64_rescale_fwd_kernel<32><<<grid, 32, smem, st>>>(d_in, tmp, d_out, tw, pre, rs, ql, h, L, logn); break;
+            }
+        } else {
+            ref_fwd_u64_rescale_kernel<<<frames, N / 2 < 32 ? 32 : N / 2, (size_t)N * 8, st>>>(d_in, tmp, d_out, tw, pre, rs,
+                                                                                            ql, h, L, logn);
+        }
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

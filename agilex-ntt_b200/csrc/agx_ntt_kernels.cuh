@@ -903,6 +903,8 @@ __global__ void __launch_bounds__(256) elementwise_kernel(uint4 *c4, const uint4
 // N*8 bytes fits, else in the output buffer itself.
 // ref_fwd_u64_body is this kernel's body for the per-limb variant (ref_fwd_u64_rns_kernel).  ref_fwd_u64_kernel keeps its
 // own copy: routed through the shared body it compiles to different SASS, and the single-modulus kernels stay as they were.
+// TWIN: ref_fwd_u64_rescale_kernel (the rescale's fused forward below N = 1024) is a copy of this body with a prologue and
+// an epilogue; a fix here belongs there too.
 __device__ __forceinline__ void ref_fwd_u64_body(const uint64_t *__restrict__ in, const uint64_t *__restrict__ in2,
                                                  uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
                                                  const uint64_t *__restrict__ precons, uint64_t q, uint32_t logn, int use_smem,
@@ -1205,6 +1207,8 @@ __device__ __forceinline__ void ref_pass16_u64(uint64_t (&x)[16], const uint64_t
 // kernel keeps its own copy, as ref_fwd_u64_kernel does.  PAIR: the two CTAs of a split frame form a 2-CTA
 // cluster and each waits on the cluster barrier before its final global stores, so that neither overwrites a half its
 // partner has not read yet (pass 0 is the only phase that reads global memory): in place is then safe at N = 32768.
+// TWIN: ref_u64_rescale_fwd_kernel (the rescale's fused forward) is a copy of this body with a prologue in pass 0 and an
+// epilogue in the final store; a fix here belongs there too.
 template <int NT, bool PAIR = false>
 __device__ __forceinline__ void ref_u64_frame_body(const uint64_t *in, const uint64_t *in2, uint64_t *out,
                                                    const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
@@ -1928,6 +1932,264 @@ __global__ void __launch_bounds__(256) gen_tables64_kernel(uint64_t *__restrict_
     const size_t at = (size_t)(inverse ? 2 : 0) * L * n + (size_t)limb * n + k;
     tab[at] = w;
     tab[at + (size_t)L * n] = wp;
+}
+
+// ------------------------------------------------------------------ u64 RNS rescale ([B][L][N] -> [B][L-1][N])
+// Division by the last prime q_L' = q_{L-1} with rounding (agx_rescale64): with h = floor(q_L' / 2) and, per coefficient,
+// u = (x_{L-1} + h) mod q_L', every other limb i < L - 1 becomes
+//   y_i = (x_i - (u - h)) * q_L'^-1  mod q_i,
+// the residues of round-half-up(X / q_L') for the CRT value X of the L residues.  u < q_L' may exceed q_i (the primes
+// come in any order): it is reduced by a Shoup product with 1, whose companion floor(2^64 / q_i) brings ANY 64-bit word
+// into [0, 2q_i) -- unlike the exact Barrett product (ref_mulmod_u64), which needs its argument below 2^(2k_i) and so
+// would fail for a small q_i beside a 62-bit q_L'.  Per-limb constants, built at create time (agx_create64, L >= 2) in
+// an array of their own; q_L' and h are the same for every limb and go in as kernel parameters.
+struct RescaleLimb64 {
+    uint64_t q;              // q_i
+    uint64_t one_p;          // floor(2^64 / q_i): Shoup companion of 1
+    uint64_t h;              // h mod q_i
+    uint64_t qinv, qinv_p;   // q_L'^-1 mod q_i and floor(qinv * 2^64 / q_i)
+};
+
+// The forward's input from a word t < q_L' of limb L - 1 in coefficient form: u = (t + h) mod q_L', returned as a word
+// congruent to u - h (mod q_i) in (q_i, 4q_i), the forward transform's input range.  twice_minus_h = 2q_i - (h mod q_i).
+__device__ __forceinline__ uint64_t rescale_lift_u64(uint64_t t, uint64_t qlast, uint64_t h, uint64_t one_p, uint64_t q,
+                                                     uint64_t twice_minus_h) {
+    return ref_shoup_u64(ref_csub_u64(t + h, qlast), 1, one_p, q) + twice_minus_h;
+}
+
+// (x - r) * q_L'^-1 mod q_i in [0, q_i), for x < 2q_i and r < 2q_i   (x + 2q_i - r < 4q_i < 2^64; Shoup gives [0, 2q_i))
+__device__ __forceinline__ uint64_t rescale_finish_u64(uint64_t x, uint64_t r, uint64_t q, uint64_t qinv, uint64_t qinv_p) {
+    return ref_csub_u64(ref_shoup_u64(x + (q << 1) - r, qinv, qinv_p, q), q);
+}
+
+// Coefficient form: grid-stride over the 16-byte pairs of one limb row of every polynomial.  A thread loads its pair of
+// x_{L-1} once, forms u, and then walks the L - 1 output limbs: B*L*n words read, B*(L-1)*n written, nothing else.
+__global__ void __launch_bounds__(256) rescale64_coeff_kernel(ulonglong2 *__restrict__ out2, const ulonglong2 *__restrict__ in2,
+                                                              const RescaleLimb64 *__restrict__ rc, uint64_t qlast, uint64_t h,
+                                                              uint32_t L, uint32_t logn, size_t pairs) {
+    const uint32_t hlog = logn - 1;                                // pairs per row
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < pairs; p += (size_t)gridDim.x * blockDim.x) {
+        const size_t b = p >> hlog, j = p & ((1u << hlog) - 1);
+        const ulonglong2 *row = in2 + ((b * L) << hlog) + j;
+        ulonglong2 *dst = out2 + ((b * (L - 1)) << hlog) + j;
+        const ulonglong2 xl = row[(size_t)(L - 1) << hlog];
+        const uint64_t u0 = ref_csub_u64(xl.x + h, qlast), u1 = ref_csub_u64(xl.y + h, qlast);
+        for (uint32_t i = 0; i < L - 1; i++) {
+            const RescaleLimb64 *c = rc + i;
+            const uint64_t q = __ldg(&c->q), one_p = __ldg(&c->one_p), qh = q - __ldg(&c->h);
+            const uint64_t qinv = __ldg(&c->qinv), qinv_p = __ldg(&c->qinv_p);
+            const ulonglong2 x = row[(size_t)i << hlog];
+            // r = (u mod q_i) + q_i - (h mod q_i), in (0, 2q_i)
+            const uint64_t r0 = ref_csub_u64(ref_shoup_u64(u0, 1, one_p, q), q) + qh;
+            const uint64_t r1 = ref_csub_u64(ref_shoup_u64(u1, 1, one_p, q), q) + qh;
+            dst[(size_t)i << hlog] = make_ulonglong2(rescale_finish_u64(x.x, r0, q, qinv, qinv_p),
+                                                     rescale_finish_u64(x.y, r1, q, qinv, qinv_p));
+        }
+    }
+}
+
+// Evaluation form, step 1: the inverse transform of limb L - 1 of every polynomial into the contiguous scratch [B][n]
+// (ref_u64_inv_frame_body / ref_inv_u64_body on pointers already offset to the polynomial's last limb and to its scratch
+// row, frame 0).  roots / precons: the inverse table of limb L - 1; last = lc + L - 1.  At N = 32768 the halves are left
+// in [0,2q) for ref_u64_rns_inv_last_stage_kernel, run on the scratch as a 1-limb batch of that limb.
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_rescale_inv_frame_kernel(const uint64_t *in, uint64_t *scratch,
+                                                                          const uint64_t *__restrict__ roots,
+                                                                          const uint64_t *__restrict__ precons,
+                                                                          const RnsLimb64 *__restrict__ last, uint32_t L,
+                                                                          uint32_t logn) {
+    const uint32_t split = logn - ref_frame_lg<NT>();
+    const size_t b = split ? blockIdx.x >> 1 : blockIdx.x;
+    ref_u64_inv_frame_body<NT>(in + ((b * L + L - 1) << logn), nullptr, scratch + (b << logn), roots, precons,
+                               RefInvLimb{last, __ldg(&last->p.q)}, logn, 0, split ? blockIdx.x & 1u : 0u);
+}
+
+__global__ void __launch_bounds__(256) ref_inv_u64_rescale_kernel(const uint64_t *in, uint64_t *scratch,
+                                                                  const uint64_t *__restrict__ roots,
+                                                                  const uint64_t *__restrict__ precons,
+                                                                  const RnsLimb64 *__restrict__ last, uint32_t L, uint32_t logn) {
+    const size_t b = blockIdx.x;
+    ref_inv_u64_body(in + ((b * L + L - 1) << logn), nullptr, scratch + (b << logn), roots, precons,
+                     RefInvLimb{last, __ldg(&last->p.q)}, logn, 0);
+}
+
+// Evaluation form, step 2: the forward transform of r_i = (u - h) mod q_i under limb i's tables, with its input computed
+// on the fly from the scratch row of polynomial b and its output merged with the caller's spectrum in the store:
+//   out[b][i] = (x_hat_i - NTT_i(r_i)) * q_L'^-1  mod q_i.
+// Frame f < B * (L - 1) is limb i = f mod (L - 1) of polynomial b = f / (L - 1).  roots / precons: the library's forward
+// tables, offset here by i * N.
+// TWIN: a copy of ref_u64_frame_body (split = 1 at N = 32768: two CTAs per frame, each reading both halves of the
+// scratch row for stage 0) with that prologue in pass 0 and that epilogue in the final store; a fix to the transform
+// belongs in both.  The output is a separate buffer from both inputs, so the split frame needs no cluster barrier.
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_rescale_fwd_kernel(const uint64_t *in, const uint64_t *scratch,
+                                                                    uint64_t *out, const uint64_t *__restrict__ roots,
+                                                                    const uint64_t *__restrict__ precons,
+                                                                    const RescaleLimb64 *__restrict__ rc, uint64_t qlast,
+                                                                    uint64_t h, uint32_t L, uint32_t logn) {
+    extern __shared__ uint64_t img[];
+    constexpr bool VEC = AGX_U64_VECTW >= 2 || (AGX_U64_VECTW == 1 && NT >= 512);   // 16-byte twiddle pairs
+    const uint32_t tid = threadIdx.x;
+    constexpr uint32_t lg = ref_frame_lg<NT>();
+    constexpr uint32_t M = 1u << lg, vthreads = M >> 4;
+    const uint32_t split = logn - lg;
+    if (split > 1) return;                                         // launch contract (never taken)
+    const uint32_t frame = split ? blockIdx.x >> 1 : blockIdx.x, half_id = split ? blockIdx.x & 1u : 0u;
+    const uint32_t limb = frame % (L - 1), b = frame / (L - 1);
+    roots += (size_t)limb << logn;
+    precons += (size_t)limb << logn;
+    const RescaleLimb64 *c = rc + limb;
+    const uint64_t q = __ldg(&c->q), twice = q << 1;
+    const uint64_t *src = scratch + ((size_t)b << logn);           // both halves of the frame come from the scratch row
+    {
+        // the epilogue's operand x_hat_i towards L2 while the transform runs: read only after the last pass, it would
+        // otherwise cost an HBM round trip at a point where this CTA has nothing else to overlap with it
+        const uint64_t *xin = in + (((size_t)b * L + limb) << logn) + (size_t)half_id * M;
+        for (uint32_t l = tid; l < M / 16; l += NT) asm volatile("prefetch.global.L2 [%0];" ::"l"(xin + 16 * l));
+    }
+    uint64_t x[16];
+
+    // ---- pass 0: stages (split ..) on index bits [lg-4, lg), coefficients from the scratch row through the prologue
+    {
+        constexpr uint32_t lo = lg - 4;
+        const uint64_t one_p = __ldg(&c->one_p), th = twice - __ldg(&c->h);
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            if (split) {
+                // stage 0 of the 32768-point frame, this CTA keeping only its half (ntt.cpp:331-369 with roots[1])
+                const uint64_t W = __ldg(roots + 1), Wp = __ldg(precons + 1);
+#pragma unroll
+                for (int k = 0; k < 16; k++) {
+                    const uint32_t i = (k << lo) + vt;
+                    uint64_t a = rescale_lift_u64(src[i], qlast, h, one_p, q, th);
+                    uint64_t bb = rescale_lift_u64(src[M + i], qlast, h, one_p, q, th);
+                    ref_bfly_u64(a, bb, W, Wp, q, twice);
+                    x[k] = half_id ? bb : a;
+                }
+            } else {
+#pragma unroll
+                for (int k = 0; k < 16; k++) {
+                    const uint32_t i = (k << lo) + vt;
+                    x[k] = rescale_lift_u64(src[i], qlast, h, one_p, q, th);
+                }
+            }
+            // this CTA's sub-transform: stage s of it is global stage s + split, group offset half_id << s
+            // (roots index = 2^(s+split) + (half_id << s) + local group)
+            ref_pass16_u64<VEC, 0>(x, roots, precons, split, half_id, q, twice);
+            uint64_t *s = img + vt + (vt >> 4);
+            constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+    }
+    __syncthreads();
+    // ---- middle passes: index bits from lg-5 down to 4, four at a time (the last one may cover fewer)
+    uint32_t s_done = 4;                                           // stages of the sub-transform finished so far
+#pragma unroll
+    for (int rem = (int)lg - 8; rem > 0; rem -= 4) {
+        const uint32_t lo = rem >= 4 ? (uint32_t)rem : 4u;
+        const uint32_t jfirst = rem >= 4 ? 0u : (uint32_t)(4 - rem);
+        const uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint32_t t_lo = vt & ((1u << lo) - 1), t_hi = vt >> lo;
+            const uint32_t idx0 = (t_hi << (lo + 4)) + t_lo;
+            uint64_t *s = img + idx0 + (idx0 >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            // twiddle index: 2^(s+split) + ((half_id << s) + group) with group = (t_hi << j) + g at local stage j
+            const uint32_t sg = s_done + split;                    // global stage of the first active local stage
+            const uint32_t th = t_hi + (half_id << (s_done - jfirst));   // the CTA's half as the top bit of the group index
+            if (jfirst == 0) ref_pass16_u64<VEC, 0>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 1) ref_pass16_u64<VEC, 1>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 2) ref_pass16_u64<VEC, 2>(x, roots, precons, sg, th, q, twice);
+            else ref_pass16_u64<VEC, 3>(x, roots, precons, sg, th, q, twice);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+        s_done += 4 - jfirst;
+        __syncthreads();
+    }
+    // ---- final pass: bits 3..0 (16 consecutive coefficients), reduction to [0,q) (ntt.cpp:377-393)
+#pragma unroll 1
+    for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+        uint64_t *s = img + vt * 17;
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = s[k];
+        ref_pass16_u64<VEC, 0>(x, roots, precons, s_done + split, vt + (half_id << s_done), q, twice);
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            s[k] = ref_csub_u64(ref_csub_u64(x[k], twice), q);
+        }
+    }
+    __syncthreads();
+    // ---- epilogue: merge with the caller's spectrum of limb i and scale by q_L'^-1; 16 reads of x_hat_i in flight per
+    // thread (M = 32 * NT: two rounds)
+    const uint64_t qinv = __ldg(&c->qinv), qinv_p = __ldg(&c->qinv_p);
+    const uint64_t *xin = in + (((size_t)b * L + limb) << logn) + (size_t)half_id * M;
+    uint64_t *dst = out + ((size_t)frame << logn) + (size_t)half_id * M;
+#pragma unroll 1
+    for (uint32_t i0 = tid; i0 < M; i0 += 16 * NT) {
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = xin[i0 + k * NT];
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            const uint32_t i = i0 + k * NT;
+            dst[i] = rescale_finish_u64(x[k], img[i + (i >> 4)], q, qinv, qinv_p);
+        }
+    }
+}
+
+// N < 1024: the same on the radix-2 forward.  TWIN: a copy of ref_fwd_u64_body (shared-memory work array) with the
+// rescale's prologue on the load and its epilogue on the store; a fix to the transform belongs in both.
+__global__ void __launch_bounds__(1024) ref_fwd_u64_rescale_kernel(const uint64_t *__restrict__ in,
+                                                                   const uint64_t *__restrict__ scratch,
+                                                                   uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
+                                                                   const uint64_t *__restrict__ precons,
+                                                                   const RescaleLimb64 *__restrict__ rc, uint64_t qlast,
+                                                                   uint64_t h, uint32_t L, uint32_t logn) {
+    extern __shared__ uint64_t s64[];
+    const uint32_t N = 1u << logn;
+    const uint32_t frame = blockIdx.x, limb = frame % (L - 1), b = frame / (L - 1);
+    roots += (size_t)limb << logn;
+    precons += (size_t)limb << logn;
+    const RescaleLimb64 *c = rc + limb;
+    const uint64_t q = __ldg(&c->q), twice = q << 1;
+    uint64_t *X = s64;
+    {
+        const uint64_t *src = scratch + ((size_t)b << logn);
+        const uint64_t one_p = __ldg(&c->one_p), th = twice - __ldg(&c->h);
+        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x)
+            X[i] = rescale_lift_u64(src[i], qlast, h, one_p, q, th);
+    }
+    __syncthreads();
+    uint32_t tlog = logn - 1;
+    for (uint32_t m = 1; m < N; m <<= 1, tlog--) {
+        const bool last = (m == N / 2);
+        for (uint32_t bf = threadIdx.x; bf < N / 2; bf += blockDim.x) {
+            const uint32_t i = bf >> tlog, j = bf & ((1u << tlog) - 1);
+            const uint32_t a0 = (i << (tlog + 1)) + j, a1 = a0 + (1u << tlog);
+            const uint64_t W = roots[m + i], Wp = precons[m + i];
+            uint64_t tx = X[a0];
+            if (tx >= twice) tx -= twice;
+            const uint64_t a = X[a1];
+            const uint64_t c1 = __umul64hi(a, Wp);
+            const uint64_t Q = W * a - c1 * q;
+            uint64_t o0 = tx + Q, o1 = tx + twice - Q;
+            if (last) {
+                if (o0 >= twice) o0 -= twice;
+                if (o0 >= q) o0 -= q;
+                if (o1 >= twice) o1 -= twice;
+                if (o1 >= q) o1 -= q;
+            }
+            X[a0] = o0; X[a1] = o1;
+        }
+        __syncthreads();
+    }
+    const uint64_t qinv = __ldg(&c->qinv), qinv_p = __ldg(&c->qinv_p);
+    const uint64_t *xin = in + (((size_t)b * L + limb) << logn);
+    uint64_t *dst = out + ((size_t)frame << logn);
+    for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) dst[i] = rescale_finish_u64(xin[i], X[i], q, qinv, qinv_p);
 }
 
 // ------------------------------------------------------------------------------------- twiddle tables on device

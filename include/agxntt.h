@@ -246,6 +246,31 @@ int agx_polymul64_by_spectrum(agx_ctx *ctx, uint64_t *d_c, const uint64_t *d_a, 
 int agx_elementwise64(agx_ctx *ctx, int op, uint64_t *d_c, const uint64_t *d_a, const uint64_t *d_b, size_t B,
                       void *stream);
 
+/* ---- u64 RNS rescale: division by the last prime with rounding, L limbs -> L - 1 (the step that brings a product back
+ * down the modulus chain; no reference counterpart).  Primes q_0 .. q_{L-1}, L >= 2, Q = prod q_l, q_L' = q_{L-1},
+ * Q' = Q / q_L', h = floor(q_L' / 2).  For each polynomial and coefficient j, X in [0, Q) is the CRT value of its L
+ * residues, and the result is
+ *     Y = floor((X + h) / q_L') mod Q'   (round half up of X / q_L'),
+ * given as its residues mod q_0 .. q_{L-2}; since Q / q_L' = Q', it is the same residue vector whether X is read in
+ * [0, Q) or centred.  In RNS form, with u = (x_{L-1} + h) mod q_L':  y_i = (x_i - (u - h)) * q_L'^-1 mod q_i, i < L - 1.
+ *
+ * d_in [B][L][n] -> d_out [B][L-1][n] over the context's first L - 1 primes.  ntt_form == 0: coefficient form (natural
+ * order) in and out; ntt_form != 0: evaluation form as agx_ntt64_fwd leaves it (bit-reversed), in and out -- the result
+ * is then agx_ntt64_fwd, over the first L - 1 primes, of the coefficient-form rescale of agx_ntt64_inv(d_in).
+ * Input words must be reduced (< q_l); results are in [0, q_i); d_in is not modified.
+ * AGX_E_INVALID, launching nothing, for: a u32 context; L < 2; a context whose last prime equals an earlier one; a null
+ * pointer with B > 0; a pointer not 16-byte aligned; B * L > 2^31 - 1; byte ranges of d_in (B * L * n words) and d_out
+ * (B * (L - 1) * n words) that overlap (in place is refused: compacting the stride from L to L - 1 would let one
+ * polynomial's CTAs overwrite input another polynomial has not read yet).  B == 0 returns AGX_OK and launches nothing.
+ * The evaluation form takes a stream-ordered scratch buffer of B * n words (cudaMallocAsync on `stream`).
+ * Launches (agx_launch_count): coefficient form 1; evaluation form 2 (the inverse of limb L - 1; the forward of every
+ * other limb with the rescale fused into its load and its store), 3 at n = 32768, where the inverse's last stage streams.
+ *
+ * The output belongs to the level below: run the other calls on it with a context created over q_0 .. q_{L-2} (with
+ * psi[0 .. L-2] when the roots were the caller's).  That context's tables are the full context's first L - 1 limbs, bit
+ * for bit, so a chain of levels is a chain of such contexts. ---- */
+int agx_rescale64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

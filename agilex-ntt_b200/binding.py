@@ -80,6 +80,8 @@ def _load() -> C.CDLL:
         "agx_polymul64_by_spectrum": [vp, vp, vp, vp, C.c_size_t, vp],
         "agx_elementwise64": [vp, C.c_int, vp, vp, vp, C.c_size_t, vp],
         "agx_rescale64": [vp, vp, vp, C.c_size_t, C.c_int, vp],
+        "agx_moddown64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_int, vp],
+        "agx_modup64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -98,7 +100,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_ntt_fwd_host agx_ntt_inv_host agx_polymul_host agx_host_alloc agx_host_free agx_fill_synthetic "
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
-           "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64").split()
+           "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64").split()
 
 _lib = None
 
@@ -428,6 +430,45 @@ class Context64:
             raise ValueError(f"out must have shape ({B}, {self.L - 1}, {self.n})")
         _ck(lib().agx_rescale64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, int(bool(ntt_form)), _stream_ptr(stream)),
             "agx_rescale64")
+        return out
+
+    def _check_dev(self, *ts):
+        for t in ts:
+            if not t.is_cuda or t.device.index != self.device:
+                raise ValueError(f"need CUDA tensors on device {self.device}")
+
+    def moddown(self, out, inp, k, ntt_form=True, stream=None):
+        """Divide by P = q_{L-k} ... q_{L-1}, the last k primes, and round (agx_moddown64): inp (B, L, n) ->
+        out (B, L - k, n), the residues of floor((X + (P - 1) / 2) / P) over the first L - k primes.  ntt_form: both in
+        evaluation form as fwd leaves them (else both in coefficient form).  k = 1 is rescale.  Reduced inputs; out must
+        not overlap inp.  The result belongs to a context over primes[:L - k] (same roots)."""
+        self._check_dev(out, inp)
+        if inp.dim() != 3 or tuple(inp.shape[1:]) != (self.L, self.n):
+            raise ValueError(f"inp must have shape (B, {self.L}, {self.n})")
+        B = inp.shape[0]
+        if not 0 < k < self.L:
+            raise ValueError(f"k must be in [1, {self.L - 1}]")
+        if tuple(out.shape) != (B, self.L - k, self.n):
+            raise ValueError(f"out must have shape ({B}, {self.L - k}, {self.n})")
+        _ck(lib().agx_moddown64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, k, int(bool(ntt_form)), _stream_ptr(stream)),
+            "agx_moddown64")
+        return out
+
+    def modup(self, out, inp, first, count, ntt_form=True, stream=None):
+        """Extend from the primes q_first .. q_{first+count-1} (product S) to all L primes (agx_modup64): inp
+        (B, count, n) -> out (B, L, n), every limb the residue of the centred lift ((X + h) mod S) - h, h = (S - 1) / 2;
+        out's limbs first .. first + count - 1 equal inp.  ntt_form: both in evaluation form (else both in coefficient
+        form).  Reduced inputs; out must not overlap inp."""
+        self._check_dev(out, inp)
+        if not (0 < count < self.L and 0 <= first <= self.L - count):
+            raise ValueError(f"need 0 < count < {self.L} and 0 <= first <= {self.L} - count")
+        if inp.dim() != 3 or tuple(inp.shape[1:]) != (count, self.n):
+            raise ValueError(f"inp must have shape (B, {count}, {self.n})")
+        B = inp.shape[0]
+        if tuple(out.shape) != (B, self.L, self.n):
+            raise ValueError(f"out must have shape ({B}, {self.L}, {self.n})")
+        _ck(lib().agx_modup64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, first, count, int(bool(ntt_form)),
+                              _stream_ptr(stream)), "agx_modup64")
         return out
 
 

@@ -104,6 +104,10 @@ struct agx_ctx {
     RnsLimb64 *d_lc64 = nullptr;                           // per-limb modulus constants
     RescaleLimb64 *d_rs64 = nullptr;                       // [L-1] rescale constants (L >= 2, q_{L-1} unlike the others)
     uint64_t rs_qlast = 0, rs_h = 0;                       // q_{L-1} and floor(q_{L-1} / 2)
+    BasisLimb64 *d_bl64 = nullptr;                         // [L] limbs, then [L][L] BasisPair64 (ModUp / ModDown)
+    BasisPair64 *d_bp64 = nullptr;                         // points into d_bl64's allocation
+    std::vector<BasisLimb64> bl64;                         // host copies of both
+    std::vector<BasisPair64> bp64;
     HostPipe pipe;
     RefState ref;
     CopyCrew *crew_in = nullptr, *crew_out = nullptr;      // created with the first pageable call
@@ -821,10 +825,14 @@ int rns_fwd_launch(agx_ctx *c, const uint64_t *in, uint64_t *out, size_t T, cuda
 }
 
 // Inverse of T frames, times d_mul on load when not null (ref_inv_launch's geometry): one launch, two at N = 32768.
-int rns_inv_launch(agx_ctx *c, const uint64_t *in, const uint64_t *mul, uint64_t *out, size_t T, cudaStream_t st) {
-    const uint32_t logn = c->logn, L = c->L;
-    const uint64_t *itw = tab64(c, 2), *ipre = tab64(c, 3);
-    const RnsLimb64 *lc = c->d_lc64;
+// The frames are a [T / count][count][n] batch over the context's limbs first .. first + count - 1 (the whole context:
+// first = 0, count = L).
+int rns_inv_launch(agx_ctx *c, const uint64_t *in, const uint64_t *mul, uint64_t *out, size_t T, cudaStream_t st,
+                   uint32_t first, uint32_t count) {
+    const uint32_t logn = c->logn, L = count;
+    const size_t toff = (size_t)first << logn;
+    const uint64_t *itw = tab64(c, 2) + toff, *ipre = tab64(c, 3) + toff;
+    const RnsLimb64 *lc = c->d_lc64 + first;
     if (logn >= 10) {
         const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
         const size_t smem = ((size_t)17 << (lg - 4)) * 8;
@@ -1036,6 +1044,141 @@ int ctx_new(agx_ctx **out, int device) {
     return AGX_OK;
 }
 
+// ModUp / ModDown (agx_modup64 / agx_moddown64).  The source limbs s0 .. s0 + m - 1 must each differ from every other
+// prime of the context: then S is invertible modulo every target and the MRC's p_j^-1 mod p_t exist.
+static_assert(kBasisMaxSrc == AGX_BASIS_MAX_SRC, "the header states the kernels' bound");
+
+bool basis_sources_distinct(const agx_ctx *c, uint32_t s0, uint32_t m) {
+    for (uint32_t t = s0; t < s0 + m; t++)
+        for (uint32_t j = 0; j < c->L; j++)
+            if (j != t && c->q64[j] == c->q64[t]) return false;
+    return true;
+}
+
+// The per-call constants from the host copy of the pairwise array: h = (S - 1) / 2 mod q_i = (S - 1) * 2^-1 mod q_i for
+// every limb (S odd), and for ModDown S^-1 mod q_i with its companion for every target.
+BasisCall64 basis_call(const agx_ctx *c, uint32_t s0, uint32_t m, bool down) {
+    typedef unsigned __int128 u128;
+    BasisCall64 cp{};
+    cp.L = c->L; cp.logn = c->logn; cp.s0 = s0; cp.m = m;
+    cp.ntgt = c->L - m;
+    cp.lift = !down && m == 1;
+    for (uint32_t i = 0; i < c->L; i++) {
+        const uint64_t q = c->bl64[i].q;
+        const BasisPair64 *row = c->bp64.data() + (size_t)i * c->L;
+        uint64_t Smod = 1 % q, Sinv = 1 % q;
+        for (uint32_t t = s0; t < s0 + m; t++) {
+            Smod = mulmod_u64(Smod, row[t].w, q);
+            Sinv = mulmod_u64(Sinv, row[t].inv, q);
+        }
+        cp.h[i] = mulmod_u64((Smod + q - 1) % q, (q + 1) / 2, q);
+        if (down && (i < s0 || i >= s0 + m)) {
+            cp.pinv[i] = Sinv;
+            cp.pinv_p[i] = (uint64_t)(((u128)Sinv << 64) / q);
+        }
+    }
+    return cp;
+}
+
+// The launches of both calls once the arguments are checked (B > 0).  in: [B][L][n] (down) or [B][m][n];
+// out: [B][L-m][n] (down) or [B][L][n].
+int basis_launch(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t s0, uint32_t m, bool down,
+                 int ntt_form, cudaStream_t st) {
+    const uint32_t logn = c->logn, L = c->L, N = c->n;
+    const BasisCall64 cp = basis_call(c, s0, m, down);
+    const BasisLimb64 *bl = c->d_bl64;
+    const BasisPair64 *bp = c->d_bp64;
+    const size_t pairs = B * N / 2;
+    const unsigned pblocks = (unsigned)std::min<size_t>((pairs + 255) / 256, (size_t)c->sms * 16);
+    if (!ntt_form) {
+        auto *o2 = reinterpret_cast<ulonglong2 *>(d_out);
+        auto *i2 = reinterpret_cast<const ulonglong2 *>(d_in);
+        if (down) basis64_coeff_kernel<true><<<pblocks, 256, 0, st>>>(o2, i2, bl, bp, cp, pairs);
+        else basis64_coeff_kernel<false><<<pblocks, 256, 0, st>>>(o2, i2, bl, bp, cp, pairs);
+        c->launches++;
+        return (int)cudaGetLastError();
+    }
+    int rc = AGX_OK;
+    if (!down)                                                     // the source spectra are the output's source limbs
+        rc = (int)cudaMemcpy2DAsync(d_out + ((size_t)s0 << logn), (size_t)L * N * sizeof(uint64_t), d_in,
+                                    (size_t)m * N * sizeof(uint64_t), (size_t)m * N * sizeof(uint64_t), B,
+                                    cudaMemcpyDeviceToDevice, st);
+    // scratch[b][t] = INTT(source limb t of polynomial b), then its digits in place; then the fused forward
+    uint64_t *tmp = nullptr;
+    if (!rc) rc = (int)cudaMallocAsync(&tmp, B * m * N * sizeof(uint64_t), st);
+    if (!rc) {
+        if (!down) {
+            rc = rns_inv_launch(c, d_in, nullptr, tmp, B * m, st, s0, m);
+        } else {
+            const uint64_t *itw = tab64(c, 2), *ipre = tab64(c, 3);
+            const RnsLimb64 *lc = c->d_lc64;
+            if (logn >= 10) {
+                const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+                const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+                const unsigned grid = (unsigned)((B * m) << split);
+                switch (lg) {
+                    case 14: ref_u64_basis_inv_frame_kernel<512><<<grid, 512, smem, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn); break;
+                    case 13: ref_u64_basis_inv_frame_kernel<256><<<grid, 256, smem, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn); break;
+                    case 12: ref_u64_basis_inv_frame_kernel<128><<<grid, 128, smem, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn); break;
+                    case 11: ref_u64_basis_inv_frame_kernel<64><<<grid, 64, smem, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn); break;
+                    default: ref_u64_basis_inv_frame_kernel<32><<<grid, 32, smem, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn); break;
+                }
+                c->launches++;
+                if (split) {                                       // the scratch as a batch of B polynomials over the m limbs
+                    const size_t units = (B * m) << (logn - 2);
+                    const unsigned blocks = (unsigned)std::min<size_t>((units + 255) / 256, (size_t)c->sms * 8);
+                    ref_u64_rns_inv_last_stage_kernel<<<blocks, 256, 0, st>>>(tmp, lc + s0, m, logn, B * m);
+                    c->launches++;
+                }
+            } else {
+                ref_inv_u64_basis_kernel<<<(unsigned)(B * m), N / 2 < 32 ? 32 : N / 2, 0, st>>>(d_in, tmp, itw, ipre, lc, L, m, logn);
+                c->launches++;
+            }
+            rc = (int)cudaGetLastError();
+        }
+    }
+    if (!rc && m >= 2) {
+        basis64_digits_kernel<<<pblocks, 256, 0, st>>>(reinterpret_cast<ulonglong2 *>(tmp), bl, bp, cp, pairs);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc) {
+        const uint64_t *tw = tab64(c, 0), *pre = tab64(c, 1);
+        const unsigned frames = (unsigned)(B * cp.ntgt);
+        if (logn >= 10) {
+            const uint32_t split = logn == 15 ? 1u : 0u, lg = logn - split;
+            const size_t smem = ((size_t)17 << (lg - 4)) * 8;
+            const unsigned grid = frames << split;
+#define AGX_BASIS_FWD(NT)                                                                                                \
+    (down ? ref_u64_basis_fwd_kernel<NT, true><<<grid, NT, smem, st>>>(d_in, tmp, d_out, tw, pre, bl, bp, cp)            \
+          : ref_u64_basis_fwd_kernel<NT, false><<<grid, NT, smem, st>>>(d_in, tmp, d_out, tw, pre, bl, bp, cp))
+            switch (lg) {
+                case 14: AGX_BASIS_FWD(512); break;
+                case 13: AGX_BASIS_FWD(256); break;
+                case 12: AGX_BASIS_FWD(128); break;
+                case 11: AGX_BASIS_FWD(64); break;
+                default: AGX_BASIS_FWD(32); break;
+            }
+#undef AGX_BASIS_FWD
+        } else {
+            const unsigned nt = N / 2 < 32 ? 32 : N / 2;
+            if (down) ref_fwd_u64_basis_kernel<true><<<frames, nt, (size_t)N * 8, st>>>(d_in, tmp, d_out, tw, pre, bl, bp, cp);
+            else ref_fwd_u64_basis_kernel<false><<<frames, nt, (size_t)N * 8, st>>>(d_in, tmp, d_out, tw, pre, bl, bp, cp);
+        }
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
+// byte ranges [p, p + words) overlap
+bool ranges_overlap(const void *a, size_t wa, const void *b, size_t wb) {
+    const uintptr_t a0 = reinterpret_cast<uintptr_t>(a), a1 = a0 + wa * sizeof(uint64_t);
+    const uintptr_t b0 = reinterpret_cast<uintptr_t>(b), b1 = b0 + wb * sizeof(uint64_t);
+    return a0 < b1 && b0 < a1;
+}
+
 }  // namespace
 
 // ================================================================================================== C ABI
@@ -1102,7 +1245,7 @@ int agx_destroy(agx_ctx *c) {
         cudaFree(c->d_tw_fwd); cudaFree(c->d_tw_inv); cudaFree(c->d_nat_fwd); cudaFree(c->d_nat_inv);
         cudaFree(c->d_twc_fwd); cudaFree(c->d_twc_inv);
         cudaFree(c->d_lc); cudaFree(c->d_sum);
-        cudaFree(c->d_tab64); cudaFree(c->d_lc64); cudaFree(c->d_rs64);
+        cudaFree(c->d_tab64); cudaFree(c->d_lc64); cudaFree(c->d_rs64); cudaFree(c->d_bl64);
 #if AGX_WITH_R16
         cudaFree(c->d_tw16_fwd); cudaFree(c->d_tw16_inv); cudaFree(c->d_u16_fwd); cudaFree(c->d_u16_inv);
 #endif
@@ -1459,6 +1602,12 @@ int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, i
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_fwd_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_rescale_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_fwd_kernel<512, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_fwd_kernel<256, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_fwd_kernel<512, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_fwd_kernel<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
     const size_t entries = (size_t)L * n;
     if (e == cudaSuccess) e = cudaMalloc(&c->d_tab64, 4 * entries * sizeof(uint64_t));
     if (e == cudaSuccess) e = cudaMalloc(&c->d_lc64, L * sizeof(RnsLimb64));
@@ -1483,6 +1632,28 @@ int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, i
         }
         e = cudaMalloc(&c->d_rs64, (L - 1) * sizeof(RescaleLimb64));
         if (e == cudaSuccess) e = cudaMemcpy(c->d_rs64, rs.data(), (L - 1) * sizeof(RescaleLimb64), cudaMemcpyHostToDevice);
+    }
+    // the basis conversions' constants (agx_modup64 / agx_moddown64): per limb q_i, floor(2^64 / q_i) and the largest
+    // multiple of q_i not above 2^63; per pair (i, j) q_j mod q_i and q_j^-1 mod q_i with their Shoup companions (the
+    // inverse is 0 where q_j = q_i: the calls refuse such source sets).  Kept on the host too, for the per-call constants.
+    if (e == cudaSuccess) {
+        c->bl64.resize(L);
+        c->bp64.resize((size_t)L * L);
+        for (uint32_t i = 0; i < L; i++) {
+            const uint64_t q = parms->q[i];
+            c->bl64[i] = BasisLimb64{q, (uint64_t)(((u128)1 << 64) / q), q * ((1ull << 63) / q)};
+            for (uint32_t j = 0; j < L; j++) {
+                const uint64_t w = parms->q[j] % q, inv = w ? powmod_u64(w, q - 2, q) : 0;
+                c->bp64[(size_t)i * L + j] = BasisPair64{w, (uint64_t)(((u128)w << 64) / q), inv, (uint64_t)(((u128)inv << 64) / q)};
+            }
+        }
+        const size_t lb = L * sizeof(BasisLimb64), pb = (size_t)L * L * sizeof(BasisPair64);
+        e = cudaMalloc(&c->d_bl64, lb + pb);
+        if (e == cudaSuccess) {
+            c->d_bp64 = reinterpret_cast<BasisPair64 *>(reinterpret_cast<char *>(c->d_bl64) + lb);
+            e = cudaMemcpy(c->d_bl64, c->bl64.data(), lb, cudaMemcpyHostToDevice);
+        }
+        if (e == cudaSuccess) e = cudaMemcpy(c->d_bp64, c->bp64.data(), pb, cudaMemcpyHostToDevice);
     }
     if (e == cudaSuccess) {
         const size_t total = 2 * entries;
@@ -1524,7 +1695,7 @@ int agx_ntt64_inv(agx_ctx *c, uint64_t *d, size_t B, void *stream) {
     if (const int rc = check_dev_call64(c, {d}, B, &T)) return rc;
     if (T == 0) return AGX_OK;
     AGX_ON_DEVICE(c);
-    return rns_inv_launch(c, d, nullptr, d, T, (cudaStream_t)stream);
+    return rns_inv_launch(c, d, nullptr, d, T, (cudaStream_t)stream, 0, c->L);
 }
 
 int agx_polymul64(agx_ctx *c, uint64_t *dc, const uint64_t *da, const uint64_t *db, size_t B, void *stream) {
@@ -1541,7 +1712,7 @@ int agx_polymul64(agx_ctx *c, uint64_t *dc, const uint64_t *da, const uint64_t *
         rc = (int)cudaMallocAsync(&tmp, T * c->n * sizeof(uint64_t), st);
         if (!rc) rc = rns_fwd_launch(c, db, tmp, T, st);
     }
-    if (!rc) rc = rns_inv_launch(c, dc, tmp ? tmp : dc, dc, T, st);
+    if (!rc) rc = rns_inv_launch(c, dc, tmp ? tmp : dc, dc, T, st, 0, c->L);
     if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
     return rc;
 }
@@ -1560,7 +1731,7 @@ int agx_polymul64_by_spectrum(agx_ctx *c, uint64_t *dc, const uint64_t *da, cons
         spec = tmp;
     }
     if (!rc) rc = rns_fwd_launch(c, da, spec, T, st);
-    if (!rc) rc = rns_inv_launch(c, spec, db_hat, dc, T, st);
+    if (!rc) rc = rns_inv_launch(c, spec, db_hat, dc, T, st, 0, c->L);
     if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }
     return rc;
 }
@@ -1664,6 +1835,32 @@ int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, i
     }
     if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
     return rc;
+}
+
+int agx_moddown64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t k, int ntt_form, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
+    const uint32_t L = c->L;
+    if (k == 0 || k >= L || !basis_sources_distinct(c, L - k, k)) return AGX_E_INVALID;
+    if (B && ranges_overlap(d_in, T * c->n, d_out, B * (L - k) * c->n)) return AGX_E_INVALID;
+    if (k > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (B == 0) return AGX_OK;
+    if (k == 1) return agx_rescale64(c, d_out, d_in, B, ntt_form, stream);   // the same division: its own kernels
+    AGX_ON_DEVICE(c);
+    return basis_launch(c, d_out, d_in, B, L - k, k, true, ntt_form, (cudaStream_t)stream);
+}
+
+int agx_modup64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t first, uint32_t count,
+                int ntt_form, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
+    const uint32_t L = c->L;
+    if (count == 0 || count >= L || first > L - count || !basis_sources_distinct(c, first, count)) return AGX_E_INVALID;
+    if (B && ranges_overlap(d_in, B * count * c->n, d_out, T * c->n)) return AGX_E_INVALID;
+    if (count > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    return basis_launch(c, d_out, d_in, B, first, count, false, ntt_form, (cudaStream_t)stream);
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

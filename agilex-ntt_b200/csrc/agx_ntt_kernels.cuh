@@ -905,6 +905,8 @@ __global__ void __launch_bounds__(256) elementwise_kernel(uint4 *c4, const uint4
 // own copy: routed through the shared body it compiles to different SASS, and the single-modulus kernels stay as they were.
 // TWIN: ref_fwd_u64_rescale_kernel (the rescale's fused forward below N = 1024) is a copy of this body with a prologue and
 // an epilogue; a fix here belongs there too.
+// TWIN: ref_fwd_u64_basis_kernel (ModUp / ModDown's fused forward below N = 1024) is another such copy; a fix here
+// belongs there too.
 __device__ __forceinline__ void ref_fwd_u64_body(const uint64_t *__restrict__ in, const uint64_t *__restrict__ in2,
                                                  uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
                                                  const uint64_t *__restrict__ precons, uint64_t q, uint32_t logn, int use_smem,
@@ -1209,6 +1211,7 @@ __device__ __forceinline__ void ref_pass16_u64(uint64_t (&x)[16], const uint64_t
 // partner has not read yet (pass 0 is the only phase that reads global memory): in place is then safe at N = 32768.
 // TWIN: ref_u64_rescale_fwd_kernel (the rescale's fused forward) is a copy of this body with a prologue in pass 0 and an
 // epilogue in the final store; a fix here belongs there too.
+// TWIN: ref_u64_basis_fwd_kernel (ModUp / ModDown's fused forward) is another such copy; a fix here belongs there too.
 template <int NT, bool PAIR = false>
 __device__ __forceinline__ void ref_u64_frame_body(const uint64_t *in, const uint64_t *in2, uint64_t *out,
                                                    const uint64_t *__restrict__ roots, const uint64_t *__restrict__ precons,
@@ -2190,6 +2193,408 @@ __global__ void __launch_bounds__(1024) ref_fwd_u64_rescale_kernel(const uint64_
     const uint64_t *xin = in + (((size_t)b * L + limb) << logn);
     uint64_t *dst = out + ((size_t)frame << logn);
     for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) dst[i] = rescale_finish_u64(xin[i], X[i], q, qinv, qinv_p);
+}
+
+// ------------------------------------------------------- u64 RNS basis conversion (ModUp / ModDown over [B][L][N])
+// Exact conversions between sub-bases of the context's primes by mixed-radix conversion (MRC), no floating point.  For m
+// source primes p_0 .. p_{m-1} (contiguous limbs s0 .. s0 + m - 1, product S) and h = (S - 1) / 2, per coefficient:
+//   1. y_t = (x_t + h) mod p_t;
+//   2. digits d_0 = y_0, d_t = (..((y_t - d_0) p_0^-1 - d_1) p_1^-1 .. - d_{t-1}) p_{t-1}^-1 mod p_t, so that
+//      V = (X + h) mod S = sum_t d_t prod_{j<t} p_j exactly (m(m-1)/2 Shoup products);
+//   3. per target prime q_i, Horner: T_i = V mod q_i = (..(d_{m-1} p_{m-2} + d_{m-2}) p_{m-3} + ..) p_0 + d_0 mod q_i
+//      (m - 1 Shoup products, and one more with 1 that reduces the sum);
+//   4. ModUp: out_i = T_i - h mod q_i, the centred lift of the source residues.  ModDown (sources = the last k limbs,
+//      S = P): out_i = (x_i + h - T_i) P^-1 mod q_i = floor((X + h) / P) mod q_i.
+// A Shoup product accepts any 64-bit word and returns [0, 2q), so Horner adds the digits (< p_t < 2^62) unreduced: the
+// sum stays below 2q_i + 2^62 < 2^64.  In step 2, d_j < 2^62 may exceed p_t: it is subtracted from y + big_t, big_t the
+// largest multiple of p_t not above 2^63 (> 2^62 > d_j), and the sum, below 2p_t + 2^63 < 2^64, goes into the product.
+constexpr uint32_t kBasisMaxSrc = 16;        // m <= 16: a coefficient's digits stay in registers (agx_modup64 / moddown64)
+constexpr uint32_t kBasisMaxLimbs = 64;      // agx_create64's limit on L
+
+struct BasisLimb64 {
+    uint64_t q;              // q_i
+    uint64_t one_p;          // floor(2^64 / q_i): Shoup companion of 1
+    uint64_t big;            // q_i * floor(2^63 / q_i)
+};
+
+// entry [i][j] of the L x L array that follows the L BasisLimb64 entries: constants modulo q_i of prime q_j
+struct BasisPair64 {
+    uint64_t w, w_p;         // q_j mod q_i and floor(w * 2^64 / q_i)
+    uint64_t inv, inv_p;     // q_j^-1 mod q_i and its companion (0 when q_j = q_i)
+};
+
+// The per-call constants, passed by value as a kernel parameter (at most ~1.5 KB): nothing is uploaded per call.
+struct BasisCall64 {
+    uint32_t L, logn;
+    uint32_t s0, m;          // source limbs s0 .. s0 + m - 1
+    uint32_t ntgt;           // target limbs: t < s0 is limb t, t >= s0 is limb t + m
+    uint32_t lift;           // 1: the forward's scratch rows hold y_0 - h ... (m = 1, no digits kernel): add h first
+    uint64_t h[kBasisMaxLimbs];                           // h mod q_i
+    uint64_t pinv[kBasisMaxLimbs], pinv_p[kBasisMaxLimbs]; // ModDown: P^-1 mod q_i and its companion
+};
+
+__device__ __forceinline__ uint32_t basis_target_limb(const BasisCall64 &cp, uint32_t t) { return t < cp.s0 ? t : t + cp.m; }
+
+// steps 1 and 2 on W lanes: d[t][w] = x_t (reduced) in, digit t out, for t < m
+template <int W>
+__device__ __forceinline__ void basis_digits_u64(uint64_t (&d)[kBasisMaxSrc][W], const BasisLimb64 *__restrict__ bl,
+                                                 const BasisPair64 *__restrict__ pr, const BasisCall64 &cp) {
+#pragma unroll
+    for (uint32_t t = 0; t < kBasisMaxSrc; t++) {
+        if (t < cp.m) {
+            const uint32_t lt = cp.s0 + t;
+            const uint64_t p = __ldg(&bl[lt].q), big = __ldg(&bl[lt].big), h = cp.h[lt];
+#pragma unroll
+            for (int w = 0; w < W; w++) d[t][w] = ref_csub_u64(d[t][w] + h, p);
+#pragma unroll
+            for (uint32_t j = 0; j < t; j++) {
+                const BasisPair64 *c = pr + (size_t)lt * cp.L + cp.s0 + j;
+                const uint64_t v = __ldg(&c->inv), vp = __ldg(&c->inv_p);
+#pragma unroll
+                for (int w = 0; w < W; w++) d[t][w] = ref_shoup_u64(d[t][w] + big - d[j][w], v, vp, p);
+            }
+#pragma unroll
+            for (int w = 0; w < W; w++) d[t][w] = ref_csub_u64(d[t][w], p);
+        }
+    }
+}
+
+// step 3 on W lanes for target limb i: T_i in [0, 2q_i)
+template <int W>
+__device__ __forceinline__ void basis_horner_u64(uint64_t (&T)[W], const uint64_t (&d)[kBasisMaxSrc][W],
+                                                 const BasisPair64 *__restrict__ row, uint64_t q, uint64_t one_p,
+                                                 const BasisCall64 &cp) {
+#pragma unroll
+    for (int w = 0; w < W; w++) T[w] = 0;
+#pragma unroll
+    for (int t = kBasisMaxSrc - 1; t >= 0; t--) {
+        if ((uint32_t)t < cp.m) {
+            if ((uint32_t)t + 1 < cp.m) {
+                const uint64_t v = __ldg(&row[cp.s0 + t].w), vp = __ldg(&row[cp.s0 + t].w_p);
+#pragma unroll
+                for (int w = 0; w < W; w++) T[w] = ref_shoup_u64(T[w], v, vp, q);
+            }
+#pragma unroll
+            for (int w = 0; w < W; w++) T[w] += d[t][w];
+        }
+    }
+#pragma unroll
+    for (int w = 0; w < W; w++) T[w] = ref_shoup_u64(T[w], 1, one_p, q);
+}
+
+// Coefficient form, one launch: grid-stride over the 16-byte pairs of one limb row of every polynomial.  A thread reads
+// its m source pairs once, forms the digits, then walks the target limbs.  DOWN: in [B][L][n] -> out [B][L-m][n];
+// else in [B][m][n] -> out [B][L][n], the source words written through to limbs s0 .. s0 + m - 1.
+template <bool DOWN>
+__global__ void __launch_bounds__(256) basis64_coeff_kernel(ulonglong2 *__restrict__ out2, const ulonglong2 *__restrict__ in2,
+                                                            const BasisLimb64 *__restrict__ bl,
+                                                            const BasisPair64 *__restrict__ pr, const __grid_constant__ BasisCall64 cp,
+                                                            size_t pairs) {
+    const uint32_t hlog = cp.logn - 1;                             // pairs per row
+    const uint32_t inL = DOWN ? cp.L : cp.m, outL = DOWN ? cp.L - cp.m : cp.L, src0 = DOWN ? cp.s0 : 0;
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < pairs; p += (size_t)gridDim.x * blockDim.x) {
+        const size_t b = p >> hlog, j = p & ((1u << hlog) - 1);
+        const ulonglong2 *row = in2 + ((b * inL) << hlog) + j;
+        ulonglong2 *dst = out2 + ((b * outL) << hlog) + j;
+        uint64_t d[kBasisMaxSrc][2];
+#pragma unroll
+        for (uint32_t t = 0; t < kBasisMaxSrc; t++) {
+            if (t < cp.m) {
+                const ulonglong2 x = row[(size_t)(src0 + t) << hlog];
+                d[t][0] = x.x;
+                d[t][1] = x.y;
+                if (!DOWN) dst[(size_t)(cp.s0 + t) << hlog] = x;
+            }
+        }
+        basis_digits_u64<2>(d, bl, pr, cp);
+        for (uint32_t t = 0; t < cp.ntgt; t++) {
+            const uint32_t i = basis_target_limb(cp, t);
+            const uint64_t q = __ldg(&bl[i].q), one_p = __ldg(&bl[i].one_p);
+            uint64_t T[2];
+            basis_horner_u64<2>(T, d, pr + (size_t)i * cp.L, q, one_p, cp);
+            const uint64_t h = cp.h[i];
+            if (DOWN) {
+                const ulonglong2 x = row[(size_t)i << hlog];
+                const uint64_t xh0 = x.x + h + (q << 1), xh1 = x.y + h + (q << 1);   // < 4q_i; T < 2q_i
+                dst[(size_t)i << hlog] = make_ulonglong2(
+                    ref_csub_u64(ref_shoup_u64(xh0 - T[0], cp.pinv[i], cp.pinv_p[i], q), q),
+                    ref_csub_u64(ref_shoup_u64(xh1 - T[1], cp.pinv[i], cp.pinv_p[i], q), q));
+            } else {
+                dst[(size_t)i << hlog] = make_ulonglong2(ref_csub_u64(ref_csub_u64(T[0], q) + q - h, q),
+                                                         ref_csub_u64(ref_csub_u64(T[1], q) + q - h, q));
+            }
+        }
+    }
+}
+
+// Evaluation form, step 2 (m >= 2): the scratch [B][m][n] of source residues in coefficient form becomes, in place, the
+// m rows of mixed-radix digits of (X + h) mod S.  Grid-stride over 16-byte pairs.
+__global__ void __launch_bounds__(256) basis64_digits_kernel(ulonglong2 *scr2, const BasisLimb64 *__restrict__ bl,
+                                                             const BasisPair64 *__restrict__ pr, const __grid_constant__ BasisCall64 cp,
+                                                             size_t pairs) {
+    const uint32_t hlog = cp.logn - 1;
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < pairs; p += (size_t)gridDim.x * blockDim.x) {
+        const size_t b = p >> hlog, j = p & ((1u << hlog) - 1);
+        ulonglong2 *row = scr2 + ((b * cp.m) << hlog) + j;
+        uint64_t d[kBasisMaxSrc][2];
+#pragma unroll
+        for (uint32_t t = 0; t < kBasisMaxSrc; t++) {
+            if (t < cp.m) {
+                const ulonglong2 x = row[(size_t)t << hlog];
+                d[t][0] = x.x;
+                d[t][1] = x.y;
+            }
+        }
+        basis_digits_u64<2>(d, bl, pr, cp);
+#pragma unroll
+        for (uint32_t t = 0; t < kBasisMaxSrc; t++)
+            if (t < cp.m) row[(size_t)t << hlog] = make_ulonglong2(d[t][0], d[t][1]);
+    }
+}
+
+// Evaluation form, step 1 of ModDown: the inverse of the last k limbs of every polynomial into the contiguous scratch
+// [B][k][n] -- ref_u64_rescale_inv_frame_kernel / ref_inv_u64_rescale_kernel from "the last limb" to "the last k limbs":
+// frame f is limb L - k + f mod k of polynomial f / k.  At N = 32768 the halves are left in [0,2q) for
+// ref_u64_rns_inv_last_stage_kernel, run on the scratch as a k-limb batch of those limbs.
+template <int NT>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_basis_inv_frame_kernel(const uint64_t *in, uint64_t *scratch,
+                                                                        const uint64_t *__restrict__ roots,
+                                                                        const uint64_t *__restrict__ precons,
+                                                                        const RnsLimb64 *__restrict__ lc, uint32_t L,
+                                                                        uint32_t k, uint32_t logn) {
+    const uint32_t split = logn - ref_frame_lg<NT>();
+    const size_t f = split ? blockIdx.x >> 1 : blockIdx.x, b = f / k;
+    const uint32_t limb = L - k + (uint32_t)(f % k);
+    const size_t toff = (size_t)limb << logn;
+    ref_u64_inv_frame_body<NT>(in + ((b * L + limb) << logn), nullptr, scratch + (f << logn), roots + toff, precons + toff,
+                               RefInvLimb{lc + limb, __ldg(&lc[limb].p.q)}, logn, 0, split ? blockIdx.x & 1u : 0u);
+}
+
+__global__ void __launch_bounds__(256) ref_inv_u64_basis_kernel(const uint64_t *in, uint64_t *scratch,
+                                                                const uint64_t *__restrict__ roots,
+                                                                const uint64_t *__restrict__ precons,
+                                                                const RnsLimb64 *__restrict__ lc, uint32_t L, uint32_t k,
+                                                                uint32_t logn) {
+    const size_t f = blockIdx.x, b = f / k;
+    const uint32_t limb = L - k + (uint32_t)(f % k);
+    const size_t toff = (size_t)limb << logn;
+    ref_inv_u64_body(in + ((b * L + limb) << logn), nullptr, scratch + (f << logn), roots + toff, precons + toff,
+                     RefInvLimb{lc + limb, __ldg(&lc[limb].p.q)}, logn, 0);
+}
+
+// The forward's input at coefficient j from the m scratch rows src[t * n + j] of one polynomial: T_i - h mod q_i as a
+// word in (0, 4q_i), the forward transform's input range.  Rows hold the digits (m >= 2), or y_0 - h when cp.lift.
+__device__ __forceinline__ uint64_t basis_lift_u64(const uint64_t *src, uint32_t j, const BasisLimb64 *__restrict__ bl,
+                                                   const BasisPair64 *__restrict__ row, const BasisCall64 &cp, uint64_t q,
+                                                   uint64_t one_p, uint64_t twice_minus_h) {
+    const uint32_t n = 1u << cp.logn;
+    uint64_t T = src[(size_t)(cp.m - 1) * n + j];
+    if (cp.lift) T = ref_csub_u64(T + cp.h[cp.s0], __ldg(&bl[cp.s0].q));
+    for (int t = (int)cp.m - 2; t >= 0; t--)
+        T = ref_shoup_u64(T, __ldg(&row[cp.s0 + t].w), __ldg(&row[cp.s0 + t].w_p), q) + src[(size_t)t * n + j];
+    return ref_shoup_u64(T, 1, one_p, q) + twice_minus_h;
+}
+
+// Evaluation form, step 3: the forward transform of T_i - h under target limb i's tables, its input computed on the fly
+// from the digit rows of polynomial b.  Frame f < B * ntgt is target t = f mod ntgt of polynomial b = f / ntgt.
+// DOWN: out[b][i] = (x_hat_i - NTT_i(T_i - h)) * P^-1 mod q_i, merged with the caller's spectrum in the store;
+// else: out[b][i] = NTT_i(T_i - h), out being [B][L][n].
+// TWIN: a copy of ref_u64_frame_body (split = 1 at N = 32768: two CTAs per frame, each reading both halves of the
+// scratch rows for stage 0) with that prologue in pass 0 and that epilogue in the final store, as
+// ref_u64_rescale_fwd_kernel is; a fix to the transform belongs in all three.
+template <int NT, bool DOWN>
+__global__ void __launch_bounds__(NT, 512 / NT) ref_u64_basis_fwd_kernel(const uint64_t *in, const uint64_t *scratch,
+                                                                  uint64_t *out, const uint64_t *__restrict__ roots,
+                                                                  const uint64_t *__restrict__ precons,
+                                                                  const BasisLimb64 *__restrict__ bl,
+                                                                  const BasisPair64 *__restrict__ pr, const __grid_constant__ BasisCall64 cp) {
+    extern __shared__ uint64_t img[];
+    constexpr bool VEC = AGX_U64_VECTW >= 2 || (AGX_U64_VECTW == 1 && NT >= 512);   // 16-byte twiddle pairs
+    const uint32_t tid = threadIdx.x, logn = cp.logn;
+    constexpr uint32_t lg = ref_frame_lg<NT>();
+    constexpr uint32_t M = 1u << lg, vthreads = M >> 4;
+    const uint32_t split = logn - lg;
+    if (split > 1) return;                                         // launch contract (never taken)
+    const uint32_t frame = split ? blockIdx.x >> 1 : blockIdx.x, half_id = split ? blockIdx.x & 1u : 0u;
+    const uint32_t b = frame / cp.ntgt, limb = basis_target_limb(cp, frame % cp.ntgt);
+    roots += (size_t)limb << logn;
+    precons += (size_t)limb << logn;
+    const BasisPair64 *row = pr + (size_t)limb * cp.L;
+    const uint64_t q = __ldg(&bl[limb].q), twice = q << 1;
+    const uint64_t *src = scratch + (((size_t)b * cp.m) << logn);  // both halves of the frame come from the scratch rows
+    if (DOWN) {
+        // the epilogue's operand x_hat_i towards L2 while the transform runs (as in ref_u64_rescale_fwd_kernel)
+        const uint64_t *xin = in + (((size_t)b * cp.L + limb) << logn) + (size_t)half_id * M;
+        for (uint32_t l = tid; l < M / 16; l += NT) asm volatile("prefetch.global.L2 [%0];" ::"l"(xin + 16 * l));
+    }
+    uint64_t x[16];
+
+    // ---- pass 0: stages (split ..) on index bits [lg-4, lg), coefficients from the scratch rows through the prologue
+    {
+        constexpr uint32_t lo = lg - 4;
+        const uint64_t one_p = __ldg(&bl[limb].one_p), th = twice - cp.h[limb];
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            if (NT == 512 && split) {                               // only NT = 512 runs N = 32768
+                // stage 0 of the 32768-point frame, this CTA keeping only its half (ntt.cpp:331-369 with roots[1])
+                const uint64_t W = __ldg(roots + 1), Wp = __ldg(precons + 1);
+#pragma unroll
+                for (int k = 0; k < 16; k++) {
+                    const uint32_t i = (k << lo) + vt;
+                    uint64_t a = basis_lift_u64(src, i, bl, row, cp, q, one_p, th);
+                    uint64_t bb = basis_lift_u64(src, M + i, bl, row, cp, q, one_p, th);
+                    ref_bfly_u64(a, bb, W, Wp, q, twice);
+                    x[k] = half_id ? bb : a;
+                }
+            } else {
+                // basis_lift_u64 on 16 coefficients at once: each Horner step's constants are loaded once
+                const uint32_t n = 1u << logn;
+                const uint64_t *top = src + (size_t)(cp.m - 1) * n + vt;
+#pragma unroll
+                for (int k = 0; k < 16; k++) x[k] = top[k << lo];
+                if (cp.lift) {
+                    const uint64_t hs = cp.h[cp.s0], ps = __ldg(&bl[cp.s0].q);
+#pragma unroll
+                    for (int k = 0; k < 16; k++) x[k] = ref_csub_u64(x[k] + hs, ps);
+                }
+#pragma unroll 1
+                for (int t = (int)cp.m - 2; t >= 0; t--) {
+                    const uint64_t w = __ldg(&row[cp.s0 + t].w), wp = __ldg(&row[cp.s0 + t].w_p);
+                    const uint64_t *dt = src + (size_t)t * n + vt;
+#pragma unroll
+                    for (int k = 0; k < 16; k++) x[k] = ref_shoup_u64(x[k], w, wp, q) + dt[k << lo];
+                }
+#pragma unroll
+                for (int k = 0; k < 16; k++) x[k] = ref_shoup_u64(x[k], 1, one_p, q) + th;
+            }
+            // this CTA's sub-transform: stage s of it is global stage s + split, group offset half_id << s
+            // (roots index = 2^(s+split) + (half_id << s) + local group)
+            ref_pass16_u64<VEC, 0>(x, roots, precons, split, half_id, q, twice);
+            uint64_t *s = img + vt + (vt >> 4);
+            constexpr uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+    }
+    __syncthreads();
+    // ---- middle passes: index bits from lg-5 down to 4, four at a time (the last one may cover fewer)
+    uint32_t s_done = 4;                                           // stages of the sub-transform finished so far
+#pragma unroll
+    for (int rem = (int)lg - 8; rem > 0; rem -= 4) {
+        const uint32_t lo = rem >= 4 ? (uint32_t)rem : 4u;
+        const uint32_t jfirst = rem >= 4 ? 0u : (uint32_t)(4 - rem);
+        const uint32_t stride = (1u << lo) + (1u << (lo - 4));
+#pragma unroll 1
+        for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+            const uint32_t t_lo = vt & ((1u << lo) - 1), t_hi = vt >> lo;
+            const uint32_t idx0 = (t_hi << (lo + 4)) + t_lo;
+            uint64_t *s = img + idx0 + (idx0 >> 4);
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = s[k * stride];
+            // twiddle index: 2^(s+split) + ((half_id << s) + group) with group = (t_hi << j) + g at local stage j
+            const uint32_t sg = s_done + split;                    // global stage of the first active local stage
+            const uint32_t th = t_hi + (half_id << (s_done - jfirst));   // the CTA's half as the top bit of the group index
+            if (jfirst == 0) ref_pass16_u64<VEC, 0>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 1) ref_pass16_u64<VEC, 1>(x, roots, precons, sg, th, q, twice);
+            else if (jfirst == 2) ref_pass16_u64<VEC, 2>(x, roots, precons, sg, th, q, twice);
+            else ref_pass16_u64<VEC, 3>(x, roots, precons, sg, th, q, twice);
+#pragma unroll
+            for (int k = 0; k < 16; k++) s[k * stride] = x[k];
+        }
+        s_done += 4 - jfirst;
+        __syncthreads();
+    }
+    // ---- final pass: bits 3..0 (16 consecutive coefficients), reduction to [0,q) (ntt.cpp:377-393)
+#pragma unroll 1
+    for (uint32_t vt = tid; vt < vthreads; vt += NT) {
+        uint64_t *s = img + vt * 17;
+#pragma unroll
+        for (int k = 0; k < 16; k++) x[k] = s[k];
+        ref_pass16_u64<VEC, 0>(x, roots, precons, s_done + split, vt + (half_id << s_done), q, twice);
+#pragma unroll
+        for (int k = 0; k < 16; k++) {
+            s[k] = ref_csub_u64(ref_csub_u64(x[k], twice), q);
+        }
+    }
+    __syncthreads();
+    // ---- epilogue.  DOWN: merge with the caller's spectrum of limb i and scale by P^-1, 16 reads of x_hat_i in flight
+    // per thread (M = 32 * NT: two rounds).  Else: store into output limb i.
+    if (DOWN) {
+        const uint64_t pinv = cp.pinv[limb], pinv_p = cp.pinv_p[limb];
+        const uint64_t *xin = in + (((size_t)b * cp.L + limb) << logn) + (size_t)half_id * M;
+        uint64_t *dst = out + ((size_t)frame << logn) + (size_t)half_id * M;
+#pragma unroll 1
+        for (uint32_t i0 = tid; i0 < M; i0 += 16 * NT) {
+#pragma unroll
+            for (int k = 0; k < 16; k++) x[k] = xin[i0 + k * NT];
+#pragma unroll
+            for (int k = 0; k < 16; k++) {
+                const uint32_t i = i0 + k * NT;
+                dst[i] = rescale_finish_u64(x[k], img[i + (i >> 4)], q, pinv, pinv_p);
+            }
+        }
+    } else {
+        uint64_t *dst = out + (((size_t)b * cp.L + limb) << logn) + (size_t)half_id * M;
+        for (uint32_t i = tid; i < M; i += NT) dst[i] = img[i + (i >> 4)];
+    }
+}
+
+// N < 1024: the same on the radix-2 forward.  TWIN: a copy of ref_fwd_u64_body (shared-memory work array) with the
+// basis conversion's prologue on the load and its epilogue on the store, as ref_fwd_u64_rescale_kernel is; a fix to the
+// transform belongs in all three.
+template <bool DOWN>
+__global__ void __launch_bounds__(1024) ref_fwd_u64_basis_kernel(const uint64_t *__restrict__ in,
+                                                                 const uint64_t *__restrict__ scratch,
+                                                                 uint64_t *__restrict__ out, const uint64_t *__restrict__ roots,
+                                                                 const uint64_t *__restrict__ precons,
+                                                                 const BasisLimb64 *__restrict__ bl,
+                                                                 const BasisPair64 *__restrict__ pr, const __grid_constant__ BasisCall64 cp) {
+    extern __shared__ uint64_t s64[];
+    const uint32_t logn = cp.logn, N = 1u << logn;
+    const uint32_t frame = blockIdx.x, b = frame / cp.ntgt, limb = basis_target_limb(cp, frame % cp.ntgt);
+    roots += (size_t)limb << logn;
+    precons += (size_t)limb << logn;
+    const uint64_t q = __ldg(&bl[limb].q), twice = q << 1;
+    uint64_t *X = s64;
+    {
+        const uint64_t *src = scratch + (((size_t)b * cp.m) << logn);
+        const BasisPair64 *row = pr + (size_t)limb * cp.L;
+        const uint64_t one_p = __ldg(&bl[limb].one_p), th = twice - cp.h[limb];
+        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) X[i] = basis_lift_u64(src, i, bl, row, cp, q, one_p, th);
+    }
+    __syncthreads();
+    uint32_t tlog = logn - 1;
+    for (uint32_t m = 1; m < N; m <<= 1, tlog--) {
+        const bool last = (m == N / 2);
+        for (uint32_t bf = threadIdx.x; bf < N / 2; bf += blockDim.x) {
+            const uint32_t i = bf >> tlog, j = bf & ((1u << tlog) - 1);
+            const uint32_t a0 = (i << (tlog + 1)) + j, a1 = a0 + (1u << tlog);
+            const uint64_t W = roots[m + i], Wp = precons[m + i];
+            uint64_t tx = X[a0];
+            if (tx >= twice) tx -= twice;
+            const uint64_t a = X[a1];
+            const uint64_t c1 = __umul64hi(a, Wp);
+            const uint64_t Q = W * a - c1 * q;
+            uint64_t o0 = tx + Q, o1 = tx + twice - Q;
+            if (last) {
+                if (o0 >= twice) o0 -= twice;
+                if (o0 >= q) o0 -= q;
+                if (o1 >= twice) o1 -= twice;
+                if (o1 >= q) o1 -= q;
+            }
+            X[a0] = o0; X[a1] = o1;
+        }
+        __syncthreads();
+    }
+    if (DOWN) {
+        const uint64_t pinv = cp.pinv[limb], pinv_p = cp.pinv_p[limb];
+        const uint64_t *xin = in + (((size_t)b * cp.L + limb) << logn);
+        uint64_t *dst = out + ((size_t)frame << logn);
+        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) dst[i] = rescale_finish_u64(xin[i], X[i], q, pinv, pinv_p);
+    } else {
+        uint64_t *dst = out + (((size_t)b * cp.L + limb) << logn);
+        for (uint32_t i = threadIdx.x; i < N; i += blockDim.x) dst[i] = X[i];
+    }
 }
 
 // ------------------------------------------------------------------------------------- twiddle tables on device

@@ -271,6 +271,48 @@ int agx_elementwise64(agx_ctx *ctx, int op, uint64_t *d_c, const uint64_t *d_a, 
  * for bit, so a chain of levels is a chain of such contexts. ---- */
 int agx_rescale64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, void *stream);
 
+/* ---- u64 RNS basis conversion: the two steps of hybrid key switching around the product with the key (no reference
+ * counterpart).  Primes q_0 .. q_{L-1}; for a set of them with product S, X in [0, S) is the CRT value of a
+ * coefficient's residues over that set and h_S = (S - 1) / 2 (every prime is odd).  Both calls are exact: mixed-radix
+ * conversion in integer arithmetic, bit for bit the stated big-int definitions (not the approximate "fast base
+ * conversion", which is off by a multiple of S).  Conventions are agx_rescale64's: device pointers 16-byte aligned,
+ * asynchronous on `stream`; inputs reduced (< q), results in [0, q); d_in is not modified; ntt_form == 0: coefficient
+ * form (natural order) in and out; ntt_form != 0: spectra as agx_ntt64_fwd leaves them, in and out, the result then being
+ * agx_ntt64_fwd of the coefficient-form result of agx_ntt64_inv(d_in), each over its own primes.  The evaluation form
+ * takes a stream-ordered scratch buffer of B * m * n words (cudaMallocAsync on `stream`; m = k or count below).
+ * Per call, the constants that depend on the source set (h mod q_i, P^-1 mod q_i) are computed on the host from a copy
+ * of the pairwise table built at agx_create64 and passed as a kernel parameter: no per-call upload.
+ *
+ * ModDown: d_in [B][L][n] -> d_out [B][L-k][n].  P = q_{L-k} .. q_{L-1} (the last k primes), Q' = q_0 .. q_{L-k-1}:
+ *     Y = floor((X + h_P) / P) mod Q',   X in [0, Q) the CRT value of the L residues,
+ * given as its residues over q_0 .. q_{L-k-1}.  k = 1 is agx_rescale64, and is served by it (same kernels, launches).
+ * The output belongs to a context over q_0 .. q_{L-k-1} (that context's tables are this one's first L - k limbs).
+ * AGX_E_INVALID, launching nothing, for: a u32 context; a null pointer with B > 0; a pointer not 16-byte aligned;
+ * B * L > 2^31 - 1; k = 0 or k >= L; two equal primes among the last k, or one of them equal to one of the first L - k;
+ * byte ranges of d_in (B * L * n words) and d_out (B * (L - k) * n words) that overlap (in place is refused, as for the
+ * rescale: the strides differ).  AGX_E_UNSUPPORTED for k > 16 (AGX_BASIS_MAX_SRC): a coefficient's k digits are kept in
+ * registers.  B == 0 returns AGX_OK and launches nothing.
+ * Launches (agx_launch_count), k >= 2: coefficient form 1; evaluation form 3 (the inverse of the last k limbs; the
+ * mixed-radix digits; the forward of the other limbs with the conversion fused into its load and its store), 4 at
+ * n = 32768, where the inverse's last stage streams.  k = 1: the rescale's (1; 2, 3 at n = 32768).
+ */
+#define AGX_BASIS_MAX_SRC 16
+int agx_moddown64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t k, int ntt_form, void *stream);
+
+/* ModUp: d_in [B][count][n] over the primes q_first .. q_{first+count-1} (product S) -> d_out [B][L][n] over all L:
+ *     X_c = ((X + h_S) mod S) - h_S,   the centred lift of the source residues, given mod every q_i;
+ * the source limbs first .. first + count - 1 of d_out equal d_in's limbs.  A key-switch digit over part of the basis
+ * thus reaches the whole extended basis Q u P.
+ * AGX_E_INVALID, launching nothing, for: a u32 context; a null pointer with B > 0; a pointer not 16-byte aligned;
+ * B * L > 2^31 - 1; count = 0, count >= L or first + count > L; two equal source primes, or a target prime equal to a
+ * source prime; overlapping byte ranges of d_in (B * count * n words) and d_out (B * L * n words).
+ * AGX_E_UNSUPPORTED for count > 16.  B == 0 returns AGX_OK and launches nothing.
+ * Launches: coefficient form 1; evaluation form 3 (the inverse of the source limbs; the digits; the forward of the
+ * target limbs), 4 at n = 32768; count = 1 needs no digits kernel: 2, 3 at n = 32768.  The evaluation form also copies
+ * the source spectra into their output limbs (one pitched device-to-device cudaMemcpy2DAsync, not a launch). ---- */
+int agx_modup64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t first, uint32_t count,
+                int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

@@ -5,6 +5,6 @@ Layout: csrc/ (CUDA kernels + the C ABI of include/agxntt.h), host/ (C++ mirror 
 a main.cpp-shaped driver), binding.py (ctypes over the C ABI), sharding.py (multi-GPU batch partition).
 The directory name carries a hyphen, so import it as `agilex_ntt_b200` (root-level alias module).
 """
-from .binding import AgxError, Context, Context64, RefPipeline, EXPORTS, error_string, lib  # noqa: F401
+from .binding import AgxError, Context, Context64, RefPipeline, EXPORTS, error_string, galois_element, lib  # noqa: F401
 from .sharding import shard_bounds, all_shards, combine_checksums  # noqa: F401
 from . import build  # noqa: F401

@@ -7,6 +7,7 @@ imported from here).
 from __future__ import annotations
 
 import ctypes as C
+import numbers
 import os
 
 import numpy as np
@@ -82,6 +83,7 @@ def _load() -> C.CDLL:
         "agx_rescale64": [vp, vp, vp, C.c_size_t, C.c_int, vp],
         "agx_moddown64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_int, vp],
         "agx_modup64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_uint32, C.c_int, vp],
+        "agx_automorph64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -100,7 +102,8 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_ntt_fwd_host agx_ntt_inv_host agx_polymul_host agx_host_alloc agx_host_free agx_fill_synthetic "
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
-           "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64").split()
+           "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
+           "agx_automorph64").split()
 
 _lib = None
 
@@ -470,6 +473,35 @@ class Context64:
         _ck(lib().agx_modup64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, first, count, int(bool(ntt_form)),
                               _stream_ptr(stream)), "agx_modup64")
         return out
+
+    def automorph(self, out, inp, galois, ntt_form=True, stream=None):
+        """Galois automorphism sigma_g: a(X) -> a(X^g) mod X^n + 1 on every limb (agx_automorph64), g odd in [1, 2n).
+        galois: one int, with inp and out of shape (B, L, n), or a sequence of G ints (at most 64), with out of shape
+        (G, B, L, n), out[t] = sigma_{galois[t]}(inp): the input is read once for all G.  galois_element(n, r) rotates the
+        slots by r steps; 2n - 1 is the conjugation.  ntt_form: both in evaluation form as fwd leaves them, where sigma_g
+        is a permutation (else both in coefficient form, where it also negates).  Reduced inputs; out must not overlap
+        inp."""
+        self._check_dev(out, inp)
+        if inp.dim() != 3 or tuple(inp.shape[1:]) != (self.L, self.n):
+            raise ValueError(f"inp must have shape (B, {self.L}, {self.n})")
+        B = inp.shape[0]
+        single = isinstance(galois, numbers.Integral)
+        gs = [int(galois)] if single else [int(g) for g in galois]
+        want = (B, self.L, self.n) if single else (len(gs), B, self.L, self.n)
+        if tuple(out.shape) != want:
+            raise ValueError(f"out must have shape {want}")
+        if any(not 0 <= g < 1 << 32 for g in gs):
+            raise ValueError("Galois elements must be 32-bit unsigned integers (odd, below 2n)")
+        arr = (C.c_uint32 * max(len(gs), 1))(*gs)
+        _ck(lib().agx_automorph64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, C.cast(arr, _u32p), len(gs),
+                                  int(bool(ntt_form)), _stream_ptr(stream)), "agx_automorph64")
+        return out
+
+
+def galois_element(n: int, step: int) -> int:
+    """The Galois element of a slot rotation by `step` on X^n + 1: 5^step mod 2n, a negative step taking the inverse of
+    5 (mod 2n).  The conjugation is 2n - 1, which no power of 5 reaches."""
+    return pow(5, int(step), 2 * int(n))
 
 
 class RefPipeline:

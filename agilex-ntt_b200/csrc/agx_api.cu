@@ -1608,6 +1608,9 @@ int agx_create64(agx_ctx **out, const agx_parms64 *parms, const uint64_t *psi, i
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_fwd_kernel<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_inv_frame_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem);
     if (e == cudaSuccess) e = cudaFuncSetAttribute(ref_u64_basis_inv_frame_kernel<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, frame_smem / 2);
+    const int automorph_smem = (16384 + 1) * 8;                        // one n = 16384 row and its q: 128 KB
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(automorph64_coeff_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, automorph_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(automorph64_coeff_cluster_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 16384 * 8);
     const size_t entries = (size_t)L * n;
     if (e == cudaSuccess) e = cudaMalloc(&c->d_tab64, 4 * entries * sizeof(uint64_t));
     if (e == cudaSuccess) e = cudaMalloc(&c->d_lc64, L * sizeof(RnsLimb64));
@@ -1861,6 +1864,46 @@ int agx_modup64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uin
     if (B == 0) return AGX_OK;
     AGX_ON_DEVICE(c);
     return basis_launch(c, d_out, d_in, B, first, count, false, ntt_form, (cudaStream_t)stream);
+}
+
+static_assert(kAutomorphMax == AGX_AUTOMORPH_MAX, "the header states the call's bound");
+
+int agx_automorph64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                    int ntt_form, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
+    if (G && !galois) return AGX_E_INVALID;
+    if (T && (size_t)G > 0x7fffffffull / T) return AGX_E_INVALID;
+    if (T && G && ranges_overlap(d_in, T * c->n, d_out, G * T * c->n)) return AGX_E_INVALID;
+    if (G > kAutomorphMax) return AGX_E_UNSUPPORTED;
+    const uint32_t m2n = 2 * c->n - 1;
+    AutomorphCall64 cp{};
+    cp.R = (uint32_t)T; cp.L = c->L; cp.logn = c->logn; cp.G = G;
+    for (uint32_t t = 0; t < G; t++) {
+        const uint32_t g = galois[t];
+        if (!(g & 1) || g > m2n) return AGX_E_INVALID;
+        uint32_t x = g;                                    // g^-1 mod 2^32 by Newton: each step doubles the correct bits
+        for (int i = 0; i < 5; i++) x *= 2 - g * x;
+        cp.gi[t] = x & m2n;
+    }
+    if (B == 0 || G == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const uint32_t logn = c->logn;
+    if (ntt_form) {
+        const size_t pairs = T * c->n / 2;
+        const unsigned blocks = (unsigned)std::min<size_t>((pairs + 255) / 256, (size_t)c->sms * 16);
+        automorph64_ntt_kernel<<<blocks, 256, 0, st>>>(reinterpret_cast<ulonglong2 *>(d_out),
+                                                       reinterpret_cast<const ulonglong2 *>(d_in), cp, pairs);
+    } else if (logn <= 14) {
+        const uint32_t rpc = (uint32_t)std::min<size_t>(std::min(kAutomorphRows, std::max(kAutomorphPart >> logn, 1u)), T);
+        const size_t smem = ((size_t)rpc * (c->n + 1)) * 8;
+        automorph64_coeff_kernel<<<(unsigned)((T + rpc - 1) / rpc), kAutomorphThreads, smem, st>>>(d_out, d_in, c->d_lc64, cp, rpc);
+    } else {
+        automorph64_coeff_cluster_kernel<2><<<(unsigned)(2 * T), kAutomorphThreads, 16384 * 8, st>>>(d_out, d_in, c->d_lc64, cp);
+    }
+    c->launches++;
+    return (int)cudaGetLastError();
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

@@ -2597,6 +2597,121 @@ __global__ void __launch_bounds__(1024) ref_fwd_u64_basis_kernel(const uint64_t 
     }
 }
 
+// ------------------------------------------------------------ u64 RNS Galois automorphisms ([B][L][N] -> [G][B][L][N])
+// sigma_g: a(X) -> a(X^g) mod X^n + 1, g odd in [1, 2n).  Both kernels work with gi = g^-1 mod 2n, the only per-element
+// value they need:
+//   coefficient form: out[j] = in[u] if u < n, else -in[u - n] mod q_l, with u = j * gi mod 2n (coefficient i goes to
+//     i * g mod 2n, and X^n = -1);
+//   evaluation form (entry k = a(psi^(2 br(k) + 1))): out[k] = in[pi_g(k)], pi_g(k) = br((g (2 br(k) + 1) mod 2n - 1) / 2),
+//     a permutation with no sign and the same on every limb.  pi_gi is its inverse, so out[pi_gi(j)] = in[j].
+// pi maps every aligned block of 2^m entries onto an aligned block of 2^m entries (an odd factor keeps the low bits of
+// 2 br(k) + 1 among the low bits, and br swaps low and high), and pi(j + 1) = pi(j) ^ 1 for even j (the top bit of
+// br(j), i.e. a summand n of 2 br(j) + 1, times odd g is again n mod 2n).  So a 16-byte input pair is a 16-byte output
+// pair, swapped when pi(j) is odd, and a warp's 32 pairs land in one aligned 512-byte block of each output.
+constexpr uint32_t kAutomorphMax = 64;       // elements per call (agx_automorph64)
+constexpr uint32_t kAutomorphThreads = 512;  // coefficient form: threads per CTA
+constexpr uint32_t kAutomorphPart = 8192;    // coefficient form, n <= 8192: words one CTA stages (64 KB)
+constexpr uint32_t kAutomorphRows = 256;     // coefficient form: most rows per CTA (n <= 32; the rows' q follow them)
+
+// The per-call constants, passed by value (272 bytes): nothing is uploaded per call.
+struct AutomorphCall64 {
+    uint32_t R;                      // rows B * L of the input; output t is rows [t * R, (t + 1) * R)
+    uint32_t L, logn, G;
+    uint32_t gi[kAutomorphMax];      // g_t^-1 mod 2n
+};
+
+__device__ __forceinline__ uint64_t automorph_neg_u64(uint64_t x, uint64_t q) { return x ? q - x : 0; }
+
+// Evaluation form, one launch: grid-stride over the 16-byte pairs of the input, each read once and written to all G
+// outputs at pi_gi.
+__global__ void __launch_bounds__(256) automorph64_ntt_kernel(ulonglong2 *__restrict__ out2, const ulonglong2 *__restrict__ in2,
+                                                              const __grid_constant__ AutomorphCall64 cp, size_t pairs) {
+    const uint32_t hlog = cp.logn - 1, sh = 32 - cp.logn, m2n = (2u << cp.logn) - 1;
+    for (size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x; p < pairs; p += (size_t)gridDim.x * blockDim.x) {
+        const ulonglong2 x = in2[p];
+        const uint32_t h = (uint32_t)p & ((1u << hlog) - 1);       // pair within the row: words j = 2h, 2h + 1
+        const size_t row = p - h;
+        const uint32_t e = ((__brev(2 * h) >> sh) << 1) | 1;       // 2 br(j) + 1
+        for (uint32_t t = 0; t < cp.G; t++) {
+            const uint32_t d = __brev(((cp.gi[t] * e) & m2n) >> 1) >> sh;   // pi_gi(j); word j + 1 goes to d ^ 1
+            out2[t * pairs + row + (d >> 1)] = (d & 1) ? make_ulonglong2(x.y, x.x) : x;
+        }
+    }
+}
+
+// Coefficient form, n <= 16384, one launch: a CTA stages `rpc` whole rows (at most kAutomorphPart words, or one row of
+// 16384 words: 128 KB) and their q in shared memory, then writes its rows of every output coalesced.  The gather reads shared memory at the odd stride gi,
+// so a half-warp's 8-byte reads hit 16 distinct bank pairs; the wrap mod n subtracts a multiple of 16 words.
+__global__ void __launch_bounds__(kAutomorphThreads, 3) automorph64_coeff_kernel(uint64_t *__restrict__ out, const uint64_t *__restrict__ in,
+                                                                                const RnsLimb64 *__restrict__ lc,
+                                                                                const __grid_constant__ AutomorphCall64 cp,
+                                                                                uint32_t rpc) {
+    extern __shared__ __align__(16) uint64_t srow[];              // [rpc][n] words, then [rpc] q
+    const uint32_t logn = cp.logn, n = 1u << logn, m2n = 2 * n - 1;
+    const uint32_t r0 = blockIdx.x * rpc, rows = min(rpc, cp.R - r0), words = rows << logn;
+    uint64_t *sq = srow + ((size_t)rpc << logn);
+    const ulonglong2 *src = reinterpret_cast<const ulonglong2 *>(in + ((size_t)r0 << logn));
+#pragma unroll 4
+    for (uint32_t i = threadIdx.x; i < words / 2; i += kAutomorphThreads) reinterpret_cast<ulonglong2 *>(srow)[i] = src[i];
+    for (uint32_t r = threadIdx.x; r < rows; r += kAutomorphThreads) sq[r] = __ldg(&lc[(r0 + r) % cp.L].p.q);
+    __syncthreads();
+    for (uint32_t t = 0; t < cp.G; t++) {
+        const uint32_t gi = cp.gi[t];
+        uint64_t *dst = out + (((size_t)t * cp.R + r0) << logn);
+#pragma unroll 4
+        for (uint32_t w = threadIdx.x; w < words; w += kAutomorphThreads) {
+            const uint32_t j = w & (n - 1), u = (j * gi) & m2n;
+            const uint64_t x = srow[(w - j) | (u & (n - 1))];
+            dst[w] = (u & n) ? automorph_neg_u64(x, sq[w >> logn]) : x;
+        }
+    }
+}
+
+// a word of CTA `rank`'s shared memory in this cluster, at the shared::cta address `saddr` of the same variable here
+__device__ __forceinline__ uint64_t ld_dsmem_u64(uint32_t saddr, uint32_t rank) {
+    uint32_t a;
+    uint64_t v;
+    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(a) : "r"(saddr), "r"(rank));
+    asm volatile("ld.shared::cluster.u64 %0, [%1];" : "=l"(v) : "r"(a));
+    return v;
+}
+
+__device__ __forceinline__ void automorph_cluster_sync() {
+    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
+}
+
+// Coefficient form, n = 32768, one launch: a row over a cluster of CL CTAs (a row of 256 KB fits no CTA).  CTA `rank`
+// stages words [rank * part, (rank + 1) * part) of the row and writes the same words of every output, gathering through
+// distributed shared memory.  The second cluster barrier keeps every CTA resident until all partners have finished
+// reading it.
+template <int CL>
+__global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kAutomorphThreads, 3)
+    automorph64_coeff_cluster_kernel(uint64_t *__restrict__ out, const uint64_t *__restrict__ in,
+                                     const RnsLimb64 *__restrict__ lc, const __grid_constant__ AutomorphCall64 cp) {
+    constexpr uint32_t part = 32768 / CL;
+    extern __shared__ __align__(16) uint64_t srow[];              // this CTA's part of the row
+    const uint32_t logn = cp.logn, n = 1u << logn, m2n = 2 * n - 1;
+    const uint32_t rank = blockIdx.x % CL, row = blockIdx.x / CL;
+    const size_t base = ((size_t)row << logn) + rank * part;
+    const ulonglong2 *src = reinterpret_cast<const ulonglong2 *>(in + base);
+#pragma unroll 8
+    for (uint32_t i = threadIdx.x; i < part / 2; i += kAutomorphThreads) reinterpret_cast<ulonglong2 *>(srow)[i] = src[i];
+    const uint64_t q = __ldg(&lc[row % cp.L].p.q);
+    const uint32_t sbase = (uint32_t)__cvta_generic_to_shared(srow);
+    automorph_cluster_sync();                                      // every part of the row is staged
+    for (uint32_t t = 0; t < cp.G; t++) {
+        const uint32_t gi = cp.gi[t];
+        uint64_t *dst = out + (size_t)t * cp.R * n + base;
+#pragma unroll 4
+        for (uint32_t w = threadIdx.x; w < part; w += kAutomorphThreads) {
+            const uint32_t u = ((rank * part + w) * gi) & m2n, v = u & (n - 1);
+            const uint64_t x = ld_dsmem_u64(sbase + (v % part) * 8, v / part);
+            dst[w] = (u & n) ? automorph_neg_u64(x, q) : x;
+        }
+    }
+    automorph_cluster_sync();                                      // no partner still reads this CTA's shared memory
+}
+
 // ------------------------------------------------------------------------------------- twiddle tables on device
 // The step before the path: the reference fills its root / precon buffers on the host (main.cpp:46-55) and the loader
 // broadcasts them (ntt.cpp:544-571).  Here one thread per (limb, direction, k) computes

@@ -313,6 +313,32 @@ int agx_moddown64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B,
 int agx_modup64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t first, uint32_t count,
                 int ntt_form, void *stream);
 
+/* ---- u64 RNS Galois automorphisms: the permutation half of a rotation or conjugation (no reference counterpart).  For
+ * a Galois element g, odd with 1 <= g < 2n,
+ *     sigma_g: a(X) -> a(X^g) mod X^n + 1,
+ * the same map on every limb.  d_in [B][L][n] -> d_out [G][B][L][n]: output t, itself an ordinary [B][L][n] batch, is
+ * sigma_{galois[t]}(d_in).  galois is a host array of G elements; with G > 1 the input is read once for all G outputs
+ * (the hoisted rotations of key switching: one ModUp, then every rotation of the extended digit).  A slot rotation by
+ * r steps is g = 5^r mod 2n (r < 0: the inverse of 5^-r), the conjugation g = 2n - 1.
+ *   ntt_form == 0, coefficient form (natural order): coefficient i moves to i * g mod 2n; from position m >= n it goes to
+ *     m - n negated (X^n = -1), where the negation of x is q_l - x for x != 0 and 0 for x = 0.  As a gather:
+ *     out[j] = in[u] for u < n, -in[u - n] for u >= n, with u = j * g^-1 mod 2n.
+ *   ntt_form != 0, evaluation form (bit-reversed, as agx_ntt64_fwd leaves it: entry k = a(psi^(2 br(k) + 1))): a pure
+ *     permutation, no sign,
+ *     out[k] = in[br(((g * (2 br(k) + 1)) mod 2n - 1) / 2)],
+ *     equal to agx_ntt64_fwd(sigma_g(agx_ntt64_inv(d_in))) for every primitive 2n-th root, the caller's ones included.
+ * Conventions are agx_rescale64's: device pointers 16-byte aligned, asynchronous on `stream`; inputs reduced (< q_l),
+ * results in [0, q_l); d_in is not modified.  No scratch memory, no host <-> device copies; the inverses g^-1 mod 2n are
+ * passed by value as a kernel parameter.
+ * AGX_E_INVALID, launching nothing, for: a u32 context; a null device pointer with B > 0; a null galois with G > 0; a
+ * pointer not 16-byte aligned; G * B * L > 2^31 - 1; byte ranges of d_in (B * L * n words) and d_out (G * B * L * n
+ * words) that overlap (in place is refused); any element that is even, 0 or >= 2n.  AGX_E_UNSUPPORTED for G > 64
+ * (AGX_AUTOMORPH_MAX; the elements are then not read).  B == 0 or G == 0 returns AGX_OK and launches nothing.
+ * Launches: 1 per call, in both forms, at every n and every G. ---- */
+#define AGX_AUTOMORPH_MAX 64
+int agx_automorph64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                    int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

@@ -84,6 +84,7 @@ def _load() -> C.CDLL:
         "agx_moddown64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_int, vp],
         "agx_modup64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_automorph64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.c_int, vp],
+        "agx_keyswitch64": [vp, vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -103,7 +104,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
            "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
-           "agx_automorph64").split()
+           "agx_automorph64 agx_keyswitch64").split()
 
 _lib = None
 
@@ -495,6 +496,34 @@ class Context64:
         arr = (C.c_uint32 * max(len(gs), 1))(*gs)
         _ck(lib().agx_automorph64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, C.cast(arr, _u32p), len(gs),
                                   int(bool(ntt_form)), _stream_ptr(stream)), "agx_automorph64")
+        return out
+
+    def keyswitch(self, out, inp, ksk, alpha, k, ntt_form=True, stream=None):
+        """Hybrid key switching in one call (agx_keyswitch64), this context being Q_l u P with the k special primes last:
+        inp (B, L - k, n) over Q_l -> out (2, B, L - k, n), out[c] = ModDown_P(sum_j ModUp_j(digit_j) * ksk[j][c]).
+        Digit j is limbs j*alpha .. (j+1)*alpha - 1 of inp (the last one may be shorter; alpha >= L - k is one digit).
+        ksk (D, 2, key_limbs, n), D >= the number of digits, in evaluation form as fwd leaves it; key_limbs >= L: limb
+        i < L - k reads key row i, special prime t reads row key_limbs - k + t, so one key over Q_top u P serves every
+        level.  ntt_form: inp and out in evaluation form (else both in coefficient form; the key is in evaluation form
+        either way).  Reduced inputs; out must not overlap inp or ksk.  The result belongs to a context over
+        primes[:L - k]."""
+        self._check_dev(out, inp, ksk)
+        if not 0 < int(k) < self.L:
+            raise ValueError(f"k must be in [1, {self.L - 1}]")
+        alpha, k = int(alpha), int(k)
+        if not 1 <= alpha < 1 << 32:
+            raise ValueError("alpha must be a 32-bit unsigned integer, at least 1")
+        ell1 = self.L - k
+        if inp.dim() != 3 or tuple(inp.shape[1:]) != (ell1, self.n):
+            raise ValueError(f"inp must have shape (B, {ell1}, {self.n})")
+        B = inp.shape[0]
+        if tuple(out.shape) != (2, B, ell1, self.n):
+            raise ValueError(f"out must have shape (2, {B}, {ell1}, {self.n})")
+        dnum = -(-ell1 // min(alpha, ell1))
+        if ksk.dim() != 4 or ksk.shape[0] < dnum or ksk.shape[1] != 2 or ksk.shape[2] < self.L or ksk.shape[3] != self.n:
+            raise ValueError(f"ksk must have shape (D >= {dnum}, 2, key_limbs >= {self.L}, {self.n})")
+        _ck(lib().agx_keyswitch64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, _dev_ptr8(ksk), ksk.shape[2], alpha, k,
+                                  int(bool(ntt_form)), _stream_ptr(stream)), "agx_keyswitch64")
         return out
 
 

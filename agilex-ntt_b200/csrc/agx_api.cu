@@ -106,6 +106,9 @@ struct agx_ctx {
     uint64_t rs_qlast = 0, rs_h = 0;                       // q_{L-1} and floor(q_{L-1} / 2)
     BasisLimb64 *d_bl64 = nullptr;                         // [L] limbs, then [L][L] BasisPair64 (ModUp / ModDown)
     BasisPair64 *d_bp64 = nullptr;                         // points into d_bl64's allocation
+    // agx_keyswitch64's scratch (gigabytes at real batch sizes): a pool of this context that keeps its memory between
+    // calls, so that a call does not map it afresh, as the device's default pool would after every synchronisation
+    cudaMemPool_t ks_pool = nullptr;
     std::vector<BasisLimb64> bl64;                         // host copies of both
     std::vector<BasisPair64> bp64;
     HostPipe pipe;
@@ -1246,6 +1249,7 @@ int agx_destroy(agx_ctx *c) {
         cudaFree(c->d_twc_fwd); cudaFree(c->d_twc_inv);
         cudaFree(c->d_lc); cudaFree(c->d_sum);
         cudaFree(c->d_tab64); cudaFree(c->d_lc64); cudaFree(c->d_rs64); cudaFree(c->d_bl64);
+        if (c->ks_pool) cudaMemPoolDestroy(c->ks_pool);
 #if AGX_WITH_R16
         cudaFree(c->d_tw16_fwd); cudaFree(c->d_tw16_inv); cudaFree(c->d_u16_fwd); cudaFree(c->d_u16_inv);
 #endif
@@ -1904,6 +1908,80 @@ int agx_automorph64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B,
     }
     c->launches++;
     return (int)cudaGetLastError();
+}
+
+int agx_keyswitch64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint64_t *d_ksk,
+                    uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_out, (const void *)d_in, (const void *)d_ksk})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    const uint32_t L = c->L;
+    if (k == 0 || k >= L || alpha == 0 || key_limbs < L) return AGX_E_INVALID;
+    for (uint32_t i = 0; i < L; i++)                               // every prime is a digit's source or one of P's
+        for (uint32_t j = 0; j < i; j++)
+            if (c->q64[i] == c->q64[j]) return AGX_E_INVALID;
+    const uint32_t ell1 = L - k, m = std::min(alpha, ell1), dnum = (ell1 + m - 1) / m;
+    if (B > 0x7fffffffull / (2ull * L) || B > 0x7fffffffull / ((size_t)dnum * L)) return AGX_E_INVALID;
+    const size_t N = c->n;
+    if (B && (ranges_overlap(d_out, 2 * B * ell1 * N, d_in, B * ell1 * N) ||
+              ranges_overlap(d_out, 2 * B * ell1 * N, d_ksk, (size_t)dnum * 2 * key_limbs * N)))
+        return AGX_E_INVALID;
+    if (m > kBasisMaxSrc || k > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t T = B * L;
+    // scratch: U [dnum][B][L][n] (the extended digits), A [2][B][L][n] (the inner products), and with dnum > 1 one
+    // digit [B][m][n] gathered out of d_in for ModUp, which reads its source limbs contiguously
+    int rc = AGX_OK;
+    if (!c->ks_pool) {
+        cudaMemPoolProps props{};
+        props.allocType = cudaMemAllocationTypePinned;
+        props.location.type = cudaMemLocationTypeDevice;
+        props.location.id = c->device;
+        rc = (int)cudaMemPoolCreate(&c->ks_pool, &props);
+        uint64_t keep = UINT64_MAX;                                // never trimmed at synchronisation: freed at agx_destroy
+        if (!rc) rc = (int)cudaMemPoolSetAttribute(c->ks_pool, cudaMemPoolAttrReleaseThreshold, &keep);
+        if (rc) { if (c->ks_pool) cudaMemPoolDestroy(c->ks_pool); c->ks_pool = nullptr; return rc; }
+    }
+    uint64_t *U = nullptr;
+    rc = (int)cudaMallocFromPoolAsync(reinterpret_cast<void **>(&U),
+                                      ((dnum + 2) * T + (dnum > 1 ? B * m : 0)) * N * sizeof(uint64_t), c->ks_pool, st);
+    uint64_t *A = rc ? nullptr : U + dnum * T * N, *dig = rc ? nullptr : A + 2 * T * N;
+    for (uint32_t j = 0; !rc && j < dnum; j++) {
+        const uint32_t first = j * m, cnt = std::min(m, ell1 - first);
+        const uint64_t *src = d_in;
+        if (dnum > 1) {
+            rc = (int)cudaMemcpy2DAsync(dig, cnt * N * sizeof(uint64_t), d_in + first * N, ell1 * N * sizeof(uint64_t),
+                                        cnt * N * sizeof(uint64_t), B, cudaMemcpyDeviceToDevice, st);
+            src = dig;
+        }
+        if (!rc) rc = agx_modup64(c, U + j * T * N, src, B, first, cnt, ntt_form, stream);
+    }
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, U, U, dnum * T, st);   // the products are per limb in evaluation form
+    if (!rc) {
+        KeySwitchCall64 cp{};
+        cp.L = L; cp.logn = c->logn; cp.ell1 = ell1; cp.key_off = key_limbs - L; cp.key_limbs = key_limbs;
+        cp.dnum = dnum; cp.B = (uint32_t)B;
+        // slices of the batch: enough work items to fill the GPU, each reading the key once for its slice
+        const size_t per_slice = (size_t)L * N / 2, want = (size_t)c->sms * 1024;
+        const size_t S = std::min<size_t>(B, std::max<size_t>(1, (want + per_slice - 1) / per_slice));
+        cp.slice = (uint32_t)((B + S - 1) / S);
+        const size_t items = ((B + cp.slice - 1) / cp.slice) * per_slice;
+        const unsigned blocks = (unsigned)std::min<size_t>((items + 255) / 256, (size_t)c->sms * 8);
+        auto *a2 = reinterpret_cast<ulonglong2 *>(A);
+        const auto *u2 = reinterpret_cast<const ulonglong2 *>(U), *k2 = reinterpret_cast<const ulonglong2 *>(d_ksk);
+        if (dnum == 1) keyswitch64_inner_kernel<1><<<blocks, 256, 0, st>>>(a2, u2, k2, c->d_lc64, cp, items);
+        else if (dnum == 2) keyswitch64_inner_kernel<2><<<blocks, 256, 0, st>>>(a2, u2, k2, c->d_lc64, cp, items);
+        else if (dnum <= 4) keyswitch64_inner_kernel<4><<<blocks, 256, 0, st>>>(a2, u2, k2, c->d_lc64, cp, items);
+        else keyswitch64_inner_kernel<kKeySwitchChunk><<<blocks, 256, 0, st>>>(a2, u2, k2, c->d_lc64, cp, items);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc && !ntt_form) rc = rns_inv_launch(c, A, nullptr, A, 2 * T, st, 0, L);
+    if (!rc) rc = agx_moddown64(c, d_out, A, 2 * B, k, ntt_form, stream);   // both components as one batch of 2B
+    if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

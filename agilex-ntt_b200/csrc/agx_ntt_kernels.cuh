@@ -2712,6 +2712,95 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kAutomorphThreads, 
     automorph_cluster_sync();                                      // no partner still reads this CTA's shared memory
 }
 
+// ------------------------------------------------------------- u64 RNS key switching: the key inner product
+// agx_keyswitch64's one kernel of its own.  In: the dnum extended digits U[dnum][B][L][n] (ModUp's outputs, evaluation
+// form) and the key ksk[>= dnum][2][key_limbs][n]; out: A[2][B][L][n],
+//   A_c[b][i] = sum_j U_j[b][i] * ksk[j][c][row(i)]  mod q_i,   row(i) = i (i < l + 1), i + key_limbs - L (special primes).
+// A work item is one 16-byte pair of one limb row over a slice of the batch: its thread loads the key pairs of up to DC
+// digits into registers once and then walks the slice, so the key is read once per slice, not once per polynomial.
+// Each product is below q^2 < 2^124 and is added unreduced into a 128-bit sum: DC <= 8 products and a carried partial
+// sum (< q) stay below 2^128.  The sum x = hi * 2^64 + lo is then reduced exactly over its whole range by two Shoup
+// products, hi * (2^64 mod q) and lo * 1, each of which takes any 64-bit word into [0, 2q).  With dnum > DC the digits
+// run in chunks of DC, each chunk's reduced sum stored in A and carried into the next.
+constexpr uint32_t kKeySwitchChunk = 8;      // most digits a thread holds key words for at once
+
+struct KeySwitchCall64 {
+    uint32_t L, logn;
+    uint32_t ell1;           // l + 1: the limbs of Q_l, which read key rows 0 .. l
+    uint32_t key_off;        // key_limbs - L: special prime i >= l + 1 reads key row i + key_off
+    uint32_t key_limbs, dnum;
+    uint32_t B, slice;       // polynomials, and polynomials per work item
+};
+
+template <int DC>
+__global__ void __launch_bounds__(256) keyswitch64_inner_kernel(ulonglong2 *__restrict__ acc2,
+                                                                const ulonglong2 *__restrict__ u2,
+                                                                const ulonglong2 *__restrict__ k2,
+                                                                const RnsLimb64 *__restrict__ lc,
+                                                                const KeySwitchCall64 cp, size_t items) {
+    const uint32_t hlog = cp.logn - 1;
+    const size_t row2 = (size_t)1 << hlog;                         // pairs per limb row
+    const size_t poly2 = (size_t)cp.L << hlog;                     // pairs per polynomial
+    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < items; w += (size_t)gridDim.x * blockDim.x) {
+        const size_t j = w & (row2 - 1), r = w >> hlog;
+        const uint32_t i = (uint32_t)(r % cp.L);
+        const uint32_t b0 = (uint32_t)(r / cp.L) * cp.slice, b1 = min(cp.B, b0 + cp.slice);
+        const RnsLimb64 *l = lc + i;
+        const uint64_t q = __ldg(&l->p.q);
+        const RefInvConst p = RefInvLimb{l, q}.consts();
+        const uint64_t one_p = ref_shoup_companion(1, p);          // floor(2^64 / q)
+        const uint64_t r64 = 0 - one_p * q;                        // 2^64 mod q
+        const uint64_t r64_p = ref_shoup_companion(r64, p);
+        const size_t krow = i < cp.ell1 ? i : i + cp.key_off;
+        const ulonglong2 *ukey = k2 + (krow << hlog) + j;
+        const ulonglong2 *ubase = u2 + ((size_t)i << hlog) + j;
+        ulonglong2 *abase = acc2 + ((size_t)i << hlog) + j;
+        const size_t keyc = (size_t)cp.key_limbs << hlog, digit = (size_t)cp.B * poly2, comp = digit;
+        for (uint32_t d0 = 0; d0 < cp.dnum; d0 += DC) {
+            ulonglong2 kv[DC][2];
+#pragma unroll
+            for (int t = 0; t < DC; t++)
+                if (d0 + t < cp.dnum) {
+                    kv[t][0] = __ldg(ukey + (2 * (size_t)(d0 + t)) * keyc);
+                    kv[t][1] = __ldg(ukey + (2 * (size_t)(d0 + t) + 1) * keyc);
+                }
+            for (uint32_t b = b0; b < b1; b++) {
+                uint64_t lo[2][2] = {}, hi[2][2] = {};             // [component][word]
+                if (d0) {
+                    const ulonglong2 a0 = abase[b * poly2], a1 = abase[comp + b * poly2];
+                    lo[0][0] = a0.x; lo[0][1] = a0.y; lo[1][0] = a1.x; lo[1][1] = a1.y;
+                }
+#pragma unroll
+                for (int t = 0; t < DC; t++)
+                    if (d0 + t < cp.dnum) {
+                        const ulonglong2 x = __ldg(ubase + (d0 + t) * digit + b * poly2);
+                        const uint64_t xv[2] = {x.x, x.y};
+#pragma unroll
+                        for (int c = 0; c < 2; c++) {
+                            const uint64_t kw[2] = {kv[t][c].x, kv[t][c].y};
+#pragma unroll
+                            for (int v = 0; v < 2; v++) {
+                                const uint64_t pl = xv[v] * kw[v], ph = __umul64hi(xv[v], kw[v]);
+                                lo[c][v] += pl;
+                                hi[c][v] += ph + (lo[c][v] < pl);
+                            }
+                        }
+                    }
+                uint64_t y[2][2];
+#pragma unroll
+                for (int c = 0; c < 2; c++)
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        const uint64_t s = ref_shoup_u64(hi[c][v], r64, r64_p, q) + ref_shoup_u64(lo[c][v], 1, one_p, q);
+                        y[c][v] = ref_csub_u64(ref_csub_u64(s, q << 1), q);   // s < 4q
+                    }
+                abase[b * poly2] = make_ulonglong2(y[0][0], y[0][1]);
+                abase[comp + b * poly2] = make_ulonglong2(y[1][0], y[1][1]);
+            }
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------- twiddle tables on device
 // The step before the path: the reference fills its root / precon buffers on the host (main.cpp:46-55) and the loader
 // broadcasts them (ntt.cpp:544-571).  Here one thread per (limb, direction, k) computes

@@ -339,6 +339,47 @@ int agx_modup64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, u
 int agx_automorph64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
                     int ntt_form, void *stream);
 
+/* ---- u64 RNS hybrid key switching in one call (no reference counterpart): the relinearisation of a product, or the
+ * key-switch half of a rotation (agx_automorph64, then this).  ctx is a u64 context over Q_l u P, special primes last:
+ * L = l + 1 + k primes q_0 .. q_l, p_0 .. p_{k-1}.
+ *   d_in  [B][l+1][n] over Q_l, the context's first L - k primes.
+ *   Digits: digit j is limbs j*alpha .. min((j+1)*alpha, l+1) - 1 of d_in; dnum = ceil((l+1) / alpha).  alpha >= l + 1
+ *     means one digit, so a caller may keep alpha fixed as l drops below it.
+ *   d_ksk [>= dnum][2][key_limbs][n], in evaluation form as agx_ntt64_fwd leaves it under this context's roots (the key
+ *     is in evaluation form in both forms of the call); the caller guarantees dnum digits.  key_limbs >= L, and context
+ *     limb i <= l reads key row i, context limb l + 1 + t (special prime p_t) reads key row key_limbs - k + t.  So
+ *     key_limbs = L is a key over exactly this basis, and key_limbs = L_top + k is one key over Q_top u P, generated
+ *     once and used unchanged at every level l <= L_top - 1.
+ *   d_out [2][B][l+1][n], for c = 0, 1:
+ *     out_c = ModDown_P( sum_j ModUp_j(digit_j) (.) ksk[j][c] ),
+ *   ModUp_j = agx_modup64(first = j*alpha, count = the digit's size), ModDown_P = agx_moddown64(k), (.) the product of
+ *   each limb with its key row: element-wise in evaluation form, the negacyclic product in coefficient form.  Every
+ *   step is exact: the result equals, bit for bit, that sequence of public calls with the key rows sliced out of d_ksk
+ *   and replicated over the batch.  The output belongs to the context over Q_l.
+ *   ntt_form != 0: d_in and d_out are spectra; ntt_form == 0: both in natural coefficient order, d_out then being
+ *   agx_ntt64_inv (over Q_l) of the evaluation form applied to agx_ntt64_fwd(d_in).
+ * Conventions are agx_moddown64's: device pointers 16-byte aligned, asynchronous on `stream`; inputs reduced, results in
+ * [0, q); d_in and d_ksk are not modified.  Scratch: one stream-ordered buffer (cudaMallocFromPoolAsync on `stream`)
+ * of (dnum + 2) * B * L * n words, plus B * min(alpha, l+1) * n when dnum > 1, plus what the ModUps and the ModDown take
+ * (see above) while they run.  The buffer comes from a memory pool the context creates at its first key switch and
+ * keeps until agx_destroy: the pool holds on to the largest scratch a call has used, so later calls do not map it
+ * again (the device's default pool returns freed memory at every synchronisation, and mapping gigabytes per call
+ * doubled the time of a call at the sizes measured in DESIGN.md).  The digits' constants come from the host copy of the pairwise table: no per-call upload,
+ * no host synchronisation.  With dnum > 1 each digit is first gathered into the scratch by one pitched
+ * cudaMemcpy2DAsync (not a launch).
+ * AGX_E_INVALID, launching nothing, for: a u32 context; a null pointer with B > 0; a pointer not 16-byte aligned;
+ * k = 0 or k >= L; alpha = 0; key_limbs < L; two equal primes anywhere in the context; 2 * B * L or dnum * B * L above
+ * 2^31 - 1; d_out (2 * B * (l+1) * n words) overlapping d_in (B * (l+1) * n words) or the dnum digits of d_ksk that are
+ * read (dnum * 2 * key_limbs * n words).  AGX_E_UNSUPPORTED for min(alpha, l+1) > 16 or k > 16 (AGX_BASIS_MAX_SRC).
+ * B == 0 returns AGX_OK and launches nothing.
+ * Launches (agx_launch_count): evaluation form sum_j up_j + 1 + down, with up_j the ModUp's launches for digit j (3; 2
+ * for a one-prime digit; one more each at n = 32768) and down the ModDown's (3, or 2 for k = 1; one more at n = 32768):
+ * 3 * dnum + 4 for digits of two or more primes and k >= 2, 4 * dnum + 5 at n = 32768.  Coefficient form
+ * dnum + 4 (one ModUp per digit; the forward of every extended digit; the inner product; the inverse of the two
+ * products; the ModDown), dnum + 5 at n = 32768. ---- */
+int agx_keyswitch64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint64_t *d_ksk,
+                    uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

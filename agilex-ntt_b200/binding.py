@@ -85,6 +85,8 @@ def _load() -> C.CDLL:
         "agx_modup64": [vp, vp, vp, C.c_size_t, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_automorph64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.c_int, vp],
         "agx_keyswitch64": [vp, vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
+        "agx_rotate64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.POINTER(vp), C.c_uint32, C.c_uint32, C.c_uint32,
+                         C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -104,7 +106,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
            "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
-           "agx_automorph64 agx_keyswitch64").split()
+           "agx_automorph64 agx_keyswitch64 agx_rotate64").split()
 
 _lib = None
 
@@ -524,6 +526,48 @@ class Context64:
             raise ValueError(f"ksk must have shape (D >= {dnum}, 2, key_limbs >= {self.L}, {self.n})")
         _ck(lib().agx_keyswitch64(self._h, _dev_ptr8(out), _dev_ptr8(inp), B, _dev_ptr8(ksk), ksk.shape[2], alpha, k,
                                   int(bool(ntt_form)), _stream_ptr(stream)), "agx_keyswitch64")
+        return out
+
+    def rotate(self, out, ct, galois, rks, alpha, k, ntt_form=True, stream=None):
+        """Hoisted rotations in one call (agx_rotate64), this context being Q_l u P with the k special primes last:
+        ct (2, B, L - k, n), ciphertexts (c0, c1) over Q_l.  galois: one int with out of shape (2, B, L - k, n), or a
+        sequence of G ints (at most 64) with out of shape (G, 2, B, L - k, n); rks: a sequence of G keys (D, 2, key_limbs,
+        n) with one key_limbs, key t switching sigma_{galois[t]}(s) to s, laid out as for keyswitch (the same tensor may
+        serve several elements).  out[t] = (sigma_t(c0) + KS_t(sigma_t(c1))[0], KS_t(sigma_t(c1))[1]), bit for bit what
+        automorph, keyswitch with rks[t] and an elementwise add give, with one ModUp of c1 for all G.  ntt_form: ct and
+        out in evaluation form (else both in coefficient form; the keys are in evaluation form either way).  out must
+        not overlap ct or the keys.  The result belongs to a context over primes[:L - k]."""
+        single = isinstance(galois, numbers.Integral)
+        gs = [int(galois)] if single else [int(g) for g in galois]
+        rks = list(rks)
+        self._check_dev(out, ct, *rks)
+        if not 0 < int(k) < self.L:
+            raise ValueError(f"k must be in [1, {self.L - 1}]")
+        alpha, k = int(alpha), int(k)
+        if not 1 <= alpha < 1 << 32:
+            raise ValueError("alpha must be a 32-bit unsigned integer, at least 1")
+        ell1 = self.L - k
+        if ct.dim() != 4 or ct.shape[0] != 2 or tuple(ct.shape[2:]) != (ell1, self.n):
+            raise ValueError(f"ct must have shape (2, B, {ell1}, {self.n})")
+        B = ct.shape[1]
+        want = (2, B, ell1, self.n) if single else (len(gs), 2, B, ell1, self.n)
+        if tuple(out.shape) != want:
+            raise ValueError(f"out must have shape {want}")
+        if any(not 0 <= g < 1 << 32 for g in gs):
+            raise ValueError("Galois elements must be 32-bit unsigned integers (odd, below 2n)")
+        if len(rks) != len(gs):
+            raise ValueError(f"rks must hold one key per Galois element ({len(gs)})")
+        dnum = -(-ell1 // min(alpha, ell1))
+        key_limbs = rks[0].shape[2] if rks and rks[0].dim() == 4 else 0
+        for rk in rks:
+            if rk.dim() != 4 or rk.shape[0] < dnum or rk.shape[1] != 2 or rk.shape[2] != key_limbs or \
+                    key_limbs < self.L or rk.shape[3] != self.n:
+                raise ValueError(f"every key must have shape (D >= {dnum}, 2, key_limbs >= {self.L}, {self.n}), "
+                                 "with one key_limbs for all")
+        arr = (C.c_uint32 * max(len(gs), 1))(*gs)
+        ptrs = (C.c_void_p * max(len(rks), 1))(*[_dev_ptr8(rk) for rk in rks])
+        _ck(lib().agx_rotate64(self._h, _dev_ptr8(out), _dev_ptr8(ct), B, C.cast(arr, _u32p), len(gs), ptrs, key_limbs,
+                               alpha, k, int(bool(ntt_form)), _stream_ptr(stream)), "agx_rotate64")
         return out
 
 

@@ -803,12 +803,15 @@ int ref_inv_check(agx_ctx *c, uint32_t N, std::initializer_list<const void *> pt
 // The library's tables of the u64 parameter set: forward roots, forward companions, inverse roots, inverse companions.
 const uint64_t *tab64(const agx_ctx *c, int which) { return c->d_tab64 + (size_t)which * c->L * c->n; }
 
-// Forward transform of T = B * L frames [T][n] (frame f = limb f % L), in -> out (in == out or disjoint): one launch.
-// N = 32768 runs the 2-CTA cluster kernel, which is safe in place.
-int rns_fwd_launch(agx_ctx *c, const uint64_t *in, uint64_t *out, size_t T, cudaStream_t st) {
-    const uint32_t logn = c->logn, L = c->L;
-    const uint64_t *tw = tab64(c, 0), *pre = tab64(c, 1);
-    const RnsLimb64 *lc = c->d_lc64;
+// Forward transform of T frames [T][n], in -> out (in == out or disjoint): one launch.  The frames are a
+// [T / count][count][n] batch over the context's limbs first .. first + count - 1 (the whole context: first = 0,
+// count = L).  N = 32768 runs the 2-CTA cluster kernel, which is safe in place.
+int rns_fwd_launch(agx_ctx *c, const uint64_t *in, uint64_t *out, size_t T, cudaStream_t st, uint32_t first,
+                   uint32_t count) {
+    const uint32_t logn = c->logn, L = count;
+    const size_t toff = (size_t)first << logn;
+    const uint64_t *tw = tab64(c, 0) + toff, *pre = tab64(c, 1) + toff;
+    const RnsLimb64 *lc = c->d_lc64 + first;
     const unsigned grid = (unsigned)T;
     const size_t smem = logn >= 10 ? ((size_t)17 << (std::min(logn, 14u) - 4)) * 8 : 0;
     switch (logn) {
@@ -1083,10 +1086,17 @@ BasisCall64 basis_call(const agx_ctx *c, uint32_t s0, uint32_t m, bool down) {
     return cp;
 }
 
+// Stream-ordered scratch: from `pool` when not null, else from the device's default pool.
+int scratch_alloc(uint64_t **p, size_t words, cudaMemPool_t pool, cudaStream_t st) {
+    void **v = reinterpret_cast<void **>(p);
+    const size_t bytes = words * sizeof(uint64_t);
+    return (int)(pool ? cudaMallocFromPoolAsync(v, bytes, pool, st) : cudaMallocAsync(v, bytes, st));
+}
+
 // The launches of both calls once the arguments are checked (B > 0).  in: [B][L][n] (down) or [B][m][n];
-// out: [B][L-m][n] (down) or [B][L][n].
+// out: [B][L-m][n] (down) or [B][L][n].  The evaluation form's scratch comes from `pool` (see scratch_alloc).
 int basis_launch(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t s0, uint32_t m, bool down,
-                 int ntt_form, cudaStream_t st) {
+                 int ntt_form, cudaStream_t st, cudaMemPool_t pool = nullptr) {
     const uint32_t logn = c->logn, L = c->L, N = c->n;
     const BasisCall64 cp = basis_call(c, s0, m, down);
     const BasisLimb64 *bl = c->d_bl64;
@@ -1108,7 +1118,7 @@ int basis_launch(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, ui
                                     cudaMemcpyDeviceToDevice, st);
     // scratch[b][t] = INTT(source limb t of polynomial b), then its digits in place; then the fused forward
     uint64_t *tmp = nullptr;
-    if (!rc) rc = (int)cudaMallocAsync(&tmp, B * m * N * sizeof(uint64_t), st);
+    if (!rc) rc = scratch_alloc(&tmp, B * m * N, pool, st);
     if (!rc) {
         if (!down) {
             rc = rns_inv_launch(c, d_in, nullptr, tmp, B * m, st, s0, m);
@@ -1180,6 +1190,73 @@ bool ranges_overlap(const void *a, size_t wa, const void *b, size_t wb) {
     const uintptr_t a0 = reinterpret_cast<uintptr_t>(a), a1 = a0 + wa * sizeof(uint64_t);
     const uintptr_t b0 = reinterpret_cast<uintptr_t>(b), b1 = b0 + wb * sizeof(uint64_t);
     return a0 < b1 && b0 < a1;
+}
+
+// Galois elements of agx_automorph64 and agx_rotate64: false unless every g_t is odd and in [1, 2n); gi[t] = g_t^-1 mod 2n.
+bool galois_inverses(const agx_ctx *c, const uint32_t *galois, uint32_t G, uint32_t *gi) {
+    const uint32_t m2n = 2 * c->n - 1;
+    for (uint32_t t = 0; t < G; t++) {
+        const uint32_t g = galois[t];
+        if (!(g & 1) || g > m2n) return false;
+        uint32_t x = g;                                    // g^-1 mod 2^32 by Newton: each step doubles the correct bits
+        for (int i = 0; i < 5; i++) x *= 2 - g * x;
+        gi[t] = x & m2n;
+    }
+    return true;
+}
+
+// The key-switch scratch pool of the context (agx_keyswitch64, agx_rotate64): gigabytes at real batch sizes, kept
+// between calls so that a call does not map it afresh, as the device's default pool would after every synchronisation.
+int ks_pool_ready(agx_ctx *c) {
+    if (c->ks_pool) return AGX_OK;
+    cudaMemPoolProps props{};
+    props.allocType = cudaMemAllocationTypePinned;
+    props.location.type = cudaMemLocationTypeDevice;
+    props.location.id = c->device;
+    int rc = (int)cudaMemPoolCreate(&c->ks_pool, &props);
+    uint64_t keep = UINT64_MAX;                                    // never trimmed at synchronisation: freed at agx_destroy
+    if (!rc) rc = (int)cudaMemPoolSetAttribute(c->ks_pool, cudaMemPoolAttrReleaseThreshold, &keep);
+    if (rc) { if (c->ks_pool) cudaMemPoolDestroy(c->ks_pool); c->ks_pool = nullptr; }
+    return rc;
+}
+
+// ModUp of the dnum gadget digits of d_in[B][l+1][n] (digit j: limbs j*m .. min((j+1)*m, l+1) - 1) into
+// U[dnum][B][L][n].  With dnum > 1 each digit is first gathered into dig[B][m][n] by one pitched copy, since ModUp
+// reads its source limbs contiguously.
+int ks_modup_digits(agx_ctx *c, uint64_t *U, uint64_t *dig, const uint64_t *d_in, size_t B, uint32_t ell1, uint32_t m,
+                    uint32_t dnum, int ntt_form, cudaStream_t st) {
+    const size_t N = c->n, T = B * c->L;
+    int rc = AGX_OK;
+    for (uint32_t j = 0; !rc && j < dnum; j++) {
+        const uint32_t first = j * m, cnt = std::min(m, ell1 - first);
+        const uint64_t *src = d_in;
+        if (dnum > 1) {
+            rc = (int)cudaMemcpy2DAsync(dig, cnt * N * sizeof(uint64_t), d_in + first * N, ell1 * N * sizeof(uint64_t),
+                                        cnt * N * sizeof(uint64_t), B, cudaMemcpyDeviceToDevice, st);
+            src = dig;
+        }
+        if (!rc) rc = agx_modup64(c, U + j * T * N, src, B, first, cnt, ntt_form, st);
+    }
+    return rc;
+}
+
+// The key-switch parameters of agx_keyswitch64 and agx_rotate64 against a u64 context over Q_l u P: 0 < k < L,
+// alpha > 0, key_limbs >= L, and no two equal primes (every prime is a digit's source or one of P's).
+bool ks_params_valid(const agx_ctx *c, uint32_t key_limbs, uint32_t alpha, uint32_t k) {
+    const uint32_t L = c->L;
+    if (k == 0 || k >= L || alpha == 0 || key_limbs < L) return false;
+    for (uint32_t i = 0; i < L; i++)
+        for (uint32_t j = 0; j < i; j++)
+            if (c->q64[i] == c->q64[j]) return false;
+    return true;
+}
+
+// Slices of the batch for the key inner products: enough work items to fill the GPU, each reading its key words once
+// for its slice.  per_slice: work items per slice.  Returns polynomials per slice.
+uint32_t ks_slice(const agx_ctx *c, size_t B, size_t per_slice) {
+    const size_t want = (size_t)c->sms * 1024;
+    const size_t S = std::min<size_t>(B, std::max<size_t>(1, (want + per_slice - 1) / per_slice));
+    return (uint32_t)((B + S - 1) / S);
 }
 
 }  // namespace
@@ -1694,7 +1771,7 @@ int agx_ntt64_fwd(agx_ctx *c, uint64_t *d, size_t B, void *stream) {
     if (const int rc = check_dev_call64(c, {d}, B, &T)) return rc;
     if (T == 0) return AGX_OK;
     AGX_ON_DEVICE(c);
-    return rns_fwd_launch(c, d, d, T, (cudaStream_t)stream);
+    return rns_fwd_launch(c, d, d, T, (cudaStream_t)stream, 0, c->L);
 }
 
 int agx_ntt64_inv(agx_ctx *c, uint64_t *d, size_t B, void *stream) {
@@ -1714,10 +1791,10 @@ int agx_polymul64(agx_ctx *c, uint64_t *dc, const uint64_t *da, const uint64_t *
     if (dc == db && dc != da) std::swap(da, db);                   // the product commutes: c == a from here on
     // c = NTT(a); scratch = NTT(b) unless squaring; c = INTT(c .* (scratch or c))  (agx_ref_polymul_dev's sequence)
     uint64_t *tmp = nullptr;
-    int rc = rns_fwd_launch(c, da, dc, T, st);
+    int rc = rns_fwd_launch(c, da, dc, T, st, 0, c->L);
     if (!rc && da != db) {
         rc = (int)cudaMallocAsync(&tmp, T * c->n * sizeof(uint64_t), st);
-        if (!rc) rc = rns_fwd_launch(c, db, tmp, T, st);
+        if (!rc) rc = rns_fwd_launch(c, db, tmp, T, st, 0, c->L);
     }
     if (!rc) rc = rns_inv_launch(c, dc, tmp ? tmp : dc, dc, T, st, 0, c->L);
     if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }   // freed on every path
@@ -1737,7 +1814,7 @@ int agx_polymul64_by_spectrum(agx_ctx *c, uint64_t *dc, const uint64_t *da, cons
         rc = (int)cudaMallocAsync(&tmp, T * c->n * sizeof(uint64_t), st);
         spec = tmp;
     }
-    if (!rc) rc = rns_fwd_launch(c, da, spec, T, st);
+    if (!rc) rc = rns_fwd_launch(c, da, spec, T, st, 0, c->L);
     if (!rc) rc = rns_inv_launch(c, spec, db_hat, dc, T, st, 0, c->L);
     if (tmp) { const int rf = (int)cudaFreeAsync(tmp, st); if (!rc) rc = rf; }
     return rc;
@@ -1764,19 +1841,12 @@ int agx_elementwise64(agx_ctx *c, int op, uint64_t *dc, const uint64_t *da, cons
     return (int)cudaGetLastError();
 }
 
-int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, void *stream) {
-    size_t T = 0;
-    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
-    if (c->L < 2 || !c->d_rs64) return AGX_E_INVALID;
-    // in place is refused: the compaction from stride L to L - 1 lets one polynomial's CTAs overwrite input that
-    // another polynomial's CTAs have not read yet
-    const uintptr_t i0 = reinterpret_cast<uintptr_t>(d_in), i1 = i0 + T * c->n * sizeof(uint64_t);
-    const uintptr_t o0 = reinterpret_cast<uintptr_t>(d_out), o1 = o0 + (T - B) * c->n * sizeof(uint64_t);
-    if (B && i0 < o1 && o0 < i1) return AGX_E_INVALID;
-    if (B == 0) return AGX_OK;
-    AGX_ON_DEVICE(c);
-    const cudaStream_t st = (cudaStream_t)stream;
+// The launches of agx_rescale64 once the arguments are checked (B > 0); the evaluation form's scratch comes from `pool`
+// (see scratch_alloc).
+static int rescale_launch(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, cudaStream_t st,
+                          cudaMemPool_t pool) {
     const uint32_t logn = c->logn, L = c->L, N = c->n;
+    const size_t T = B * L;
     if (!ntt_form) {
         const size_t pairs = B * N / 2;
         const unsigned blocks = (unsigned)std::min<size_t>((pairs + 255) / 256, (size_t)c->sms * 16);
@@ -1788,7 +1858,7 @@ int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, i
     }
     // evaluation form: scratch[b] = INTT_{L-1}(x_hat[b][L-1]); out[b][i] = (x_hat[b][i] - NTT_i(r_i(scratch[b]))) / q_{L-1}
     uint64_t *tmp = nullptr;
-    int rc = (int)cudaMallocAsync(&tmp, B * N * sizeof(uint64_t), st);
+    int rc = scratch_alloc(&tmp, B * N, pool, st);
     if (!rc) {
         const RnsLimb64 *last = c->d_lc64 + (L - 1);
         const size_t toff = (size_t)(L - 1) * N;
@@ -1844,6 +1914,20 @@ int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, i
     return rc;
 }
 
+int agx_rescale64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, int ntt_form, void *stream) {
+    size_t T = 0;
+    if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
+    if (c->L < 2 || !c->d_rs64) return AGX_E_INVALID;
+    // in place is refused: the compaction from stride L to L - 1 lets one polynomial's CTAs overwrite input that
+    // another polynomial's CTAs have not read yet
+    const uintptr_t i0 = reinterpret_cast<uintptr_t>(d_in), i1 = i0 + T * c->n * sizeof(uint64_t);
+    const uintptr_t o0 = reinterpret_cast<uintptr_t>(d_out), o1 = o0 + (T - B) * c->n * sizeof(uint64_t);
+    if (B && i0 < o1 && o0 < i1) return AGX_E_INVALID;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    return rescale_launch(c, d_out, d_in, B, ntt_form, (cudaStream_t)stream, nullptr);
+}
+
 int agx_moddown64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t k, int ntt_form, void *stream) {
     size_t T = 0;
     if (const int rc = check_dev_call64(c, {d_out, d_in}, B, &T)) return rc;
@@ -1855,6 +1939,13 @@ int agx_moddown64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, u
     if (k == 1) return agx_rescale64(c, d_out, d_in, B, ntt_form, stream);   // the same division: its own kernels
     AGX_ON_DEVICE(c);
     return basis_launch(c, d_out, d_in, B, L - k, k, true, ntt_form, (cudaStream_t)stream);
+}
+
+// agx_moddown64's launches once the arguments are checked (B > 0), with the scratch from `pool` (see scratch_alloc).
+static int moddown_launch(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t k, int ntt_form,
+                          cudaStream_t st, cudaMemPool_t pool) {
+    if (k == 1) return rescale_launch(c, d_out, d_in, B, ntt_form, st, pool);
+    return basis_launch(c, d_out, d_in, B, c->L - k, k, true, ntt_form, st, pool);
 }
 
 int agx_modup64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, uint32_t first, uint32_t count,
@@ -1880,16 +1971,9 @@ int agx_automorph64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B,
     if (T && (size_t)G > 0x7fffffffull / T) return AGX_E_INVALID;
     if (T && G && ranges_overlap(d_in, T * c->n, d_out, G * T * c->n)) return AGX_E_INVALID;
     if (G > kAutomorphMax) return AGX_E_UNSUPPORTED;
-    const uint32_t m2n = 2 * c->n - 1;
     AutomorphCall64 cp{};
     cp.R = (uint32_t)T; cp.L = c->L; cp.logn = c->logn; cp.G = G;
-    for (uint32_t t = 0; t < G; t++) {
-        const uint32_t g = galois[t];
-        if (!(g & 1) || g > m2n) return AGX_E_INVALID;
-        uint32_t x = g;                                    // g^-1 mod 2^32 by Newton: each step doubles the correct bits
-        for (int i = 0; i < 5; i++) x *= 2 - g * x;
-        cp.gi[t] = x & m2n;
-    }
+    if (!galois_inverses(c, galois, G, cp.gi)) return AGX_E_INVALID;
     if (B == 0 || G == 0) return AGX_OK;
     AGX_ON_DEVICE(c);
     const cudaStream_t st = (cudaStream_t)stream;
@@ -1916,10 +2000,7 @@ int agx_keyswitch64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B,
     for (const void *p : {(const void *)d_out, (const void *)d_in, (const void *)d_ksk})
         if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
     const uint32_t L = c->L;
-    if (k == 0 || k >= L || alpha == 0 || key_limbs < L) return AGX_E_INVALID;
-    for (uint32_t i = 0; i < L; i++)                               // every prime is a digit's source or one of P's
-        for (uint32_t j = 0; j < i; j++)
-            if (c->q64[i] == c->q64[j]) return AGX_E_INVALID;
+    if (!ks_params_valid(c, key_limbs, alpha, k)) return AGX_E_INVALID;
     const uint32_t ell1 = L - k, m = std::min(alpha, ell1), dnum = (ell1 + m - 1) / m;
     if (B > 0x7fffffffull / (2ull * L) || B > 0x7fffffffull / ((size_t)dnum * L)) return AGX_E_INVALID;
     const size_t N = c->n;
@@ -1933,40 +2014,20 @@ int agx_keyswitch64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B,
     const size_t T = B * L;
     // scratch: U [dnum][B][L][n] (the extended digits), A [2][B][L][n] (the inner products), and with dnum > 1 one
     // digit [B][m][n] gathered out of d_in for ModUp, which reads its source limbs contiguously
-    int rc = AGX_OK;
-    if (!c->ks_pool) {
-        cudaMemPoolProps props{};
-        props.allocType = cudaMemAllocationTypePinned;
-        props.location.type = cudaMemLocationTypeDevice;
-        props.location.id = c->device;
-        rc = (int)cudaMemPoolCreate(&c->ks_pool, &props);
-        uint64_t keep = UINT64_MAX;                                // never trimmed at synchronisation: freed at agx_destroy
-        if (!rc) rc = (int)cudaMemPoolSetAttribute(c->ks_pool, cudaMemPoolAttrReleaseThreshold, &keep);
-        if (rc) { if (c->ks_pool) cudaMemPoolDestroy(c->ks_pool); c->ks_pool = nullptr; return rc; }
-    }
+    int rc = ks_pool_ready(c);
+    if (rc) return rc;
     uint64_t *U = nullptr;
     rc = (int)cudaMallocFromPoolAsync(reinterpret_cast<void **>(&U),
                                       ((dnum + 2) * T + (dnum > 1 ? B * m : 0)) * N * sizeof(uint64_t), c->ks_pool, st);
     uint64_t *A = rc ? nullptr : U + dnum * T * N, *dig = rc ? nullptr : A + 2 * T * N;
-    for (uint32_t j = 0; !rc && j < dnum; j++) {
-        const uint32_t first = j * m, cnt = std::min(m, ell1 - first);
-        const uint64_t *src = d_in;
-        if (dnum > 1) {
-            rc = (int)cudaMemcpy2DAsync(dig, cnt * N * sizeof(uint64_t), d_in + first * N, ell1 * N * sizeof(uint64_t),
-                                        cnt * N * sizeof(uint64_t), B, cudaMemcpyDeviceToDevice, st);
-            src = dig;
-        }
-        if (!rc) rc = agx_modup64(c, U + j * T * N, src, B, first, cnt, ntt_form, stream);
-    }
-    if (!rc && !ntt_form) rc = rns_fwd_launch(c, U, U, dnum * T, st);   // the products are per limb in evaluation form
+    if (!rc) rc = ks_modup_digits(c, U, dig, d_in, B, ell1, m, dnum, ntt_form, st);
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, U, U, dnum * T, st, 0, L);   // the products are per limb in evaluation form
     if (!rc) {
         KeySwitchCall64 cp{};
         cp.L = L; cp.logn = c->logn; cp.ell1 = ell1; cp.key_off = key_limbs - L; cp.key_limbs = key_limbs;
         cp.dnum = dnum; cp.B = (uint32_t)B;
-        // slices of the batch: enough work items to fill the GPU, each reading the key once for its slice
-        const size_t per_slice = (size_t)L * N / 2, want = (size_t)c->sms * 1024;
-        const size_t S = std::min<size_t>(B, std::max<size_t>(1, (want + per_slice - 1) / per_slice));
-        cp.slice = (uint32_t)((B + S - 1) / S);
+        const size_t per_slice = (size_t)L * N / 2;
+        cp.slice = ks_slice(c, B, per_slice);
         const size_t items = ((B + cp.slice - 1) / cp.slice) * per_slice;
         const unsigned blocks = (unsigned)std::min<size_t>((items + 255) / 256, (size_t)c->sms * 8);
         auto *a2 = reinterpret_cast<ulonglong2 *>(A);
@@ -1980,6 +2041,73 @@ int agx_keyswitch64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B,
     }
     if (!rc && !ntt_form) rc = rns_inv_launch(c, A, nullptr, A, 2 * T, st, 0, L);
     if (!rc) rc = agx_moddown64(c, d_out, A, 2 * B, k, ntt_form, stream);   // both components as one batch of 2B
+    if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
+int agx_rotate64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                 const uint64_t *const *d_rk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_out, (const void *)d_in})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    if (G && (!galois || !d_rk)) return AGX_E_INVALID;
+    const uint32_t L = c->L;
+    if (!ks_params_valid(c, key_limbs, alpha, k)) return AGX_E_INVALID;
+    const uint32_t ell1 = L - k, m = std::min(alpha, ell1), dnum = (ell1 + m - 1) / m;
+    if (B > 0x7fffffffull / ((size_t)dnum * L) || (B && G > 0x7fffffffull / (2ull * L * B))) return AGX_E_INVALID;
+    const size_t N = c->n;
+    const size_t in_w = 2 * B * ell1 * N, out_w = (size_t)G * in_w, key_w = (size_t)dnum * 2 * key_limbs * N;
+    if (B && G && ranges_overlap(d_out, out_w, d_in, in_w)) return AGX_E_INVALID;
+    if (G > kAutomorphMax) return AGX_E_UNSUPPORTED;               // elements and keys are not read
+    RotateCall64 cp{};
+    if (!galois_inverses(c, galois, G, cp.gi)) return AGX_E_INVALID;
+    for (uint32_t t = 0; t < G; t++) {
+        const uint64_t *rk = d_rk[t];
+        if ((B && !rk) || (reinterpret_cast<uintptr_t>(rk) & 15)) return AGX_E_INVALID;
+        if (B && ranges_overlap(d_out, out_w, rk, key_w)) return AGX_E_INVALID;
+        cp.rk[t] = reinterpret_cast<const ulonglong2 *>(rk);
+    }
+    if (m > kBasisMaxSrc || k > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (B == 0 || G == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t T = B * L;
+    // scratch: U [dnum][B][L][n] (c1's extended digits), A [G][2][B][L][n] (the inner products), with dnum > 1 one digit
+    // [B][m][n] gathered for ModUp, and in coefficient form c0's spectrum [B][l+1][n]
+    int rc = ks_pool_ready(c);
+    if (rc) return rc;
+    uint64_t *U = nullptr;
+    const size_t words = (dnum + 2 * (size_t)G) * T + (dnum > 1 ? B * m : 0) + (ntt_form ? 0 : B * ell1);
+    rc = (int)cudaMallocFromPoolAsync(reinterpret_cast<void **>(&U), words * N * sizeof(uint64_t), c->ks_pool, st);
+    uint64_t *A = rc ? nullptr : U + dnum * T * N, *dig = rc ? nullptr : A + 2 * G * T * N;
+    uint64_t *c0h = rc ? nullptr : dig + (dnum > 1 ? B * m * N : 0);
+    const uint64_t *c1 = d_in + B * ell1 * N;
+    if (!rc) rc = ks_modup_digits(c, U, dig, c1, B, ell1, m, dnum, ntt_form, st);
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, U, U, dnum * T, st, 0, L);   // the products are per limb in evaluation form
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, d_in, c0h, B * ell1, st, 0, ell1);
+    if (!rc) {
+        KeySwitchCall64 &ks = cp.ks;
+        ks.L = L; ks.logn = c->logn; ks.ell1 = ell1; ks.key_off = key_limbs - L; ks.key_limbs = key_limbs;
+        ks.dnum = dnum; ks.B = (uint32_t)B;
+        cp.G = G;
+        const size_t per_slice = (size_t)G * L * N / 2;
+        ks.slice = ks_slice(c, B, per_slice);
+        const size_t items = ((B + ks.slice - 1) / ks.slice) * per_slice;
+        const unsigned blocks = (unsigned)std::min<size_t>((items + 255) / 256, (size_t)c->sms * 8);
+        auto *a2 = reinterpret_cast<ulonglong2 *>(A);
+        const auto *u2 = reinterpret_cast<const ulonglong2 *>(U);
+        const auto *c02 = reinterpret_cast<const ulonglong2 *>(ntt_form ? d_in : c0h);
+        const BasisPair64 *bp = c->d_bp64;
+        if (dnum == 1) rotate64_inner_kernel<1><<<blocks, 256, 0, st>>>(a2, u2, c02, c->d_lc64, bp, cp, items);
+        else if (dnum == 2) rotate64_inner_kernel<2><<<blocks, 256, 0, st>>>(a2, u2, c02, c->d_lc64, bp, cp, items);
+        else if (dnum <= 4) rotate64_inner_kernel<4><<<blocks, 256, 0, st>>>(a2, u2, c02, c->d_lc64, bp, cp, items);
+        else rotate64_inner_kernel<kKeySwitchChunk><<<blocks, 256, 0, st>>>(a2, u2, c02, c->d_lc64, bp, cp, items);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc && !ntt_form) rc = rns_inv_launch(c, A, nullptr, A, 2 * G * T, st, 0, L);
+    // every output's two components as one batch of 2 G B, with its scratch from the pool too
+    if (!rc) rc = moddown_launch(c, d_out, A, 2 * G * B, k, ntt_form, st, c->ks_pool);
     if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
     return rc;
 }

@@ -2801,6 +2801,123 @@ __global__ void __launch_bounds__(256) keyswitch64_inner_kernel(ulonglong2 *__re
     }
 }
 
+// ------------------------------------------------------------- u64 RNS hoisted rotations: the G key inner products
+// agx_rotate64's one kernel of its own.  In: the dnum extended digits U[dnum][B][L][n] of c1 (ModUp's outputs), the
+// spectrum c0h[B][l+1][n] of c0 and G keys rk_t[>= dnum][2][key_limbs][n], all in evaluation form; out: A[G][2][B][L][n],
+//   A_t[c][b][i][k] = sum_j U_j[b][i][pi_t(k)] * rk_t[j][c][row(i)][k]  +  [c = 0, i <= l] (P mod q_i) c0h[b][i][pi_t(k)]
+// mod q_i, with row(i) keyswitch64_inner_kernel's and pi_t automorph64_ntt_kernel's permutation for g_t (out[k] =
+// in[pi_g(k)], i.e. input entry j lands at pi_{g^-1}(j), which is how this kernel, like that one, uses it).  ModDown of
+// A_t is sigma_t(c0) + KS_t(sigma_t(c1)): floor((X + P C + h_P) / P) = C + floor((X + h_P) / P), and P C = 0 mod p_t.
+// A work item is one 16-byte pair j of one input limb row, for one element t, over a slice of the batch.  Its thread
+// loads key t's words at the pair's destination pi_{g^-1}(j) into registers once, then walks the slice.  Items run in
+// the order (slice and limb row, 32-pair block of the input, t, pair): the G warps that read one 512-byte block of U
+// and of c0h follow one another, so each block comes from HBM once and its G - 1 re-reads from L2.  The permutation
+// maps that block onto one aligned block of every key and output, and keeps pairs together (swapped when the
+// destination word is odd), so every warp access covers whole 512-byte blocks.
+// The 128-bit lazy sum and its reduction are keyswitch64_inner_kernel's.  The first chunk holds DC <= 8 products and
+// the c0 product, a later one DC products and the carried sum (< q): at most 9 * 2^124 < 2^128.
+struct RotateCall64 {
+    KeySwitchCall64 ks;                          // slice: polynomials per work item
+    uint32_t G;
+    uint32_t gi[kAutomorphMax];                  // g_t^-1 mod 2n
+    const ulonglong2 *rk[kAutomorphMax];         // key t
+};
+
+template <int DC>
+__global__ void __launch_bounds__(256) rotate64_inner_kernel(ulonglong2 *__restrict__ acc2,
+                                                             const ulonglong2 *__restrict__ u2,
+                                                             const ulonglong2 *__restrict__ c02,
+                                                             const RnsLimb64 *__restrict__ lc,
+                                                             const BasisPair64 *__restrict__ bp,
+                                                             const __grid_constant__ RotateCall64 cp, size_t items) {
+    const KeySwitchCall64 &ks = cp.ks;
+    const uint32_t hlog = ks.logn - 1, sh = 32 - ks.logn, m2n = (2u << ks.logn) - 1;
+    const uint32_t lb = min(hlog, 5u);                             // log2 of the pairs in a block
+    const size_t row2 = (size_t)1 << hlog;
+    const size_t poly2 = (size_t)ks.L << hlog;
+    const size_t digit = (size_t)ks.B * poly2, comp = digit, keyc = (size_t)ks.key_limbs << hlog;
+    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < items; w += (size_t)gridDim.x * blockDim.x) {
+        const size_t blk = w >> lb, rest = blk / cp.G;             // rest: (row r, block of the row)
+        const uint32_t t = (uint32_t)(blk - rest * cp.G);
+        const size_t r = rest >> (hlog - lb);
+        const uint32_t j = (uint32_t)(((rest << lb) & (row2 - 1)) | (w & ((1u << lb) - 1)));   // input pair
+        const uint32_t i = (uint32_t)(r % ks.L);
+        const uint32_t b0 = (uint32_t)(r / ks.L) * ks.slice, b1 = min(ks.B, b0 + ks.slice);
+        const uint32_t e = ((__brev(2 * j) >> sh) << 1) | 1;       // 2 br(2j) + 1
+        const uint32_t d = __brev(((cp.gi[t] * e) & m2n) >> 1) >> sh;   // word 2j goes to d, word 2j + 1 to d ^ 1
+        const bool swap = d & 1;
+        const size_t o = d >> 1;                                   // the destination pair
+        const RnsLimb64 *l = lc + i;
+        const uint64_t q = __ldg(&l->p.q);
+        const RefInvConst p = RefInvLimb{l, q}.consts();
+        const uint64_t one_p = ref_shoup_companion(1, p);          // floor(2^64 / q)
+        const uint64_t r64 = 0 - one_p * q;                        // 2^64 mod q
+        const uint64_t r64_p = ref_shoup_companion(r64, p);
+        const bool has_c0 = i < ks.ell1;
+        uint64_t pm = 1;                                           // P mod q_i, P the special primes' product
+        if (has_c0) {
+            const BasisPair64 *row = bp + (size_t)i * ks.L;
+            for (uint32_t s = ks.ell1; s < ks.L; s++)
+                pm = ref_csub_u64(ref_shoup_u64(pm, __ldg(&row[s].w), __ldg(&row[s].w_p), q), q);
+        }
+        const size_t krow = has_c0 ? i : i + ks.key_off;
+        const ulonglong2 *ukey = cp.rk[t] + (krow << hlog) + o;
+        const ulonglong2 *ubase = u2 + ((size_t)i << hlog) + j;
+        const ulonglong2 *cbase = c02 + ((size_t)i << hlog) + j;   // c0h row b * (l + 1) + i
+        ulonglong2 *abase = acc2 + (size_t)t * 2 * digit + ((size_t)i << hlog) + o;
+        for (uint32_t d0 = 0; d0 < ks.dnum; d0 += DC) {
+            ulonglong2 kv[DC][2];
+#pragma unroll
+            for (int u = 0; u < DC; u++)
+                if (d0 + u < ks.dnum) {
+                    kv[u][0] = __ldg(ukey + (2 * (size_t)(d0 + u)) * keyc);
+                    kv[u][1] = __ldg(ukey + (2 * (size_t)(d0 + u) + 1) * keyc);
+                }
+            for (uint32_t b = b0; b < b1; b++) {
+                uint64_t lo[2][2] = {}, hi[2][2] = {};             // [component][word]
+                if (d0) {
+                    const ulonglong2 a0 = abase[b * poly2], a1 = abase[comp + b * poly2];
+                    lo[0][0] = a0.x; lo[0][1] = a0.y; lo[1][0] = a1.x; lo[1][1] = a1.y;
+                } else if (has_c0) {
+                    const ulonglong2 x = __ldg(cbase + (size_t)b * ks.ell1 * row2);
+                    const uint64_t xv[2] = {swap ? x.y : x.x, swap ? x.x : x.y};
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        lo[0][v] = xv[v] * pm;
+                        hi[0][v] = __umul64hi(xv[v], pm);
+                    }
+                }
+#pragma unroll
+                for (int u = 0; u < DC; u++)
+                    if (d0 + u < ks.dnum) {
+                        const ulonglong2 x = __ldg(ubase + (d0 + u) * digit + b * poly2);
+                        const uint64_t xv[2] = {swap ? x.y : x.x, swap ? x.x : x.y};
+#pragma unroll
+                        for (int c = 0; c < 2; c++) {
+                            const uint64_t kw[2] = {kv[u][c].x, kv[u][c].y};
+#pragma unroll
+                            for (int v = 0; v < 2; v++) {
+                                const uint64_t pl = xv[v] * kw[v], ph = __umul64hi(xv[v], kw[v]);
+                                lo[c][v] += pl;
+                                hi[c][v] += ph + (lo[c][v] < pl);
+                            }
+                        }
+                    }
+                uint64_t y[2][2];
+#pragma unroll
+                for (int c = 0; c < 2; c++)
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        const uint64_t s = ref_shoup_u64(hi[c][v], r64, r64_p, q) + ref_shoup_u64(lo[c][v], 1, one_p, q);
+                        y[c][v] = ref_csub_u64(ref_csub_u64(s, q << 1), q);   // s < 4q
+                    }
+                abase[b * poly2] = make_ulonglong2(y[0][0], y[0][1]);
+                abase[comp + b * poly2] = make_ulonglong2(y[1][0], y[1][1]);
+            }
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------- twiddle tables on device
 // The step before the path: the reference fills its root / precon buffers on the host (main.cpp:46-55) and the loader
 // broadcasts them (ntt.cpp:544-571).  Here one thread per (limb, direction, k) computes

@@ -380,6 +380,37 @@ int agx_automorph64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t 
 int agx_keyswitch64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint64_t *d_ksk,
                     uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream);
 
+/* ---- u64 RNS hoisted rotations in one call (no reference counterpart): G rotations or conjugations of the same
+ * ciphertexts, each with its own key, with one ModUp of c1 for all G.  ctx, alpha, k, key_limbs and the key layout are
+ * agx_keyswitch64's (dnum = ceil((l+1) / alpha) digits, the row map that lets one top-level key serve every level).
+ *   d_in  [2][B][l+1][n]: ciphertexts (c0, c1) over Q_l (the layout agx_keyswitch64 writes, so outputs can be fed back).
+ *   galois: a host array of G elements, agx_automorph64's rules (odd, in [1, 2n), G <= AGX_AUTOMORPH_MAX).
+ *   d_rk: a host array of G device pointers; key t, [>= dnum][2][key_limbs][n] in evaluation form, switches
+ *     sigma_{galois[t]}(s) back to s.  Two elements may share a key pointer; one key_limbs serves all G keys.
+ *   d_out [G][2][B][l+1][n], output t being, bit for bit and in both forms, the plain recipe of public calls:
+ *     out[t] = ( sigma_t(c0) + KS_t(sigma_t(c1))[0],  KS_t(sigma_t(c1))[1] ),
+ *   with sigma_t = agx_automorph64 with galois[t], KS_t = agx_keyswitch64 with key t and the sum agx_elementwise64's add.
+ *   The call runs the ModUp of c1's digits once, then for every t the key inner product over the permuted extended
+ *   digits with sigma_t(c0) folded in as P * sigma_t(c0) (which ModDown returns exactly), then one ModDown of all 2 G B
+ *   polynomials.
+ * Conventions are agx_keyswitch64's: device pointers 16-byte aligned, asynchronous on `stream`, inputs reduced, results
+ * in [0, q); d_in and the keys are not modified.  Scratch: one buffer from the context's key-switch pool (see
+ * agx_keyswitch64) of (dnum + 2 G) * B * L * n words, plus B * min(alpha, l+1) * n when dnum > 1, plus B * (l+1) * n in
+ * coefficient form; the ModDown's scratch (evaluation form: 2 G B k n words) comes from the same pool; the ModUps take
+ * their own (agx_modup64).  The elements' inverses and the key pointers are passed by value as a kernel parameter.
+ * AGX_E_INVALID, launching nothing, for: a u32 context; with B > 0 a null d_out, d_in or d_rk[t]; with G > 0 a null
+ * galois or d_rk; a pointer not 16-byte aligned; k = 0 or k >= L; alpha = 0; key_limbs < L; two equal primes anywhere in
+ * the context; an element that is even, 0 or >= 2n; 2 * G * B * L or dnum * B * L above 2^31 - 1; d_out (2 G B (l+1) n
+ * words) overlapping d_in (2 B (l+1) n words) or the dnum * 2 * key_limbs * n words read from any key.
+ * AGX_E_UNSUPPORTED for G > 64 (the elements and keys are then not read), min(alpha, l+1) > 16 or k > 16.
+ * B == 0 or G == 0 returns AGX_OK and launches nothing.
+ * Launches (agx_launch_count), independent of G: evaluation form sum_j up_j + 1 + down with agx_keyswitch64's up_j and
+ * down: 3 * dnum + 4 for digits of two or more primes and k >= 2, 4 * dnum + 5 at n = 32768 (one fewer per one-prime
+ * digit, and one fewer for k = 1).  Coefficient form dnum + 5 (one ModUp per digit; the forward of the extended digits;
+ * the forward of c0; the inner products; the inverse of A; the ModDown), dnum + 6 at n = 32768. ---- */
+int agx_rotate64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                 const uint64_t *const *d_rk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

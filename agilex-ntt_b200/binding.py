@@ -87,6 +87,8 @@ def _load() -> C.CDLL:
         "agx_keyswitch64": [vp, vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_rotate64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.POINTER(vp), C.c_uint32, C.c_uint32, C.c_uint32,
                          C.c_int, vp],
+        "agx_lintrans64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.POINTER(vp), C.c_uint32, C.POINTER(vp),
+                           C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -106,7 +108,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
            "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
-           "agx_automorph64 agx_keyswitch64 agx_rotate64").split()
+           "agx_automorph64 agx_keyswitch64 agx_rotate64 agx_lintrans64").split()
 
 _lib = None
 
@@ -568,6 +570,58 @@ class Context64:
         ptrs = (C.c_void_p * max(len(rks), 1))(*[_dev_ptr8(rk) for rk in rks])
         _ck(lib().agx_rotate64(self._h, _dev_ptr8(out), _dev_ptr8(ct), B, C.cast(arr, _u32p), len(gs), ptrs, key_limbs,
                                alpha, k, int(bool(ntt_form)), _stream_ptr(stream)), "agx_rotate64")
+        return out
+
+    def lintrans(self, out, ct, galois, rks, diags, alpha, k, ntt_form=True, stream=None):
+        """Hoisted linear transform in one call (agx_lintrans64), this context being Q_l u P with the k special primes
+        last: ct (2, B, L - k, n), ciphertexts (c0, c1) over Q_l; galois a sequence of G ints (at most 64); rks G keys
+        laid out as for rotate, or None where the element is 1 (the identity term, with no key switch); diags M
+        sequences (at most 16, M * G <= 256) of G entries, each an (L, n) tensor over all L primes in evaluation form, or
+        None for a zero diagonal.  out (M, 2, B, L - k, n): out[m] = ModDown_P(sum_t diags[m][t] * A_t), A_t rotate's
+        inner product for element t before its ModDown, so out[m] is sum_t d_{m,t} rot_t(ct) with one ModUp for all G
+        and one rounding per output (not bit-equal to summing rotate's outputs, which rounds G times).  ntt_form: ct and
+        out in evaluation form (else both in coefficient form; keys and diagonals are in evaluation form either way).
+        out must not overlap ct, the keys or the diagonals.  The result belongs to a context over primes[:L - k]."""
+        gs = [int(g) for g in galois]
+        rks = list(rks)
+        diags = [list(row) for row in diags]
+        keys = [rk for rk in rks if rk is not None]
+        dlist = [d for row in diags for d in row if d is not None]
+        self._check_dev(out, ct, *keys, *dlist)
+        if not 0 < int(k) < self.L:
+            raise ValueError(f"k must be in [1, {self.L - 1}]")
+        alpha, k = int(alpha), int(k)
+        if not 1 <= alpha < 1 << 32:
+            raise ValueError("alpha must be a 32-bit unsigned integer, at least 1")
+        ell1 = self.L - k
+        if ct.dim() != 4 or ct.shape[0] != 2 or tuple(ct.shape[2:]) != (ell1, self.n):
+            raise ValueError(f"ct must have shape (2, B, {ell1}, {self.n})")
+        B, G, M = ct.shape[1], len(gs), len(diags)
+        if tuple(out.shape) != (M, 2, B, ell1, self.n):
+            raise ValueError(f"out must have shape {(M, 2, B, ell1, self.n)}")
+        if any(not 0 <= g < 1 << 32 for g in gs):
+            raise ValueError("Galois elements must be 32-bit unsigned integers (odd, below 2n)")
+        if len(rks) != G:
+            raise ValueError(f"rks must hold one key (or None for the element 1) per Galois element ({G})")
+        if any(rk is None and g != 1 for rk, g in zip(rks, gs)):
+            raise ValueError("only the element 1 may go without a key")
+        if any(len(row) != G for row in diags):
+            raise ValueError(f"every row of diags must hold one entry (or None) per Galois element ({G})")
+        dnum = -(-ell1 // min(alpha, ell1))
+        key_limbs = keys[0].shape[2] if keys and keys[0].dim() == 4 else self.L
+        for rk in keys:
+            if rk.dim() != 4 or rk.shape[0] < dnum or rk.shape[1] != 2 or rk.shape[2] != key_limbs or \
+                    key_limbs < self.L or rk.shape[3] != self.n:
+                raise ValueError(f"every key must have shape (D >= {dnum}, 2, key_limbs >= {self.L}, {self.n}), "
+                                 "with one key_limbs for all")
+        for d in dlist:
+            if tuple(d.shape) != (self.L, self.n):
+                raise ValueError(f"every diagonal must have shape ({self.L}, {self.n})")
+        arr = (C.c_uint32 * max(G, 1))(*gs)
+        kp = (C.c_void_p * max(G, 1))(*[None if rk is None else _dev_ptr8(rk) for rk in rks])
+        dp = (C.c_void_p * max(M * G, 1))(*[None if d is None else _dev_ptr8(d) for row in diags for d in row])
+        _ck(lib().agx_lintrans64(self._h, _dev_ptr8(out), _dev_ptr8(ct), B, C.cast(arr, _u32p), G, kp, key_limbs, dp, M,
+                                 alpha, k, int(bool(ntt_form)), _stream_ptr(stream)), "agx_lintrans64")
         return out
 
 

@@ -2112,6 +2112,98 @@ int agx_rotate64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, co
     return rc;
 }
 
+static_assert(kLintransMaxOut == AGX_LINTRANS_MAX_OUT && kLintransMaxTerms == AGX_LINTRANS_MAX_TERMS,
+              "the header states the call's bounds");
+
+int agx_lintrans64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                   const uint64_t *const *d_rk, uint32_t key_limbs, const uint64_t *const *d_diag, uint32_t M,
+                   uint32_t alpha, uint32_t k, int ntt_form, void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_out, (const void *)d_in})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    if (G && (!galois || !d_rk)) return AGX_E_INVALID;
+    if (M && (!G || !d_diag)) return AGX_E_INVALID;
+    const uint32_t L = c->L;
+    if (!ks_params_valid(c, key_limbs, alpha, k)) return AGX_E_INVALID;
+    const uint32_t ell1 = L - k, m = std::min(alpha, ell1), dnum = (ell1 + m - 1) / m;
+    if (B > 0x7fffffffull / ((size_t)dnum * L) || (B && M > 0x7fffffffull / (2ull * L * B))) return AGX_E_INVALID;
+    const size_t N = c->n;
+    const size_t in_w = 2 * B * ell1 * N, out_w = (size_t)M * in_w, key_w = (size_t)dnum * 2 * key_limbs * N;
+    const bool work = B && M;
+    if (work && ranges_overlap(d_out, out_w, d_in, in_w)) return AGX_E_INVALID;
+    if (G > kAutomorphMax || M > kLintransMaxOut || (size_t)M * G > kLintransMaxTerms) return AGX_E_UNSUPPORTED;
+    LintransCall64 cp{};
+    uint32_t gi[kAutomorphMax];                                    // unused: the kernel gathers with g itself
+    if (!galois_inverses(c, galois, G, gi)) return AGX_E_INVALID;
+    for (uint32_t t = 0; t < G; t++) {
+        const uint64_t *rk = d_rk[t];
+        if ((B && !rk && galois[t] != 1) || (reinterpret_cast<uintptr_t>(rk) & 15)) return AGX_E_INVALID;
+        if (work && rk && ranges_overlap(d_out, out_w, rk, key_w)) return AGX_E_INVALID;
+    }
+    uint32_t keep[kAutomorphMax];                                  // the terms with a non-zero diagonal: the others add nothing
+    for (uint32_t t = 0; t < G; t++) {
+        bool used = false;
+        for (uint32_t j = 0; j < M; j++) {
+            const uint64_t *d = d_diag[(size_t)j * G + t];
+            if (reinterpret_cast<uintptr_t>(d) & 15) return AGX_E_INVALID;
+            if (work && d && ranges_overlap(d_out, out_w, d, (size_t)L * N)) return AGX_E_INVALID;
+            used |= d != nullptr;
+        }
+        if (used) keep[cp.G++] = t;
+    }
+    if (m > kBasisMaxSrc || k > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (!work) return AGX_OK;
+    for (uint32_t u = 0; u < cp.G; u++) {
+        const uint32_t t = keep[u];
+        cp.g[u] = galois[t];
+        cp.rk[u] = reinterpret_cast<const ulonglong2 *>(d_rk[t]);
+        for (uint32_t j = 0; j < M; j++) cp.diag[j * cp.G + u] = reinterpret_cast<const ulonglong2 *>(d_diag[(size_t)j * G + t]);
+    }
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t T = B * L;
+    // scratch: U [dnum][B][L][n] (c1's extended digits), Acc [M][2][B][L][n] (the sums), with dnum > 1 one digit
+    // [B][m][n] gathered for ModUp, and in coefficient form the spectra of c0 and c1 [2][B][l+1][n]
+    int rc = ks_pool_ready(c);
+    if (rc) return rc;
+    uint64_t *U = nullptr;
+    const size_t words = (dnum + 2 * (size_t)M) * T + (dnum > 1 ? B * m : 0) + (ntt_form ? 0 : 2 * B * ell1);
+    rc = (int)cudaMallocFromPoolAsync(reinterpret_cast<void **>(&U), words * N * sizeof(uint64_t), c->ks_pool, st);
+    uint64_t *Acc = rc ? nullptr : U + dnum * T * N, *dig = rc ? nullptr : Acc + 2 * M * T * N;
+    uint64_t *cth = rc ? nullptr : dig + (dnum > 1 ? B * m * N : 0);
+    if (!rc) rc = ks_modup_digits(c, U, dig, d_in + B * ell1 * N, B, ell1, m, dnum, ntt_form, st);
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, U, U, dnum * T, st, 0, L);   // the products are per limb in evaluation form
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, d_in, cth, 2 * B * ell1, st, 0, ell1);   // c0 and c1 in one launch
+    if (!rc) {
+        KeySwitchCall64 &ks = cp.ks;
+        ks.L = L; ks.logn = c->logn; ks.ell1 = ell1; ks.key_off = key_limbs - L; ks.key_limbs = key_limbs;
+        ks.dnum = dnum; ks.B = (uint32_t)B;
+        cp.M = M;
+        const size_t items = T * N / 2;
+        const unsigned blocks = (unsigned)std::min<size_t>((items + 255) / 256, (size_t)c->sms * 8);
+        auto *a2 = reinterpret_cast<ulonglong2 *>(Acc);
+        const auto *u2 = reinterpret_cast<const ulonglong2 *>(U);
+        const auto *c2 = reinterpret_cast<const ulonglong2 *>(ntt_form ? d_in : cth);
+        const RnsLimb64 *lc = c->d_lc64;
+        const BasisPair64 *bp = c->d_bp64;
+#define AGX_LINTRANS(DC)                                                                               \
+    (M <= 4 ? lintrans64_inner_kernel<DC, 4><<<blocks, 256, 0, st>>>(a2, u2, c2, lc, bp, cp, items)    \
+            : lintrans64_inner_kernel<DC, 16><<<blocks, 256, 0, st>>>(a2, u2, c2, lc, bp, cp, items))
+        if (dnum == 1) AGX_LINTRANS(1);
+        else if (dnum == 2) AGX_LINTRANS(2);
+        else if (dnum <= 4) AGX_LINTRANS(4);
+        else AGX_LINTRANS(kKeySwitchChunk);
+#undef AGX_LINTRANS
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc && !ntt_form) rc = rns_inv_launch(c, Acc, nullptr, Acc, 2 * M * T, st, 0, L);
+    // every output's two components as one batch of 2 M B, with its scratch from the pool too
+    if (!rc) rc = moddown_launch(c, d_out, Acc, 2 * M * B, k, ntt_form, st, c->ks_pool);
+    if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {
     if (!c || !per_clk_per_sm || kind < 0 || kind > 6) return AGX_E_INVALID;
     if (threads_per_sm < 128 || threads_per_sm > 1024 || threads_per_sm % 128) return AGX_E_INVALID;

@@ -2724,6 +2724,34 @@ __global__ void __cluster_dims__(CL, 1, 1) __launch_bounds__(kAutomorphThreads, 
 // run in chunks of DC, each chunk's reduced sum stored in A and carried into the next.
 constexpr uint32_t kKeySwitchChunk = 8;      // most digits a thread holds key words for at once
 
+// The constants of limb q that reduce a 128-bit lazy sum: floor(2^64 / q), 2^64 mod q and its Shoup companion.
+struct LazyRed64 {
+    uint64_t q, one_p, r64, r64_p;
+};
+
+__device__ __forceinline__ LazyRed64 lazy_red64(const RnsLimb64 *l) {
+    LazyRed64 r;
+    r.q = __ldg(&l->p.q);
+    const RefInvConst p = RefInvLimb{l, r.q}.consts();
+    r.one_p = ref_shoup_companion(1, p);
+    r.r64 = 0 - r.one_p * r.q;
+    r.r64_p = ref_shoup_companion(r.r64, p);
+    return r;
+}
+
+// hi * 2^64 + lo += a * b
+__device__ __forceinline__ void mac128(uint64_t &lo, uint64_t &hi, uint64_t a, uint64_t b) {
+    const uint64_t pl = a * b, ph = __umul64hi(a, b);
+    lo += pl;
+    hi += ph + (lo < pl);
+}
+
+// (hi * 2^64 + lo) mod q, exact for every 128-bit value
+__device__ __forceinline__ uint64_t reduce128(uint64_t lo, uint64_t hi, const LazyRed64 &r) {
+    const uint64_t s = ref_shoup_u64(hi, r.r64, r.r64_p, r.q) + ref_shoup_u64(lo, 1, r.one_p, r.q);
+    return ref_csub_u64(ref_csub_u64(s, r.q << 1), r.q);           // s < 4q
+}
+
 struct KeySwitchCall64 {
     uint32_t L, logn;
     uint32_t ell1;           // l + 1: the limbs of Q_l, which read key rows 0 .. l
@@ -2745,12 +2773,7 @@ __global__ void __launch_bounds__(256) keyswitch64_inner_kernel(ulonglong2 *__re
         const size_t j = w & (row2 - 1), r = w >> hlog;
         const uint32_t i = (uint32_t)(r % cp.L);
         const uint32_t b0 = (uint32_t)(r / cp.L) * cp.slice, b1 = min(cp.B, b0 + cp.slice);
-        const RnsLimb64 *l = lc + i;
-        const uint64_t q = __ldg(&l->p.q);
-        const RefInvConst p = RefInvLimb{l, q}.consts();
-        const uint64_t one_p = ref_shoup_companion(1, p);          // floor(2^64 / q)
-        const uint64_t r64 = 0 - one_p * q;                        // 2^64 mod q
-        const uint64_t r64_p = ref_shoup_companion(r64, p);
+        const LazyRed64 red = lazy_red64(lc + i);
         const size_t krow = i < cp.ell1 ? i : i + cp.key_off;
         const ulonglong2 *ukey = k2 + (krow << hlog) + j;
         const ulonglong2 *ubase = u2 + ((size_t)i << hlog) + j;
@@ -2779,26 +2802,35 @@ __global__ void __launch_bounds__(256) keyswitch64_inner_kernel(ulonglong2 *__re
                         for (int c = 0; c < 2; c++) {
                             const uint64_t kw[2] = {kv[t][c].x, kv[t][c].y};
 #pragma unroll
-                            for (int v = 0; v < 2; v++) {
-                                const uint64_t pl = xv[v] * kw[v], ph = __umul64hi(xv[v], kw[v]);
-                                lo[c][v] += pl;
-                                hi[c][v] += ph + (lo[c][v] < pl);
-                            }
+                            for (int v = 0; v < 2; v++) mac128(lo[c][v], hi[c][v], xv[v], kw[v]);
                         }
                     }
                 uint64_t y[2][2];
 #pragma unroll
                 for (int c = 0; c < 2; c++)
 #pragma unroll
-                    for (int v = 0; v < 2; v++) {
-                        const uint64_t s = ref_shoup_u64(hi[c][v], r64, r64_p, q) + ref_shoup_u64(lo[c][v], 1, one_p, q);
-                        y[c][v] = ref_csub_u64(ref_csub_u64(s, q << 1), q);   // s < 4q
-                    }
+                    for (int v = 0; v < 2; v++) y[c][v] = reduce128(lo[c][v], hi[c][v], red);
                 abase[b * poly2] = make_ulonglong2(y[0][0], y[0][1]);
                 abase[comp + b * poly2] = make_ulonglong2(y[1][0], y[1][1]);
             }
         }
     }
+}
+
+// P mod q_i for a limb i of Q_l, P the product of the special primes q_{l+1} .. q_{L-1}, from the pairwise table
+__device__ __forceinline__ uint64_t p_mod_q(const BasisPair64 *__restrict__ bp, uint32_t i, uint32_t ell1, uint32_t L,
+                                            uint64_t q) {
+    const BasisPair64 *row = bp + (size_t)i * L;
+    uint64_t pm = 1;
+    for (uint32_t s = ell1; s < L; s++) pm = ref_csub_u64(ref_shoup_u64(pm, __ldg(&row[s].w), __ldg(&row[s].w_p), q), q);
+    return pm;
+}
+
+// automorph64_ntt_kernel's permutation in evaluation form: the entry that word `word` of a row comes from under element
+// `g` (out[k] = in[pi_g(k)]), or where it goes under g^-1.  sh = 32 - log n, m2n = 2n - 1.
+__device__ __forceinline__ uint32_t eval_perm(uint32_t g, uint32_t word, uint32_t sh, uint32_t m2n) {
+    const uint32_t e = ((__brev(word) >> sh) << 1) | 1;            // 2 br(word) + 1
+    return __brev(((g * e) & m2n) >> 1) >> sh;
 }
 
 // ------------------------------------------------------------- u64 RNS hoisted rotations: the G key inner products
@@ -2843,23 +2875,12 @@ __global__ void __launch_bounds__(256) rotate64_inner_kernel(ulonglong2 *__restr
         const uint32_t j = (uint32_t)(((rest << lb) & (row2 - 1)) | (w & ((1u << lb) - 1)));   // input pair
         const uint32_t i = (uint32_t)(r % ks.L);
         const uint32_t b0 = (uint32_t)(r / ks.L) * ks.slice, b1 = min(ks.B, b0 + ks.slice);
-        const uint32_t e = ((__brev(2 * j) >> sh) << 1) | 1;       // 2 br(2j) + 1
-        const uint32_t d = __brev(((cp.gi[t] * e) & m2n) >> 1) >> sh;   // word 2j goes to d, word 2j + 1 to d ^ 1
+        const uint32_t d = eval_perm(cp.gi[t], 2 * j, sh, m2n);   // word 2j goes to d, word 2j + 1 to d ^ 1
         const bool swap = d & 1;
         const size_t o = d >> 1;                                   // the destination pair
-        const RnsLimb64 *l = lc + i;
-        const uint64_t q = __ldg(&l->p.q);
-        const RefInvConst p = RefInvLimb{l, q}.consts();
-        const uint64_t one_p = ref_shoup_companion(1, p);          // floor(2^64 / q)
-        const uint64_t r64 = 0 - one_p * q;                        // 2^64 mod q
-        const uint64_t r64_p = ref_shoup_companion(r64, p);
+        const LazyRed64 red = lazy_red64(lc + i);
         const bool has_c0 = i < ks.ell1;
-        uint64_t pm = 1;                                           // P mod q_i, P the special primes' product
-        if (has_c0) {
-            const BasisPair64 *row = bp + (size_t)i * ks.L;
-            for (uint32_t s = ks.ell1; s < ks.L; s++)
-                pm = ref_csub_u64(ref_shoup_u64(pm, __ldg(&row[s].w), __ldg(&row[s].w_p), q), q);
-        }
+        const uint64_t pm = has_c0 ? p_mod_q(bp, i, ks.ell1, ks.L, red.q) : 1;   // P mod q_i
         const size_t krow = has_c0 ? i : i + ks.key_off;
         const ulonglong2 *ukey = cp.rk[t] + (krow << hlog) + o;
         const ulonglong2 *ubase = u2 + ((size_t)i << hlog) + j;
@@ -2896,25 +2917,150 @@ __global__ void __launch_bounds__(256) rotate64_inner_kernel(ulonglong2 *__restr
                         for (int c = 0; c < 2; c++) {
                             const uint64_t kw[2] = {kv[u][c].x, kv[u][c].y};
 #pragma unroll
-                            for (int v = 0; v < 2; v++) {
-                                const uint64_t pl = xv[v] * kw[v], ph = __umul64hi(xv[v], kw[v]);
-                                lo[c][v] += pl;
-                                hi[c][v] += ph + (lo[c][v] < pl);
-                            }
+                            for (int v = 0; v < 2; v++) mac128(lo[c][v], hi[c][v], xv[v], kw[v]);
                         }
                     }
                 uint64_t y[2][2];
 #pragma unroll
                 for (int c = 0; c < 2; c++)
 #pragma unroll
-                    for (int v = 0; v < 2; v++) {
-                        const uint64_t s = ref_shoup_u64(hi[c][v], r64, r64_p, q) + ref_shoup_u64(lo[c][v], 1, one_p, q);
-                        y[c][v] = ref_csub_u64(ref_csub_u64(s, q << 1), q);   // s < 4q
-                    }
+                    for (int v = 0; v < 2; v++) y[c][v] = reduce128(lo[c][v], hi[c][v], red);
                 abase[b * poly2] = make_ulonglong2(y[0][0], y[0][1]);
                 abase[comp + b * poly2] = make_ulonglong2(y[1][0], y[1][1]);
             }
         }
+    }
+}
+
+// ------------------------------------------------------------- u64 RNS hoisted linear transforms: sum_t d_t (.) A_t
+// agx_lintrans64's one kernel of its own.  In: agx_rotate64's U[dnum][B][L][n] and keys, the ciphertexts'
+// spectra ct[2][B][l+1][n] (c0, then c1), and M x G diagonals d_{m,t}[L][n] over Q_l u P; all in evaluation form.
+// Out: Acc[M][2][B][L][n],
+//   Acc[m][c][b][i][o] = sum_t d_{m,t}[i][o] * A_t[c][b][i][o]  mod q_i,
+// A_t being rotate64_inner_kernel's output t (the key inner product over the permuted digits plus P sigma_t(c0)), or
+// (P c0, P c1) for a keyless term (g = 1).  ModDown of Acc[m] is then sum_t d_{m,t} sigma_t(c0) + ModDown(sum_t d_{m,t}
+// KS_t) by the same fold as agx_rotate64's.  A work item owns one output pair o of one limb row of one polynomial and
+// gathers: for each term t it reads key t's words at o and U and ct at the source pair pi_t(o) (out[k] =
+// in[pi_g(k)], automorph64_ntt_kernel's map; the pair is swapped when pi_t(2o) is odd), forms A_t in registers, and
+// adds d_{m,t} * A_t into each of the M accumulators.  So no A_t reaches memory, and keys and digits are read once per
+// (element, term) however large M is.  pi_t maps an aligned 32-pair block onto an aligned block and keeps pairs
+// together, so every warp gather covers whole 512-byte blocks.  Items run limb-major, (limb, polynomial, pair): the B
+// polynomials of one limb follow one another and share that limb's key and diagonal rows (2 G dnum + M G rows of
+// n / 2 pairs), which therefore come from HBM once per call and from L2 for the other polynomials, while the rows being
+// gathered (U, c0, c1 of a few polynomials) are small enough to serve their G re-reads from L2 too.
+// A_t's lazy sum is rotate64_inner_kernel's chunking (DC <= 8 products plus the c0 product or the carried sum).  The
+// accumulators are kept reduced: each d * A_t (< q^2 < 2^124) is added to one (< q) and the 128-bit sum reduced at
+// once, so a thread holds MC x 4 words, MC = 4 or 16 (the most outputs of its instantiation).  Terms whose diagonals
+// are all zero are dropped on the host; a NULL d_{m,t} is skipped.
+constexpr uint32_t kLintransMaxOut = 16;      // outputs per call (agx_lintrans64)
+constexpr uint32_t kLintransMaxTerms = 256;   // diagonals per call: M * G
+
+struct LintransCall64 {
+    KeySwitchCall64 ks;                          // slice unused
+    uint32_t G, M;                               // terms kept, outputs
+    uint32_t g[kAutomorphMax];                   // term t's Galois element
+    const ulonglong2 *rk[kAutomorphMax];         // key t; nullptr: a keyless identity term
+    const ulonglong2 *diag[kLintransMaxTerms];   // d_{m,t} at [m * G + t]; nullptr: zero
+};
+
+template <int DC, int MC>
+__global__ void __launch_bounds__(256) lintrans64_inner_kernel(ulonglong2 *__restrict__ acc2,
+                                                               const ulonglong2 *__restrict__ u2,
+                                                               const ulonglong2 *__restrict__ ct2,
+                                                               const RnsLimb64 *__restrict__ lc,
+                                                               const BasisPair64 *__restrict__ bp,
+                                                               const __grid_constant__ LintransCall64 cp, size_t items) {
+    const KeySwitchCall64 &ks = cp.ks;
+    const uint32_t hlog = ks.logn - 1, sh = 32 - ks.logn, m2n = (2u << ks.logn) - 1;
+    const size_t row2 = (size_t)1 << hlog;
+    const size_t poly2 = (size_t)ks.L << hlog;
+    const size_t digit = (size_t)ks.B * poly2, keyc = (size_t)ks.key_limbs << hlog;
+    const size_t c1off = (size_t)ks.B * ks.ell1 * row2;            // c1 after c0 in ct
+    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < items; w += (size_t)gridDim.x * blockDim.x) {
+        const size_t r = w >> hlog;                                // (limb i, polynomial b), limb-major
+        const uint32_t o = (uint32_t)(w & (row2 - 1));             // output pair
+        const uint32_t i = (uint32_t)(r / ks.B), b = (uint32_t)(r - (size_t)i * ks.B);
+        const LazyRed64 red = lazy_red64(lc + i);
+        const bool has_c0 = i < ks.ell1;
+        const uint64_t pm = has_c0 ? p_mod_q(bp, i, ks.ell1, ks.L, red.q) : 0;   // P mod q_i; P = 0 mod p_t
+        const size_t krow = has_c0 ? i : i + ks.key_off;
+        const ulonglong2 *ubase = u2 + (size_t)b * poly2 + ((size_t)i << hlog);
+        const ulonglong2 *cbase = ct2 + ((size_t)b * ks.ell1 + i) * row2;
+        const size_t dof = ((size_t)i << hlog) + o;                // the output pair in a diagonal
+        uint64_t acc[MC][2][2] = {};                               // [output][component][word], reduced
+        for (uint32_t t = 0; t < cp.G; t++) {
+            const ulonglong2 *rk = cp.rk[t];
+            if (!rk && !has_c0) continue;                          // (P c0, P c1) is zero on the special primes
+            const uint32_t s = eval_perm(cp.g[t], 2 * o, sh, m2n);   // word 2o comes from s, word 2o + 1 from s ^ 1
+            const bool swap = s & 1;
+            const size_t src = s >> 1;
+            uint64_t a[2][2];                                      // A_t at the output pair: [component][word]
+            if (!rk) {
+#pragma unroll
+                for (int c = 0; c < 2; c++) {
+                    const ulonglong2 x = __ldg(cbase + c * c1off + src);
+                    const uint64_t xv[2] = {swap ? x.y : x.x, swap ? x.x : x.y};
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        uint64_t lo = 0, hi = 0;
+                        mac128(lo, hi, xv[v], pm);
+                        a[c][v] = reduce128(lo, hi, red);
+                    }
+                }
+            } else {
+                const ulonglong2 *ukey = rk + (krow << hlog) + o;
+                for (uint32_t d0 = 0; d0 < ks.dnum; d0 += DC) {
+                    uint64_t lo[2][2] = {}, hi[2][2] = {};
+                    if (d0) {
+#pragma unroll
+                        for (int c = 0; c < 2; c++)
+#pragma unroll
+                            for (int v = 0; v < 2; v++) lo[c][v] = a[c][v];
+                    } else if (has_c0) {
+                        const ulonglong2 x = __ldg(cbase + src);
+                        mac128(lo[0][0], hi[0][0], swap ? x.y : x.x, pm);
+                        mac128(lo[0][1], hi[0][1], swap ? x.x : x.y, pm);
+                    }
+#pragma unroll
+                    for (int u = 0; u < DC; u++)
+                        if (d0 + u < ks.dnum) {
+                            const ulonglong2 x = __ldg(ubase + (d0 + u) * digit + src);
+                            const uint64_t xv[2] = {swap ? x.y : x.x, swap ? x.x : x.y};
+#pragma unroll
+                            for (int c = 0; c < 2; c++) {
+                                const ulonglong2 kv = __ldg(ukey + (2 * (size_t)(d0 + u) + c) * keyc);
+                                mac128(lo[c][0], hi[c][0], xv[0], kv.x);
+                                mac128(lo[c][1], hi[c][1], xv[1], kv.y);
+                            }
+                        }
+#pragma unroll
+                    for (int c = 0; c < 2; c++)
+#pragma unroll
+                        for (int v = 0; v < 2; v++) a[c][v] = reduce128(lo[c][v], hi[c][v], red);
+                }
+            }
+#pragma unroll
+            for (int m = 0; m < MC; m++) {
+                const ulonglong2 *dg = m < (int)cp.M ? cp.diag[m * cp.G + t] : nullptr;
+                if (!dg) continue;
+                const ulonglong2 dv = __ldg(dg + dof);
+                const uint64_t dw[2] = {dv.x, dv.y};
+#pragma unroll
+                for (int c = 0; c < 2; c++)
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        uint64_t lo = acc[m][c][v], hi = 0;
+                        mac128(lo, hi, dw[v], a[c][v]);
+                        acc[m][c][v] = reduce128(lo, hi, red);
+                    }
+            }
+        }
+        ulonglong2 *abase = acc2 + (size_t)b * poly2 + ((size_t)i << hlog) + o;
+#pragma unroll
+        for (int m = 0; m < MC; m++)
+            if (m < (int)cp.M)
+#pragma unroll
+                for (int c = 0; c < 2; c++) abase[(2 * (size_t)m + c) * digit] = make_ulonglong2(acc[m][c][0], acc[m][c][1]);
     }
 }
 

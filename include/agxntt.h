@@ -411,6 +411,51 @@ int agx_keyswitch64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t 
 int agx_rotate64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
                  const uint64_t *const *d_rk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int ntt_form, void *stream);
 
+/* ---- u64 RNS hoisted linear transforms in one call (no reference counterpart): M plaintext-weighted sums of G
+ * rotations of the same ciphertexts, out[m] = sum_t d_{m,t} (.) rot_t(ct), with one ModUp of c1 for all G and one
+ * ModDown per output (double hoisting: the baby steps of a baby-step/giant-step matrix-vector product, CoeffToSlot /
+ * SlotToCoeff factors, slot sums).  ctx, alpha, k, key_limbs, the key layout and galois are agx_rotate64's.
+ *   d_in  [2][B][l+1][n]: ciphertexts (c0, c1) over Q_l, agx_rotate64's layout.
+ *   d_rk: a host array of G device pointers, key t switching sigma_t(s) to s; d_rk[t] may be NULL only when
+ *     galois[t] == 1: that term is the identity, with no key switch.
+ *   d_diag: a host array of M * G device pointers; entry m * G + t is the diagonal d_{m,t}, [L][n] over all L primes of
+ *     the context (Q_l u P), in evaluation form as agx_ntt64_fwd leaves it (in both forms of the call), shared by the
+ *     whole batch.  NULL is a zero diagonal and is skipped; entries may share a pointer.  A diagonal encoded over Q_l
+ *     reaches Q_l u P with agx_modup64.
+ *   d_out [M][2][B][l+1][n], for every m and c = 0, 1:
+ *     A_t[c]    = sum_j sigma_t(ModUp_j(digit_j(c1))) (.) rk_t[j][c] + [c = 0] P sigma_t(c0)   (agx_rotate64's, over Q_l u P)
+ *     A_t       = (P c0, P c1)                                        when galois[t] == 1 and d_rk[t] == NULL
+ *     out[m][c] = ModDown_P( sum_t d_{m,t} (.) A_t[c] ),
+ *   P x being 0 on the special primes and (P mod q_i) x on limb i of Q_l.  So out[m] = sum_t d_{m,t} sigma_t(c0) +
+ *   ModDown(sum_t d_{m,t} KS_t): one rounding per output.  Every step is exact, so the result equals, bit for bit, that
+ *   sequence of public calls (modup of each digit, automorph, elementwise products and sums, one moddown of 2 M B); it is
+ *   NOT bit-equal to sum_t d_{m,t} (.) agx_rotate64(...)[t], which rounds G times.  An output whose diagonals are all
+ *   NULL is the zero ciphertext, and it is written.  ntt_form != 0: d_in and d_out are spectra; ntt_form == 0: both in
+ *   natural coefficient order, d_out then being agx_ntt64_inv (over Q_l) of the evaluation-form result applied to
+ *   agx_ntt64_fwd(d_in).  Keys and diagonals are in evaluation form either way.
+ * Conventions are agx_rotate64's: device pointers 16-byte aligned, asynchronous on `stream`, inputs reduced, results in
+ * [0, q); d_in, keys and diagonals are not modified.  Scratch: one buffer from the context's key-switch pool (see
+ * agx_keyswitch64) of (dnum + 2 M) * B * L * n words, plus B * min(alpha, l+1) * n when dnum > 1, plus 2 B (l+1) n in
+ * coefficient form; the ModDown's scratch comes from the same pool; the ModUps take their own.  No [G] buffer: the
+ * A_t are formed in registers and never stored.  Elements, key and diagonal pointers travel by value as a kernel
+ * parameter; terms whose M diagonals are all NULL are dropped before the launch.
+ * AGX_E_INVALID, launching nothing, for agx_rotate64's cases (a u32 context; with B > 0 a null d_out or d_in; with
+ * G > 0 a null galois or d_rk; a pointer not 16-byte aligned; k = 0 or k >= L; alpha = 0; key_limbs < L; two equal
+ * primes; an even element, 0 or >= 2n) and for: with B > 0 a NULL key with g != 1; G == 0 with M > 0; M > 0 with a null
+ * d_diag; 2 M B L or dnum B L above 2^31 - 1; with B, M > 0, d_out (2 M B (l+1) n words) overlapping d_in
+ * (2 B (l+1) n), the dnum * 2 * key_limbs * n words read from any key, or any non-NULL diagonal (L n words).
+ * AGX_E_UNSUPPORTED for G > 64, M > AGX_LINTRANS_MAX_OUT or M * G > AGX_LINTRANS_MAX_TERMS (the elements, keys and
+ * diagonals are then not read), min(alpha, l+1) > 16 or k > 16.  B == 0 or M == 0 returns AGX_OK and launches nothing.
+ * Launches (agx_launch_count), independent of G and M and equal to agx_rotate64's: evaluation form 3 * dnum + 4 for
+ * digits of two or more primes and k >= 2, 4 * dnum + 5 at n = 32768 (one fewer per one-prime digit, and one fewer for
+ * k = 1).  Coefficient form dnum + 5 (one ModUp per digit; the forward of the extended digits; the forward of c0 and c1;
+ * the inner sums; the inverse of the sums; the ModDown), dnum + 6 at n = 32768. ---- */
+#define AGX_LINTRANS_MAX_OUT 16    /* M */
+#define AGX_LINTRANS_MAX_TERMS 256 /* M * G: the diagonal pointers travel by value as a kernel parameter (< 4 KB) */
+int agx_lintrans64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B, const uint32_t *galois, uint32_t G,
+                   const uint64_t *const *d_rk, uint32_t key_limbs, const uint64_t *const *d_diag, uint32_t M,
+                   uint32_t alpha, uint32_t k, int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

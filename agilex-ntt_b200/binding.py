@@ -89,6 +89,7 @@ def _load() -> C.CDLL:
                          C.c_int, vp],
         "agx_lintrans64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.POINTER(vp), C.c_uint32, C.POINTER(vp),
                            C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
+        "agx_mulrelin64": [vp, vp, vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -108,7 +109,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
            "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
-           "agx_automorph64 agx_keyswitch64 agx_rotate64 agx_lintrans64").split()
+           "agx_automorph64 agx_keyswitch64 agx_rotate64 agx_lintrans64 agx_mulrelin64").split()
 
 _lib = None
 
@@ -622,6 +623,42 @@ class Context64:
         dp = (C.c_void_p * max(M * G, 1))(*[None if d is None else _dev_ptr8(d) for row in diags for d in row])
         _ck(lib().agx_lintrans64(self._h, _dev_ptr8(out), _dev_ptr8(ct), B, C.cast(arr, _u32p), G, kp, key_limbs, dp, M,
                                  alpha, k, int(bool(ntt_form)), _stream_ptr(stream)), "agx_lintrans64")
+        return out
+
+    def mulrelin(self, out, a, b, rlk, alpha, k, rescale=False, ntt_form=True, stream=None):
+        """Ciphertext multiplication in one call (agx_mulrelin64), this context being Q_l u P with the k special primes
+        last: a and b (2, B, L - k, n), ciphertexts over Q_l (the same tensor squares); rlk the relinearisation key (the
+        key-switch key for s^2), laid out as for keyswitch.  With D_0 = a0 b0, D_1 = a0 b1 + a1 b0, D_2 = a1 b1 and
+        A_c = sum_j ModUp_j(digit_j(D_2)) * rlk[j][c] + P D_c over Q_l u P:
+        rescale False: out (2, B, L - k, n), out[c] = ModDown_P(A_c) = D_c + keyswitch(D_2)[c], bit for bit;
+        rescale True: out (2, B, L - k - 1, n), A_c divided by q_l P (the last k + 1 primes) and rounded once, i.e.
+        moddown with k + 1, which equals rescale of the unrescaled result bit for bit (the roundings compose); it
+        belongs to a context over primes[:L - k - 1].  ntt_form: a, b and out in evaluation form (else all in coefficient form; the key is in
+        evaluation form either way).  out must not overlap a, b or rlk."""
+        self._check_dev(out, a, b, rlk)
+        if not 0 < int(k) < self.L:
+            raise ValueError(f"k must be in [1, {self.L - 1}]")
+        alpha, k = int(alpha), int(k)
+        if not 1 <= alpha < 1 << 32:
+            raise ValueError("alpha must be a 32-bit unsigned integer, at least 1")
+        ell1 = self.L - k
+        for t in (a, b):
+            if t.dim() != 4 or t.shape[0] != 2 or tuple(t.shape[2:]) != (ell1, self.n):
+                raise ValueError(f"a and b must have shape (2, B, {ell1}, {self.n})")
+        B = a.shape[1]
+        if b.shape[1] != B:
+            raise ValueError("a and b must hold the same number of ciphertexts")
+        if rescale and ell1 < 2:
+            raise ValueError("rescale needs at least two primes in Q_l")
+        want = (2, B, ell1 - 1 if rescale else ell1, self.n)
+        if tuple(out.shape) != want:
+            raise ValueError(f"out must have shape {want}")
+        dnum = -(-ell1 // min(alpha, ell1))
+        if rlk.dim() != 4 or rlk.shape[0] < dnum or rlk.shape[1] != 2 or rlk.shape[2] < self.L or rlk.shape[3] != self.n:
+            raise ValueError(f"rlk must have shape (D >= {dnum}, 2, key_limbs >= {self.L}, {self.n})")
+        _ck(lib().agx_mulrelin64(self._h, _dev_ptr8(out), _dev_ptr8(a), _dev_ptr8(b), B, _dev_ptr8(rlk), rlk.shape[2],
+                                 alpha, k, int(bool(rescale)), int(bool(ntt_form)), _stream_ptr(stream)),
+            "agx_mulrelin64")
         return out
 
 

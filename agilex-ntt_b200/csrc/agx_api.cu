@@ -2204,6 +2204,81 @@ int agx_lintrans64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_in, size_t B, 
     return rc;
 }
 
+int agx_mulrelin64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_a, const uint64_t *d_b, size_t B,
+                   const uint64_t *d_rlk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int rescale, int ntt_form,
+                   void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_out, (const void *)d_a, (const void *)d_b, (const void *)d_rlk})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    const uint32_t L = c->L;
+    if (!ks_params_valid(c, key_limbs, alpha, k)) return AGX_E_INVALID;
+    const uint32_t ell1 = L - k, m = std::min(alpha, ell1), dnum = (ell1 + m - 1) / m;
+    if (rescale && ell1 < 2) return AGX_E_INVALID;
+    if (B > 0x7fffffffull / (2ull * L) || B > 0x7fffffffull / ((size_t)dnum * L)) return AGX_E_INVALID;
+    const uint32_t kd = rescale ? k + 1 : k;                       // the last kd primes are divided out: P or q_l P
+    const size_t N = c->n;
+    const size_t in_w = 2 * B * ell1 * N, out_w = 2 * B * (L - kd) * N, key_w = (size_t)dnum * 2 * key_limbs * N;
+    if (B && (ranges_overlap(d_out, out_w, d_a, in_w) || ranges_overlap(d_out, out_w, d_b, in_w) ||
+              ranges_overlap(d_out, out_w, d_rlk, key_w)))
+        return AGX_E_INVALID;
+    if (m > kBasisMaxSrc || kd > kBasisMaxSrc) return AGX_E_UNSUPPORTED;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    const size_t T = B * L, Tq = B * ell1;
+    const bool square = d_a == d_b;
+    // scratch: U [dnum][B][L][n] (D_2's extended digits), Acc [2][B][L][n] (the sums), D_2's spectrum [B][l+1][n], with
+    // dnum > 1 one digit [B][m][n] gathered for ModUp, and in coefficient form the spectra of a and b [2][B][l+1][n]
+    // (one of them when squaring)
+    int rc = ks_pool_ready(c);
+    if (rc) return rc;
+    uint64_t *U = nullptr;
+    const size_t words = (dnum + 2) * T + Tq + (dnum > 1 ? B * m : 0) + (ntt_form ? 0 : (square ? 2 : 4) * Tq);
+    rc = (int)cudaMallocFromPoolAsync(reinterpret_cast<void **>(&U), words * N * sizeof(uint64_t), c->ks_pool, st);
+    uint64_t *Acc = rc ? nullptr : U + dnum * T * N, *d2 = rc ? nullptr : Acc + 2 * T * N;
+    uint64_t *dig = rc ? nullptr : d2 + Tq * N, *ah = rc ? nullptr : dig + (dnum > 1 ? B * m * N : 0);
+    uint64_t *bh = rc || square ? ah : ah + 2 * Tq * N;
+    if (!rc && !ntt_form) rc = rns_fwd_launch(c, d_a, ah, 2 * Tq, st, 0, ell1);
+    if (!rc && !ntt_form && !square) rc = rns_fwd_launch(c, d_b, bh, 2 * Tq, st, 0, ell1);
+    const uint64_t *sa = ntt_form ? d_a : ah, *sb = ntt_form ? d_b : bh;
+    if (!rc) {                                                     // D_2's spectrum a1 b1 over Q_l, for ModUp
+        const size_t total2 = Tq * N / 2;
+        const unsigned blocks = (unsigned)std::min<size_t>((total2 + 255) / 256, (size_t)c->sms * 16);
+        elementwise64_kernel<EW_MUL><<<blocks, 256, 0, st>>>(reinterpret_cast<ulonglong2 *>(d2),
+                                                             reinterpret_cast<const ulonglong2 *>(sa + Tq * N),
+                                                             reinterpret_cast<const ulonglong2 *>(sb + Tq * N),
+                                                             c->d_lc64, ell1, c->logn, total2);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc) rc = ks_modup_digits(c, U, dig, d2, B, ell1, m, dnum, 1, st);
+    if (!rc) {
+        KeySwitchCall64 cp{};
+        cp.L = L; cp.logn = c->logn; cp.ell1 = ell1; cp.key_off = key_limbs - L; cp.key_limbs = key_limbs;
+        cp.dnum = dnum; cp.B = (uint32_t)B;
+        const size_t per_slice = (size_t)L * N / 2;
+        cp.slice = ks_slice(c, B, per_slice);
+        const size_t items = ((B + cp.slice - 1) / cp.slice) * per_slice;
+        const unsigned blocks = (unsigned)std::min<size_t>((items + 255) / 256, (size_t)c->sms * 8);
+        auto *acc2 = reinterpret_cast<ulonglong2 *>(Acc);
+        const auto *u2 = reinterpret_cast<const ulonglong2 *>(U), *k2 = reinterpret_cast<const ulonglong2 *>(d_rlk);
+        const auto *a2 = reinterpret_cast<const ulonglong2 *>(sa), *b2 = reinterpret_cast<const ulonglong2 *>(sb);
+        const RnsLimb64 *lc = c->d_lc64;
+        const BasisPair64 *bp = c->d_bp64;
+        if (dnum == 1) mulrelin64_inner_kernel<1><<<blocks, 256, 0, st>>>(acc2, u2, a2, b2, k2, lc, bp, cp, items);
+        else if (dnum == 2) mulrelin64_inner_kernel<2><<<blocks, 256, 0, st>>>(acc2, u2, a2, b2, k2, lc, bp, cp, items);
+        else if (dnum <= 4) mulrelin64_inner_kernel<4><<<blocks, 256, 0, st>>>(acc2, u2, a2, b2, k2, lc, bp, cp, items);
+        else mulrelin64_inner_kernel<kKeySwitchChunk><<<blocks, 256, 0, st>>>(acc2, u2, a2, b2, k2, lc, bp, cp, items);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc && !ntt_form) rc = rns_inv_launch(c, Acc, nullptr, Acc, 2 * T, st, 0, L);
+    // both components as one batch of 2 B over the last k primes, or the last k + 1 for the rescale
+    if (!rc) rc = moddown_launch(c, d_out, Acc, 2 * B, kd, ntt_form, st, c->ks_pool);
+    if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
+    return rc;
+}
+
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {
     if (!c || !per_clk_per_sm || kind < 0 || kind > 6) return AGX_E_INVALID;
     if (threads_per_sm < 128 || threads_per_sm > 1024 || threads_per_sm % 128) return AGX_E_INVALID;

@@ -3064,6 +3064,100 @@ __global__ void __launch_bounds__(256) lintrans64_inner_kernel(ulonglong2 *__res
     }
 }
 
+// ------------------------------------------------------------- u64 RNS ciphertext multiplication: tensor + relinearisation
+// agx_mulrelin64's one kernel of its own.  In: the dnum extended digits U[dnum][B][L][n] of D_2 = a1 b1 (ModUp's
+// outputs), the spectra a[2][B][l+1][n] and b[2][B][l+1][n] of the two ciphertexts (a == b when squaring) and the
+// relinearisation key rlk[>= dnum][2][key_limbs][n], all in evaluation form; out: A[2][B][L][n],
+//   A_c[b][i] = sum_j U_j[b][i] * rlk[j][c][row(i)]  +  [i <= l] (P mod q_i) D_c[b][i]   mod q_i,
+//   D_0 = a0 b0,  D_1 = a0 b1 + a1 b0   (per limb, mod q_i),
+// row(i) being keyswitch64_inner_kernel's.  ModDown_P of A_c is D_c + KS(D_2)[c] by rotate64_inner_kernel's fold, and
+// ModDown over q_l P (the last k + 1 primes) is the product rescaled with one rounding.  The walk is
+// keyswitch64_inner_kernel's: key words of up to DC digits in registers, one slice of the batch per work item.  D_0 and
+// D_1 are formed in registers from the four input pairs and reduced to [0, q), so (P mod q_i) D_c is one product
+// below 2^120 and the first chunk holds DC + 1 <= 9 products: below 2^128.  No D_c reaches memory.
+template <int DC>
+__global__ void __launch_bounds__(256) mulrelin64_inner_kernel(ulonglong2 *__restrict__ acc2,
+                                                               const ulonglong2 *__restrict__ u2,
+                                                               const ulonglong2 *__restrict__ a2,
+                                                               const ulonglong2 *__restrict__ b2,
+                                                               const ulonglong2 *__restrict__ k2,
+                                                               const RnsLimb64 *__restrict__ lc,
+                                                               const BasisPair64 *__restrict__ bp,
+                                                               const KeySwitchCall64 cp, size_t items) {
+    const uint32_t hlog = cp.logn - 1;
+    const size_t row2 = (size_t)1 << hlog;                         // pairs per limb row
+    const size_t poly2 = (size_t)cp.L << hlog;                     // pairs per polynomial over Q_l u P
+    const size_t ct2 = (size_t)cp.ell1 << hlog;                    // pairs per polynomial over Q_l
+    for (size_t w = (size_t)blockIdx.x * blockDim.x + threadIdx.x; w < items; w += (size_t)gridDim.x * blockDim.x) {
+        const size_t j = w & (row2 - 1), r = w >> hlog;
+        const uint32_t i = (uint32_t)(r % cp.L);
+        const uint32_t b0 = (uint32_t)(r / cp.L) * cp.slice, b1 = min(cp.B, b0 + cp.slice);
+        const LazyRed64 red = lazy_red64(lc + i);
+        const bool has_d = i < cp.ell1;                            // P D_c = 0 mod the special primes
+        const uint64_t pm = has_d ? p_mod_q(bp, i, cp.ell1, cp.L, red.q) : 0;   // P mod q_i
+        const size_t krow = has_d ? i : i + cp.key_off;
+        const ulonglong2 *ukey = k2 + (krow << hlog) + j;
+        const ulonglong2 *ubase = u2 + ((size_t)i << hlog) + j;
+        const ulonglong2 *xa = a2 + ((size_t)i << hlog) + j, *xb = b2 + ((size_t)i << hlog) + j;
+        ulonglong2 *abase = acc2 + ((size_t)i << hlog) + j;
+        const size_t keyc = (size_t)cp.key_limbs << hlog, digit = (size_t)cp.B * poly2, comp = digit;
+        const size_t ctc = (size_t)cp.B * ct2;                     // c1 after c0 in a and b
+        for (uint32_t d0 = 0; d0 < cp.dnum; d0 += DC) {
+            ulonglong2 kv[DC][2];
+#pragma unroll
+            for (int t = 0; t < DC; t++)
+                if (d0 + t < cp.dnum) {
+                    kv[t][0] = __ldg(ukey + (2 * (size_t)(d0 + t)) * keyc);
+                    kv[t][1] = __ldg(ukey + (2 * (size_t)(d0 + t) + 1) * keyc);
+                }
+            for (uint32_t b = b0; b < b1; b++) {
+                uint64_t lo[2][2] = {}, hi[2][2] = {};             // [component][word]
+                if (d0) {
+                    const ulonglong2 a0 = abase[b * poly2], a1 = abase[comp + b * poly2];
+                    lo[0][0] = a0.x; lo[0][1] = a0.y; lo[1][0] = a1.x; lo[1][1] = a1.y;
+                } else if (has_d) {
+                    const ulonglong2 x0 = __ldg(xa + b * ct2), x1 = __ldg(xa + ctc + b * ct2);
+                    const ulonglong2 y0 = __ldg(xb + b * ct2), y1 = __ldg(xb + ctc + b * ct2);
+                    const uint64_t av0[2] = {x0.x, x0.y}, av1[2] = {x1.x, x1.y};
+                    const uint64_t bv0[2] = {y0.x, y0.y}, bv1[2] = {y1.x, y1.y};
+#pragma unroll
+                    for (int v = 0; v < 2; v++) {
+                        uint64_t l0 = 0, h0 = 0, l1 = 0, h1 = 0;
+                        mac128(l0, h0, av0[v], bv0[v]);
+                        mac128(l1, h1, av0[v], bv1[v]);
+                        mac128(l1, h1, av1[v], bv0[v]);
+                        const uint64_t dc[2] = {reduce128(l0, h0, red), reduce128(l1, h1, red)};
+#pragma unroll
+                        for (int c = 0; c < 2; c++) {
+                            lo[c][v] = dc[c] * pm;
+                            hi[c][v] = __umul64hi(dc[c], pm);
+                        }
+                    }
+                }
+#pragma unroll
+                for (int t = 0; t < DC; t++)
+                    if (d0 + t < cp.dnum) {
+                        const ulonglong2 x = __ldg(ubase + (d0 + t) * digit + b * poly2);
+                        const uint64_t xv[2] = {x.x, x.y};
+#pragma unroll
+                        for (int c = 0; c < 2; c++) {
+                            const uint64_t kw[2] = {kv[t][c].x, kv[t][c].y};
+#pragma unroll
+                            for (int v = 0; v < 2; v++) mac128(lo[c][v], hi[c][v], xv[v], kw[v]);
+                        }
+                    }
+                uint64_t y[2][2];
+#pragma unroll
+                for (int c = 0; c < 2; c++)
+#pragma unroll
+                    for (int v = 0; v < 2; v++) y[c][v] = reduce128(lo[c][v], hi[c][v], red);
+                abase[b * poly2] = make_ulonglong2(y[0][0], y[0][1]);
+                abase[comp + b * poly2] = make_ulonglong2(y[1][0], y[1][1]);
+            }
+        }
+    }
+}
+
 // ------------------------------------------------------------------------------------- twiddle tables on device
 // The step before the path: the reference fills its root / precon buffers on the host (main.cpp:46-55) and the loader
 // broadcasts them (ntt.cpp:544-571).  Here one thread per (limb, direction, k) computes

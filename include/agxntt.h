@@ -456,6 +456,51 @@ int agx_lintrans64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_in, size_t B
                    const uint64_t *const *d_rk, uint32_t key_limbs, const uint64_t *const *d_diag, uint32_t M,
                    uint32_t alpha, uint32_t k, int ntt_form, void *stream);
 
+/* ---- u64 RNS ciphertext multiplication in one call (no reference counterpart): the tensor product of two
+ * ciphertexts, its relinearisation and, optionally, the rescale by q_l.  ctx, alpha, k, key_limbs and the key layout are
+ * agx_keyswitch64's: ctx is Q_l u P with the k special primes last, dnum = ceil((l+1) / min(alpha, l+1)).
+ *   d_a, d_b [2][B][l+1][n]: ciphertexts (a0, a1) and (b0, b1) over Q_l, agx_keyswitch64's output layout.  d_a == d_b
+ *     squares; both are only read, so any overlap between them is harmless.
+ *   d_rlk [>= dnum][2][key_limbs][n]: the relinearisation key, i.e. agx_keyswitch64's key for s' = s^2, in evaluation
+ *     form; its row map lets one key over Q_top u P serve every level.
+ *   For c = 0, 1, every product per limb (element-wise in evaluation form):
+ *     D_0 = a0 b0,  D_1 = a0 b1 + a1 b0,  D_2 = a1 b1                                  over Q_l
+ *     A_c = sum_j ModUp_j(digit_j(D_2)) (.) rlk[j][c]  +  P D_c                         over Q_l u P,
+ *   P D_c being (P mod q_i) D_c on limb i <= l and 0 on the special primes.
+ *   rescale == 0: d_out [2][B][l+1][n], out_c = ModDown_P(A_c) = D_c + agx_keyswitch64(D_2)[c] (the fold: ModDown of
+ *     X + P C is ModDown(X) + C exactly).  Bit for bit the recipe of public calls: the tensor, agx_keyswitch64 of D_2,
+ *     then agx_elementwise64 adds.
+ *   rescale != 0: d_out [2][B][l][n] over Q_{l-1}, belonging to the context over q_0 .. q_{l-1}:
+ *     out_c = floor((X_c + h) / (q_l P)) mod Q_{l-1},  X_c in [0, Q_l P) the CRT value of A_c, h = (q_l P - 1) / 2,
+ *     i.e. agx_moddown64 with k + 1 of A_c: bit for bit the recipe of public calls ending in one agx_moddown64(k + 1)
+ *     of the 2 B polynomials.  It rounds once, and it also equals agx_rescale64 of the rescale == 0 output bit for
+ *     bit (so the two differ by 0, within any bound of 1): h = h_P + P h_q with h_P = (P - 1) / 2 and
+ *     h_q = (q_l - 1) / 2, and floor((floor((X + h_P) / P) + h_q) / q_l) = floor((X + h) / (q_l P)) (nested floor
+ *     division); the reduction mod Q_l between the steps changes nothing mod Q_{l-1}.  The call saves the rescale's
+ *     pass, not a rounding.
+ *   ntt_form != 0: d_a, d_b and d_out are spectra; ntt_form == 0: all three in natural coefficient order, d_out then
+ *   being the inverse of the evaluation-form result on the spectra of d_a and d_b.  The key is in evaluation form
+ *   either way.
+ * Conventions are agx_keyswitch64's: device pointers 16-byte aligned, asynchronous on `stream`, inputs reduced, results
+ * in [0, q); d_a, d_b and the key are not modified.  Scratch: one buffer from the context's key-switch pool (see
+ * agx_keyswitch64) of (dnum + 2) * B * L * n + B * (l+1) * n words, plus B * min(alpha, l+1) * n when dnum > 1, plus
+ * 4 B (l+1) n in coefficient form (2 B (l+1) n when squaring); the ModDown's scratch comes from the same pool; the
+ * ModUps take their own.  D_0 and D_1 are formed in registers and never stored.
+ * AGX_E_INVALID, launching nothing, for agx_keyswitch64's cases (a u32 context; with B > 0 a null d_out, d_a, d_b or
+ * d_rlk; a pointer not 16-byte aligned; k = 0 or k >= L; alpha = 0; key_limbs < L; two equal primes) and for: rescale
+ * != 0 with l + 1 < 2; 2 B L or dnum B L above 2^31 - 1; with B > 0, d_out (2 B (l+1) n words, 2 B l n with rescale)
+ * overlapping d_a or d_b (2 B (l+1) n each) or the dnum * 2 * key_limbs * n key words read.
+ * AGX_E_UNSUPPORTED for min(alpha, l+1) > 16, k > 16, or rescale != 0 with k + 1 > 16.  B == 0 returns AGX_OK and
+ * launches nothing.
+ * Launches (agx_launch_count), independent of B: evaluation form 3 * dnum + 5 (the product D_2 = a1 b1; three per
+ * digit's ModUp; the inner sums; the ModDown's three), 4 * dnum + 6 at n = 32768; one fewer per one-prime digit, and
+ * one fewer for k = 1 without rescale (the ModDown is then agx_rescale64's two).  Coefficient form 3 * dnum + 6 (the
+ * forwards of a and b; as above; the inverse of the sums; the coefficient-form ModDown's one), 4 * dnum + 7 at
+ * n = 32768, one fewer when squaring (d_a == d_b: one forward) and one fewer per one-prime digit. ---- */
+int agx_mulrelin64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_a, const uint64_t *d_b, size_t B,
+                   const uint64_t *d_rlk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int rescale, int ntt_form,
+                   void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */

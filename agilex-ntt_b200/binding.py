@@ -90,6 +90,8 @@ def _load() -> C.CDLL:
         "agx_lintrans64": [vp, vp, vp, C.c_size_t, _u32p, C.c_uint32, C.POINTER(vp), C.c_uint32, C.POINTER(vp),
                            C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, vp],
         "agx_mulrelin64": [vp, vp, vp, vp, C.c_size_t, vp, C.c_uint32, C.c_uint32, C.c_uint32, C.c_int, C.c_int, vp],
+        "agx_encode64": [vp, vp, vp, C.c_size_t, C.c_double, C.c_uint32, C.c_int, vp],
+        "agx_decode64": [vp, vp, vp, C.c_size_t, C.c_double, C.c_uint32, C.c_int, vp],
         "agx_measure_butterfly_peak": [vp, C.c_int, C.c_int, C.POINTER(C.c_double), C.POINTER(C.c_double)],
         "agx_launch_count": [vp, _u64p],
         "agx_variant": [vp, C.c_char_p, C.c_size_t],
@@ -109,7 +111,7 @@ EXPORTS = ("agx_create agx_create_tables agx_set_tables agx_ref_fwd_dev agx_ref_
            "agx_checksum agx_ref_input agx_ref_fwd agx_ref_output agx_wait agx_error_string agx_launch_count "
            "agx_variant agx_create64 agx_get_psi64 agx_get_tables64 agx_ntt64_fwd agx_ntt64_inv agx_polymul64 "
            "agx_polymul64_by_spectrum agx_elementwise64 agx_rescale64 agx_moddown64 agx_modup64 "
-           "agx_automorph64 agx_keyswitch64 agx_rotate64 agx_lintrans64 agx_mulrelin64").split()
+           "agx_automorph64 agx_keyswitch64 agx_rotate64 agx_lintrans64 agx_mulrelin64 agx_encode64 agx_decode64").split()
 
 _lib = None
 
@@ -146,6 +148,11 @@ def _dev_ptr8(t) -> int:
     if not t.is_cuda or not t.is_contiguous() or t.element_size() != 8 or t.is_floating_point() or t.is_complex():
         raise ValueError("need a contiguous CUDA tensor of an 8-byte integer dtype")
     return t.data_ptr()
+
+
+def _complex128():
+    import torch
+    return torch.complex128
 
 
 def _stream_ptr(stream) -> int:
@@ -660,6 +667,34 @@ class Context64:
                                  alpha, k, int(bool(rescale)), int(bool(ntt_form)), _stream_ptr(stream)),
             "agx_mulrelin64")
         return out
+
+    def _slots_and_residues(self, z, res):
+        self._check_dev(z, res)
+        if z.dtype != _complex128() or z.dim() != 2 or z.shape[1] != self.n // 2 or not z.is_contiguous():
+            raise ValueError(f"slots must be a contiguous complex128 tensor of shape (B, {self.n // 2})")
+        B = z.shape[0]
+        if res.dim() != 3 or res.shape[0] != B or not 1 <= res.shape[1] <= self.L or res.shape[2] != self.n:
+            raise ValueError(f"residues must have shape ({B}, limbs, {self.n}) with 1 <= limbs <= {self.L}")
+        return B, res.shape[1]
+
+    def encode(self, out, z, scale, ntt_form=True, stream=None):
+        """CKKS encoding (agx_encode64): slots z (B, n/2) complex128 -> out (B, limbs, n) int64 or uint64 over the first
+        limbs primes (limbs from out's shape): c_i = rint(scale * m_i), m the real polynomial with m(zeta^(5^j)) = z_j,
+        zeta = exp(i pi / n), reduced mod each prime exactly at any magnitude.  ntt_form: out in evaluation form as fwd
+        leaves it (else coefficient form).  With limbs = L, out[b] is a diagonal as lintrans takes it."""
+        B, limbs = self._slots_and_residues(z, out)
+        _ck(lib().agx_encode64(self._h, _dev_ptr8(out), z.data_ptr(), B, float(scale), limbs, int(bool(ntt_form)),
+                               _stream_ptr(stream)), "agx_encode64")
+        return out
+
+    def decode(self, z, inp, scale, ntt_form=True, stream=None):
+        """CKKS decoding (agx_decode64): inp (B, limbs, n) over the first limbs primes -> slots z (B, n/2) complex128:
+        the centred CRT value of each coefficient over q_0 ... q_(limbs-1), divided by scale, then evaluated at
+        zeta^(5^j).  ntt_form: inp in evaluation form (else coefficient form); inp is not modified."""
+        B, limbs = self._slots_and_residues(z, inp)
+        _ck(lib().agx_decode64(self._h, z.data_ptr(), _dev_ptr8(inp), B, float(scale), limbs, int(bool(ntt_form)),
+                               _stream_ptr(stream)), "agx_decode64")
+        return z
 
 
 def galois_element(n: int, step: int) -> int:

@@ -1,6 +1,7 @@
 // agx_api.cu -- the C ABI of include/agxntt.h over the sm_100a kernels.  No torch types, no CPU fallback.
 #include "../../include/agxntt.h"
 
+#include <cmath>
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -16,6 +17,7 @@
 #include <vector>
 
 #include "agx_ntt_kernels.cuh"
+#include "agx_encode.cuh"
 #include "agx_diag.cuh"
 // Build-time option, OFF in the shipped library: the radix-16 three-pass kernels for n = 4096 (16 coefficients per thread,
 // 40 warps per SM).  Bit-exact, measured 6-9 % slower than the two-pass kernels (profiles/r02_experiments.md), kept out of
@@ -109,6 +111,7 @@ struct agx_ctx {
     // agx_keyswitch64's scratch (gigabytes at real batch sizes): a pool of this context that keeps its memory between
     // calls, so that a call does not map it afresh, as the device's default pool would after every synchronisation
     cudaMemPool_t ks_pool = nullptr;
+    double2 *d_slot_tw = nullptr;                          // agx_encode64 / agx_decode64: the special FFT's S twiddles
     std::vector<BasisLimb64> bl64;                         // host copies of both
     std::vector<BasisPair64> bp64;
     HostPipe pipe;
@@ -1259,6 +1262,58 @@ uint32_t ks_slice(const agx_ctx *c, size_t B, size_t per_slice) {
     return (uint32_t)((B + S - 1) / S);
 }
 
+
+// The special FFT's twiddles (agx_encode64 / agx_decode64), at the context's first encode or decode: entry h + j, for
+// h = 1 .. S/2 and j < h, is zeta^((5^j mod 8h) (2n / 8h)), computed in long double and rounded to double, uploaded by
+// one synchronous copy followed by a device synchronisation, and kept until agx_destroy.  The kernels' shared-memory limits are raised at the same time.
+int slots_ready(agx_ctx *c) {
+    if (c->d_slot_tw) return AGX_OK;
+    const uint32_t n = c->n, S = n / 2;
+    std::vector<double2> w(S, make_double2(0.0, 0.0));
+    const long double pi = 3.141592653589793238462643383279502884L;
+    for (uint32_t h = 1; h < S; h <<= 1) {
+        const uint32_t lenq = 8 * h;
+        uint32_t r = 1;                                            // 5^j mod lenq
+        for (uint32_t j = 0; j < h; j++) {
+            const long double a = pi * (long double)(r * (2 * n / lenq)) / (long double)n;
+            w[h + j] = make_double2((double)cosl(a), (double)sinl(a));
+            r = r * 5 % lenq;
+        }
+    }
+    const int fft_smem = kEncodeMaxLocal * sizeof(double2), crt_smem = kBasisMaxLimbs * kDecodeCrtThreads * 8;
+    cudaError_t e = cudaFuncSetAttribute(encode64_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fft_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(encode64_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, fft_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(decode64_fft_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fft_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(decode64_fft_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, fft_smem);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(decode64_crt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, crt_smem);
+    double2 *d = nullptr;
+    if (e == cudaSuccess) e = cudaMalloc(&d, S * sizeof(double2));
+    if (e == cudaSuccess) e = cudaMemcpy(d, w.data(), S * sizeof(double2), cudaMemcpyHostToDevice);
+    // a pageable upload may still be in flight when cudaMemcpy returns, and only the legacy stream is ordered after
+    // it: the caller's stream (a non-blocking one included) must find the table written
+    if (e == cudaSuccess) e = cudaDeviceSynchronize();
+    if (e != cudaSuccess) { cudaFree(d); return (int)e; }
+    c->d_slot_tw = d;
+    return AGX_OK;
+}
+
+// The slot kernels of agx_encode64 / agx_decode64: one CTA per polynomial, a 2-CTA cluster at n = 32768.
+void slot_fft_launch(agx_ctx *c, bool encode, void *out, const void *in, size_t B, uint32_t limbs, double sc,
+                     cudaStream_t st) {
+    const uint32_t logn = c->logn, th = slot_threads(logn);
+    const bool pair = logn == 15;
+    const unsigned grid = (unsigned)(pair ? 2 * B : B);
+    const size_t smem = (size_t)(pair ? kEncodeMaxLocal : c->n / 2) * sizeof(double2);
+    auto *o64 = static_cast<uint64_t *>(out);
+    auto *z = static_cast<const double2 *>(in);
+    auto *zo = static_cast<double2 *>(out);
+    auto *m = static_cast<const double *>(in);
+    if (encode && pair) encode64_kernel<2><<<grid, th, smem, st>>>(o64, z, c->d_slot_tw, c->d_bl64, c->d_lc64, logn, limbs, sc);
+    else if (encode) encode64_kernel<1><<<grid, th, smem, st>>>(o64, z, c->d_slot_tw, c->d_bl64, c->d_lc64, logn, limbs, sc);
+    else if (pair) decode64_fft_kernel<2><<<grid, th, smem, st>>>(zo, m, c->d_slot_tw, logn);
+    else decode64_fft_kernel<1><<<grid, th, smem, st>>>(zo, m, c->d_slot_tw, logn);
+    c->launches++;
+}
 }  // namespace
 
 // ================================================================================================== C ABI
@@ -1327,6 +1382,7 @@ int agx_destroy(agx_ctx *c) {
         cudaFree(c->d_lc); cudaFree(c->d_sum);
         cudaFree(c->d_tab64); cudaFree(c->d_lc64); cudaFree(c->d_rs64); cudaFree(c->d_bl64);
         if (c->ks_pool) cudaMemPoolDestroy(c->ks_pool);
+        cudaFree(c->d_slot_tw);
 #if AGX_WITH_R16
         cudaFree(c->d_tw16_fwd); cudaFree(c->d_tw16_inv); cudaFree(c->d_u16_fwd); cudaFree(c->d_u16_inv);
 #endif
@@ -2277,6 +2333,84 @@ int agx_mulrelin64(agx_ctx *c, uint64_t *d_out, const uint64_t *d_a, const uint6
     if (!rc) rc = moddown_launch(c, d_out, Acc, 2 * B, kd, ntt_form, st, c->ks_pool);
     if (U) { const int rf = (int)cudaFreeAsync(U, st); if (!rc) rc = rf; }   // freed on every path
     return rc;
+}
+
+int agx_encode64(agx_ctx *c, uint64_t *d_out, const double *d_slots, size_t B, double scale, uint32_t limbs,
+                 int ntt_form, void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_out, (const void *)d_slots})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    // scale / S must stay normal for the fold of 1 / S into it to be exact
+    if (limbs == 0 || limbs > c->L || !std::isfinite(scale) || !(scale >= std::ldexp(1.0, -1022) * (c->n / 2)))
+        return AGX_E_INVALID;
+    if (B > 0x7fffffffull / limbs) return AGX_E_INVALID;
+    const size_t N = c->n;
+    if (B && ranges_overlap(d_out, B * limbs * N, d_slots, B * N)) return AGX_E_INVALID;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    int rc = slots_ready(c);
+    if (rc) return rc;
+    slot_fft_launch(c, true, d_out, d_slots, B, limbs, scale / (double)(N / 2), st);   // 1 / S folded in: exact (normal)
+    rc = (int)cudaGetLastError();
+    if (!rc && ntt_form) rc = rns_fwd_launch(c, d_out, d_out, B * limbs, st, 0, limbs);
+    return rc;
+}
+
+int agx_decode64(agx_ctx *c, double *d_slots, const uint64_t *d_in, size_t B, double scale, uint32_t limbs,
+                 int ntt_form, void *stream) {
+    if (!c || !c->has_parms64) return AGX_E_INVALID;
+    for (const void *p : {(const void *)d_slots, (const void *)d_in})
+        if ((B && !p) || (reinterpret_cast<uintptr_t>(p) & 15)) return AGX_E_INVALID;
+    if (limbs == 0 || limbs > c->L || !(scale > 0) || !std::isfinite(scale)) return AGX_E_INVALID;
+    if (B > 0x7fffffffull / limbs) return AGX_E_INVALID;
+    for (uint32_t i = 0; i < limbs; i++)
+        for (uint32_t j = 0; j < i; j++)
+            if (c->q64[i] == c->q64[j]) return AGX_E_INVALID;
+    const size_t N = c->n;
+    if (B && ranges_overlap(d_slots, B * N, d_in, B * limbs * N)) return AGX_E_INVALID;
+    if (B == 0) return AGX_OK;
+    AGX_ON_DEVICE(c);
+    const cudaStream_t st = (cudaStream_t)stream;
+    int rc = slots_ready(c);
+    if (!rc) rc = ks_pool_ready(c);
+    if (rc) return rc;
+    // the CRT constants: scale = sm 2^se, and the mixed-radix digits of h = (Q - 1) / 2, whose residues are (q_t - 1) / 2
+    DecodeCall64 cp{};
+    cp.logn = c->logn; cp.limbs = limbs; cp.L = c->L;
+    cp.sm = frexp(scale, &cp.se);
+    for (uint32_t t = 0; t < limbs; t++) {
+        const uint64_t q = c->q64[t];
+        uint64_t v = (q - 1) / 2;
+        for (uint32_t j = 0; j < t; j++)
+            v = mulmod_u64((v + q - cp.hd[j] % q) % q, c->bp64[(size_t)t * c->L + j].inv, q);
+        cp.hd[t] = v;
+    }
+    // scratch: m [B][n] doubles, and in evaluation form the coefficient-form residues [B][limbs][n]
+    uint64_t *tmp = nullptr;
+    rc = scratch_alloc(&tmp, B * N + (ntt_form ? B * limbs * N : 0), c->ks_pool, st);
+    if (rc) return rc;
+    double *m = reinterpret_cast<double *>(tmp);
+    const uint64_t *src = d_in;
+    if (ntt_form) {
+        rc = rns_inv_launch(c, d_in, nullptr, tmp + B * N, B * limbs, st, 0, limbs);
+        src = tmp + B * N;
+    }
+    if (!rc) {
+        const size_t total = B * N;
+        const unsigned blocks = (unsigned)std::min<size_t>((total + kDecodeCrtThreads - 1) / kDecodeCrtThreads,
+                                                           (size_t)c->sms * 16);
+        decode64_crt_kernel<<<blocks, kDecodeCrtThreads, (size_t)limbs * kDecodeCrtThreads * 8, st>>>(
+            m, src, c->d_bl64, c->d_bp64, cp, total);
+        c->launches++;
+        rc = (int)cudaGetLastError();
+    }
+    if (!rc) {
+        slot_fft_launch(c, false, d_slots, m, B, limbs, 0.0, st);
+        rc = (int)cudaGetLastError();
+    }
+    const int rf = (int)cudaFreeAsync(tmp, st);                  // freed on every path
+    return rc ? rc : rf;
 }
 
 int agx_measure_butterfly_peak(agx_ctx *c, int kind, int threads_per_sm, double *per_clk_per_sm, double *sm_mhz) {

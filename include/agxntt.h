@@ -501,6 +501,51 @@ int agx_mulrelin64(agx_ctx *ctx, uint64_t *d_out, const uint64_t *d_a, const uin
                    const uint64_t *d_rlk, uint32_t key_limbs, uint32_t alpha, uint32_t k, int rescale, int ntt_form,
                    void *stream);
 
+/* ---- u64 RNS CKKS encoding and decoding (no reference counterpart): complex slot vectors to plaintexts and back.
+ * n = 2^logn, S = n / 2 slots, zeta = exp(i pi / n).  Slot j of a real polynomial m is m(zeta^(5^j mod 2n)), j < S, so
+ * agx_automorph64 with g = 5^r (a rotation by r steps) maps the slot vector z to out_j = z_(j+r mod S), and g = 2n - 1
+ * conjugates every slot.  Encoding is the inverse with real coefficients: m_i = (2 / n) sum_j Re(z_j zeta^(-i 5^j)).
+ * Both calls run the special FFT of length S in FP64 on the device (the HEAAN form: stage twiddles zeta^((5^j mod 8h)
+ * (2n / 8h)) for half-length h), one CTA per polynomial with its S complex words in shared memory; at n = 32768 a 2-CTA
+ * cluster per polynomial (the encode's first and the decode's last stage cross the halves).
+ *   d_slots [B][S][2] doubles (re, im): a contiguous complex128 (B, S).  Residues [B][limbs][n] over the context's first
+ *   `limbs` primes, 1 <= limbs <= L.  With limbs = L on a Q_l u P context the encode writes what agx_lintrans64 takes as
+ *   a diagonal (ntt_form = 1); with limbs = l + 1 a plaintext over Q_l.
+ * agx_encode64: m~ = the FP64 inverse special FFT of z (its 1 / S folded into the scale, exactly: scale / S is kept
+ *   normal by the refusal below), c_i = rint(fl(scale
+ *   m~_i)) rounding half to even, an integer of any magnitude a double holds, and out[b][l][i] = c_i mod q_l in [0, q_l).
+ *   The residue is exact at every magnitude: |c| < 2^63 through a 64-bit integer, above that c = M 2^e with M < 2^53 and
+ *   (M mod q) times 2^e mod q, the sign applied last (scales above 2^64, e.g. q_l q_(l-1), are normal).  Error against
+ *   the exact m: |c_i - scale m_i| <= 1/2 + scale ||z||_inf * 5 * log2(n) * 2^-53 (DESIGN.md s.4).  Slot values are not
+ *   checked: a non-finite slot gives unspecified residues.  ntt_form != 0: the output equals, bit for bit,
+ *   agx_ntt64_fwd over limbs 0 .. limbs - 1 of the coefficient-form output.
+ * agx_decode64: X_i the CRT value of in[b][0 .. limbs-1][i] over Q = q_0 ... q_(limbs-1), X_c = ((X + h) mod Q) - h with
+ *   h = (Q - 1) / 2 (agx_modup64's centred lift), m_i = X_c / scale in FP64, z = the FP64 forward special FFT of m.
+ *   ntt_form != 0: d_in is a spectrum, decoded as agx_ntt64_inv of it.  The CRT step is exact mixed-radix digits
+ *   (Garner, O(limbs^2) per coefficient: decoding normally happens at low levels), the centring done on the digits
+ *   (no cancellation), then Horner in double from the top digit and one division: |m_i - X_c / scale| <=
+ *   (2 limbs + 1) 2^-53 |X_c / scale|; |X_c| / scale >= 2^1024 gives +-inf.  The FFT adds at most
+ *   5 log2(n) 2^-53 S ||m||_inf per slot.  d_in is not modified.
+ * Conventions are agx_rescale64's: device pointers 16-byte aligned, asynchronous on `stream`; residues reduced.
+ * AGX_E_INVALID, launching nothing, for: a u32 context; a null pointer with B > 0; a pointer not 16-byte aligned;
+ * limbs = 0 or limbs > L; a scale that is not finite or is <= 0 (for the encode, below 2^-1022 * S); B * limbs >
+ * 2^31 - 1; byte ranges of the slots
+ * (B * n words) and the residues (B * limbs * n words) that overlap; for the decode, two equal primes among the first
+ * limbs.  B == 0 returns AGX_OK and launches nothing.
+ * Launches (agx_launch_count), independent of B, of the scale and of whether the call is the context's first: encode 1
+ * in coefficient form, 2 in evaluation form (the forward over the output limbs, in place); decode 2 in coefficient form
+ * (the CRT step, the FFT), 3 in evaluation form (the inverse into scratch first), 4 at n = 32768 where the inverse
+ * streams its last stage.  n = 32768 adds no launch of its own (the clusters).
+ * Scratch: the decode takes B * n doubles, plus B * limbs * n words in evaluation form, from the context's key-switch
+ * pool (agx_keyswitch64).  The S twiddles (complex128, 256 KB at n = 32768) are computed on the host in long double at
+ * the context's first encode or decode, uploaded by one synchronous cudaMemcpy followed by cudaDeviceSynchronize (a
+ * pageable upload may still be in flight when cudaMemcpy returns, and a non-blocking stream is not ordered after it),
+ * and kept until agx_destroy. ---- */
+int agx_encode64(agx_ctx *ctx, uint64_t *d_out, const double *d_slots, size_t B, double scale, uint32_t limbs,
+                 int ntt_form, void *stream);
+int agx_decode64(agx_ctx *ctx, double *d_slots, const uint64_t *d_in, size_t B, double scale, uint32_t limbs,
+                 int ntt_form, void *stream);
+
 /* ---- diagnostics ---- */
 const char *agx_error_string(int code);
 /* kernels this library launched on ctx since creation (bench.py's gpu_launches claim) */
